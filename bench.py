@@ -2,7 +2,7 @@
 """Benchmark of the NCuts hot path (BASELINE.json metric: NCuts chunks/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--config tarl_spatial|spatial|tarl_spatial_dino] [--workload batch|map]
+                    [--config tarl_spatial|spatial|tarl_spatial_dino] [--workload batch|map] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default workload (BASELINE.json configs[1]): config_tarl_spatial (alpha 1.0, theta 0.5, T 0.03) on synthetic
@@ -322,6 +322,34 @@ def emit(line: dict):
     out.flush()
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write every array of `arrays` (name -> numpy array) as out_dir/<name>.npy, float64 arrays as float64
+    and everything else as float32 (integers up to 2^24 are exact there, labels included), at most DUMP_BYTES in all.
+    Beyond that, every array over 1 MB is replaced by the same seeded sample of its flattened elements, in index order, and
+    <name>_index.npy (float64) says which elements were kept, so that two runs with the same arguments stay comparable."""
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        wide = a.dtype == np.float64 or (a.dtype.kind in "iu" and a.size and int(np.abs(a).max()) >= 1 << 24)
+        out[name] = a.astype(np.float64 if wide else np.float32)
+    big = [n for n, a in out.items() if a.nbytes > 1 << 20]
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BYTES:
+        room = DUMP_BYTES - sum(out[n].nbytes for n in out if n not in big)
+        frac = room / sum(out[n].nbytes + 8 * out[n].size for n in big)         # + the float64 index of every kept element
+        for n in big:
+            a = out[n].reshape(-1)
+            idx = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * frac), replace=False))
+            out[n] = a[idx]
+            out[n + "_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 class Dist:
     """Rank bookkeeping + the timing helper of the contract (barrier + synchronize on both sides, CUDA events on the
     current stream, MAX over ranks; min / mean over ranks reported next to it)."""
@@ -419,8 +447,10 @@ def run_batch(args):
         gat.finish()
         gather_host_ms.append(1e3 * (time.perf_counter() - t0))
 
+    last = {}
+
     def step_resident():
-        api.segment_packed(packed, dev_chunks=dev_chunks, **kw)
+        last["res"] = api.segment_packed(packed, dev_chunks=dev_chunks, **kw)
         gather()
 
     def step_single_call():             # host buffers through ONE synchronous C call: upload, cut, labels back
@@ -476,6 +506,10 @@ def run_batch(args):
     ms_step, ms_min, ms_mean = D.timed(step_resident_acct, args.steps)
     launches = hd.launch_count(reset=True)
     hd.set_stage_timing(0)
+    outputs = None
+    if args.dump_outputs and rank == 0:     # the label buffer of the last timed step, before the later legs overwrite it
+        outputs = {"labels": dev_chunks.labels[:int(packed.off[-1])].cpu().numpy(),
+                   "num_segments": last["res"].num_segments.copy()}
     mv_default = dict(mv)
     g_res = list(gather_host_ms)
     gather_host_ms.clear()
@@ -631,6 +665,8 @@ def run_batch(args):
             "cpu_baseline": cpu,
             "clocks": clocks,
         }
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     D.close()
 
@@ -711,6 +747,10 @@ def run_map(args):
     hd.launch_count(reset=True)
     ms_step, ms_min, ms_mean = D.timed(step_resident, args.steps)
     launches = hd.launch_count(reset=True)
+    outputs = None
+    if args.dump_outputs and rank == 0:     # gathered labels (chunk order) and metrics of the last timed step
+        outputs = {"labels": gat.recv[src_index].cpu().numpy()}
+        outputs.update({"metrics_" + k: np.float64(v) for k, v in last["metrics"].items()})
     ms_e2e, ms_e2e_min, ms_e2e_mean = D.timed(step_e2e, args.steps)
     stream.result()
     ms_single, _, _ = D.timed(step_single_call, min(args.steps, 3))
@@ -772,6 +812,8 @@ def run_map(args):
                                     "what": "one synchronous ancuts_segment_chunks_host call per map"}},
             "gpu_launches": int(launches) * world, "roofline": None, "cpu_baseline": None, "clocks": clocks,
         }
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     D.close()
 
@@ -804,7 +846,14 @@ def main():
     ap.add_argument("--map-lo", type=int, default=3000)
     ap.add_argument("--map-hi", type=int, default=12000)
     ap.add_argument("--min-points", type=int, default=20, help="map workload: Metrics min_points at the major level")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (labels; metrics of the map workload) as DIR/<name>.npy "
+                         "in float32 / float64, at most 64 MB (a seeded sample of larger outputs), for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path; the reference arm sizes its batch by a time budget")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
