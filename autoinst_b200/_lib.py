@@ -26,6 +26,7 @@ EXPORTS = [
     "ancuts_last_unconverged", "ancuts_set_option",
     "ancuts_merge_chunks", "ancuts_remove_semantics", "ancuts_instance_metrics", "ancuts_map_labels",
     "ancuts_last_sparse_accounting", "ancuts_dino_view_pixels", "ancuts_dino_mean",
+    "ancuts_last_reorth_accounting",
 ]
 
 # ancuts_set_option (include/autoinst_ncuts.h)
@@ -128,6 +129,7 @@ def load():
     lib.ancuts_set_option.argtypes = [vp, C.c_int, C.c_int]
     lib.ancuts_merge_chunks.argtypes = [vp, C.c_int, i64p, vp, vp, dp, C.c_double, C.c_double, vp, vp, i64p, vp]
     lib.ancuts_last_sparse_accounting.argtypes = [vp, dp]
+    lib.ancuts_last_reorth_accounting.argtypes = [vp, dp]
     lib.ancuts_dino_view_pixels.argtypes = [vp, C.c_int, vp, C.c_int, vp, C.c_double, dp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
     lib.ancuts_dino_mean.argtypes = [vp, C.c_int, C.c_int, vp, C.POINTER(vp), C.c_int, vp, vp, vp]
     lib.ancuts_map_labels.argtypes = [vp, C.c_int, i64p, vp, C.c_int, vp, vp]

@@ -67,6 +67,12 @@ class Handle:
         check(self.lib.ancuts_last_sparse_accounting(self.h, b))
         return {"entry_steps": b[0], "entries": b[1]}
 
+    def reorth_accounting(self) -> dict:
+        """Persistent Lanczos kernel, last segment call: Lanczos steps, and steps that took the full Gram-Schmidt pass."""
+        b = (C.c_double * 2)()
+        check(self.lib.ancuts_last_reorth_accounting(self.h, b))
+        return {"steps": int(b[0]), "full_passes": int(b[1])}
+
     def last_unconverged(self) -> int:
         return int(self.lib.ancuts_last_unconverged(self.h))
 
@@ -88,7 +94,8 @@ class Handle:
         """Cycles per phase of the persistent Lanczos kernel (needs ANCUTS_PHASES=1 before the handle is created)."""
         buf = (C.c_double * 32)()
         check(self.lib.ancuts_debug_phases(self.h, buf, 1 if reset else 0))
-        names = ["basis", "matvec", "alpha_3term", "check_multisection", "dots", "update_norm", "z_exchange", "check_rest"]
+        names = ["basis", "matvec", "alpha_3term_norm", "check_multisection", "full_pass_dots", "full_pass_update_norm",
+                 "norm_exchange_omega", "check_rest"]
         return {c: {nm: buf[8 * i + j] for j, nm in enumerate(names)} for i, c in enumerate((1, 2, 4, 8))}
 
     def levels(self, cap: int = 256) -> list:

@@ -31,7 +31,9 @@ enum : int { DONE_NO = 0, DONE_YES = 1, DONE_HOLD = 2 };
 
 // stages for accounting
 enum : int { SG_AFFINITY = 0, SG_DEGREE = 1, SG_MATVEC = 2, SG_REORTH = 3, SG_SCAN = 4, SG_PARTITION = 5, SG_COUNT = 6,
-             SG_SPARSE_STEPS = 6, SG_SPARSE_NNZ = 7, SG_ACCT = 8 };     // device accounting has two more slots (sparse matvec form)
+             SG_SPARSE_STEPS = 6, SG_SPARSE_NNZ = 7,     // device accounting has four more slots: sparse matvec form,
+             SG_CL_STEPS = 8, SG_CL_FULL = 9,           // Lanczos steps of the cluster kernel and those with the full pass
+             SG_ACCT = 10 };
 
 void set_error(const char* fmt, ...);
 

@@ -265,6 +265,8 @@ static int end_accounting(ancuts_handle* h, const Eng& e, cudaStream_t st) {
     for (int i = 0; i < SG_COUNT; ++i) h->stage_bytes[i] += (double)h->h_acct[i];
     h->sparse_entry_steps = (double)h->h_acct[SG_SPARSE_STEPS];
     h->sparse_nnz = (double)h->h_acct[SG_SPARSE_NNZ];
+    h->cl_steps = (double)h->h_acct[SG_CL_STEPS];
+    h->cl_full = (double)h->h_acct[SG_CL_FULL];
     for (auto& t : h->timed) {
         float ms = 0.f;
         if (cudaEventElapsedTime(&ms, t.a, t.b) == cudaSuccess) {
@@ -930,6 +932,13 @@ int ancuts_last_sparse_accounting(ancuts_handle* h, double* out2) {
     if (!h || !out2) return ANCUTS_EINVAL;
     out2[0] = h->sparse_entry_steps;
     out2[1] = h->sparse_nnz;
+    return ANCUTS_OK;
+}
+
+int ancuts_last_reorth_accounting(ancuts_handle* h, double* out2) {
+    if (!h || !out2) return ANCUTS_EINVAL;
+    out2[0] = h->cl_steps;
+    out2[1] = h->cl_full;
     return ANCUTS_OK;
 }
 

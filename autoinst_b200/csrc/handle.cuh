@@ -24,6 +24,7 @@ struct ancuts_handle {
     bool cluster16_ok = true;
     unsigned long long* h_acct = nullptr;    // pinned, ancuts::SG_ACCT
     double sparse_entry_steps = 0, sparse_nnz = 0;   // shared-memory sparse matvec: sum of k * entries, entries (last call)
+    double cl_steps = 0, cl_full = 0;                // cluster kernel: Lanczos steps, steps with the full pass (last call)
     int64_t launches_total = 0;
     int64_t stage_launches[ancuts::SG_COUNT] = {0};
     double stage_bytes[ancuts::SG_COUNT] = {0};

@@ -4,13 +4,13 @@
 // nodes of up to CL_NMAX points; larger nodes keep the grid-wide multi-launch path (kernels_lanczos.cuh).
 //
 // The C CTAs of a cluster own C row slices of the node's block.  Per step:
-//   matvec of the slice (W streamed from L2/HBM, z = S v for the whole node in shared memory),
-//   the three-term recurrence (alpha comes out of the matvec epilogue), then ONE classical Gram-Schmidt pass
-//   against u1 = D^1/2 1 and every Lanczos vector: each CTA forms the partial dots over its slice, the
-//   partials are exchanged through distributed shared memory (cluster barrier, then every CTA sums the C
-//   partials in rank order, so all CTAs hold bit-identical alpha/beta and take identical decisions); the
-//   squared norm is accumulated by the update pass.  Three cluster barriers and four block barriers per step
-//   (one CTA per node: four block barriers in all, and the partial dots are the coefficients).
+//   matvec of the slice (W streamed from L2/HBM, z = S v for the whole node in shared memory), alpha out of its
+//   epilogue and exchanged (cluster barrier 1), the three-term recurrence with the squared norm and the z push in the
+//   same pass, the norm exchanged (cluster barrier 2), then partial re-orthogonalisation: the omega recurrence decides
+//   whether this step also takes ONE classical Gram-Schmidt pass against u1 = D^1/2 1 and every Lanczos vector (partial
+//   dots over the slice exchanged through distributed shared memory, update, norm exchanged again).  Every exchange is
+//   summed by every CTA in rank order, so all CTAs hold bit-identical alpha/beta and take identical decisions.  A step
+//   without the pass: two cluster barriers and three block barriers, no sweep over the basis.
 // MODE 7 (default) keeps the slice as CSR in shared memory instead of streaming W, and a node that converged there also
 // takes its N-cut decision in the epilogue (cl_fused_cut).
 // Every sum is float64 and evaluated in a fixed order: results do not depend on scheduling.
@@ -32,6 +32,8 @@ constexpr int CL_THREADS = 512;          // 1024 threads (64 registers, 2 KB rin
 constexpr int CL_WARPS = CL_THREADS / 32;
 constexpr int CL_HALF = CL_THREADS / 2;     // shifts per eigenvalue and bisection round
 constexpr int CL_CLASSES = 6;            // node size bins (kernels_graph.cuh::cluster_class); cluster sizes 1, 2, 4, 8
+constexpr double CL_REORTH_TOL = 0x1p-26;   // sqrt(eps): an estimated |v_j . v_i| above it triggers the full Gram-Schmidt pass
+constexpr int CL_SHIFTS = CL_HALF / 2;   // shifts per eigenvalue and multisection round (cluster_tridiag_eigs)
 constexpr int CL_DYN_SMEM = 194 * 1024;  // z for the whole node + as many basis rows of the slice as fit
                                          // (one CTA per SM; 256 threads x 2 CTAs per SM measured 25 % slower)
 
@@ -44,6 +46,9 @@ struct ClusterShared {
     double be2[CL_KS], dd[CL_KS], du[CL_KS], yv[CL_KS];
     short hexp[CL_KS], pexp[CL_KS];   // exponent offsets of dd / du (cluster_tridiag_vec)
     double prev_th[2];           // the two eigenvalues at the previous check (seed of the next multisection)
+    float om[CL_KS];             // omega recurrence (partial re-orthogonalisation): om[i] estimates v_k . v_i for the newest
+                                 // Lanczos vector v_k (float: only compared with sqrt(eps)); thread i also keeps om[i] and
+                                 // its predecessor v_{k-1} . v_i in registers
     unsigned long long fdiff[NB + 1];   // fused cut: this CTA's difference array of cut weights, read by the peers
     unsigned long long fsum[NB + 1];    //            the node's difference array
     double fvol[NB];                    //            volume per bucket
@@ -56,7 +61,7 @@ struct ClusterShared {
     double red[32];
     double bounds[4];
     double gb[3];
-    int cnts[CL_THREADS];
+    int cnts[2 * CL_SHIFTS];        // Sturm counts of the multisection (two eigenvalues x CL_SHIFTS shifts); fused cut: 16 x 11
     long long tmark;             // debug phase clock: end of the multisection rounds inside cluster_tridiag
     double prev_res;             // adaptive check schedule: residual estimate and step of the last check
     int prev_k;
@@ -141,7 +146,7 @@ __device__ __forceinline__ int sturm_count_poly(const double* al, const double* 
 // dozen steps they move by less than 1e-6 between checks; the shifts of round 0 then sit at prev + (hi - prev) 2^(-0.4 j),
 // which brackets the new value to 30 % of the distance it moved, and 3-5 uniform rounds finish instead of 8.
 // th[0], th[1] = eigenvalues (also kept in S.prev_th for the next check).
-constexpr int CL_SHIFTS = CL_HALF / 2;              // 128: half as many warps on the FP64 pipe as with 256, same 8 rounds
+// CL_SHIFTS = 128: half as many warps on the FP64 pipe as with 256, same 8 rounds
 
 __device__ __forceinline__ double cl_shift(double lo, double hi, int t, bool seeded) {
     if (t < 0) return lo;
@@ -410,6 +415,22 @@ __device__ __forceinline__ double cl_update_norm(const double* __restrict__ hs, 
     return q;
 }
 
+// z = S y for the next matvec: element j of the node's z vector into the z buffer of every CTA of the cluster
+template <int C>
+__device__ __forceinline__ void cl_put_z(cg::cluster_group& cl, double* zs, int j, double zv) {
+    if (C > 1) {
+#pragma unroll
+        for (int r = 0; r < C; ++r) cl.map_shared_rank(zs, r)[j] = zv;
+    } else {
+        zs[j] = zv;
+    }
+}
+template <int C>
+__device__ __forceinline__ void cl_push_z(cg::cluster_group& cl, double* zs, const double* sv, const double* y, int r0, int nr,
+                                          int pad) {
+    for (int i = threadIdx.x; i < nr; i += CL_THREADS) cl_put_z<C>(cl, zs, r0 + i + pad, sv[i] * y[i]);
+}
+
 // sum over the CTA of one value per thread: warp partials in S.wred2, ONE block barrier, fixed order
 __device__ __forceinline__ double cl_block_sum1(ClusterShared& S, double v) {
     v = warp_sum(v);
@@ -419,6 +440,21 @@ __device__ __forceinline__ double cl_block_sum1(ClusterShared& S, double v) {
 #pragma unroll
     for (int i = 0; i < CL_WARPS; ++i) t += S.wred2[i];
     return t;
+}
+
+// norm of the node's vector from the CTAs' squared partial norms q (one cluster barrier; every CTA sums in rank order, so all
+// hold the same bits).  The barrier also publishes the z stores of cl_put_z.
+template <int C>
+__device__ __forceinline__ double cl_norm_exchange(cg::cluster_group& cl, ClusterShared& S, double q) {
+    double nn = q;
+    if (C > 1) {
+        if (threadIdx.x == 0) S.npart[0] = q;
+        cl.sync();
+        nn = 0.0;
+#pragma unroll
+        for (int r = 0; r < C; ++r) nn += cl.map_shared_rank(&S.npart[0], r)[0];
+    }
+    return sqrt(nn);
 }
 
 // float -> double widening on the integer pipe, for weights in {0} U [2^-126, 2): the bits move 29 places and the
@@ -771,6 +807,7 @@ __device__ void cl_fused_cut(cg::cluster_group& cl, ClusterShared& S, const Eng&
     // 2.7 % of the kernel's stall samples); S.hpart is free after the last Gram-Schmidt exchange: 16 x 12 counters
     unsigned long long* wdiff = reinterpret_cast<unsigned long long*>(&S.hpart[0]);
     static_assert(CL_WARPS * (NB + 1) <= CL_KS, "per-warp difference arrays alias S.hpart");
+    static_assert(CL_WARPS * NB <= 2 * CL_SHIFTS, "per-warp counts fit S.cnts");
     if (tid < CL_WARPS * (NB + 1)) wdiff[tid] = 0ull;
     __syncthreads();
     if (tid < NB) {
@@ -1030,6 +1067,11 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
     }
     __syncthreads();
 
+    float om_c = (tid == 0) ? 1.0f : 0.0f, om_p = 0.0f;  // omega_{k, tid}, omega_{k-1, tid}; omega_{0,0} = v_0 . v_0 = 1
+    if (tid == 0) S.om[0] = 1.0f;
+    double om_u = 0x1p-52, om_u_prev = 0x1p-52;          // omega of u1 against the two newest Lanczos vectors
+    bool reorth_next = false;                            // the step after a full pass takes one too
+    int nfull = 0;                                       // steps that took the full pass (accounting)
     int k = 0;
     int conv = 0;
     double th[2] = {0.0, 0.0};
@@ -1065,62 +1107,98 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
 #pragma unroll
             for (int r = 0; r < C; ++r) a1 += cl.map_shared_rank(&S.npart[0], r)[1];      // rank order
         }
-        const int rows = k + 2;
-        // ---- three-term recurrence first, then ONE classical Gram-Schmidt pass against u1 and every Lanczos
-        //      vector.  In exact arithmetic w - alpha v_k - beta v_{k-1} is already orthogonal to the basis, so the
-        //      full pass only removes rounding-level components and plays the role of the SECOND pass of "twice is
-        //      enough": orthogonality stays at 2e-15 like CGS2 (numpy model, 151 nodes, identical steps and cuts),
-        //      with two sweeps over the basis instead of four.  A single CGS pass WITHOUT the three-term part
-        //      loses orthogonality within dozens of steps (measured in round 1 and again in the model); so does a pass
-        //      that leaves alpha v_k to the Gram-Schmidt sweep (1e-3 after 60 steps in the model), which is why alpha has
-        //      its own exchange. ----
+        // ---- three-term recurrence y = M v_k - alpha v_k - beta v_{k-1}; its squared norm and z = S y for the next matvec
+        //      ride on the same pass.  z: every CTA PUSHES its slice into the z vector of all CTAs of the cluster through
+        //      distributed shared memory (every matvec of this step has ended before the alpha exchange above, so the peers'
+        //      z is free; the barrier of the norm exchange below publishes the stores). ----
+        double q = 0.0;
         {
             const double bk = (k > 0) ? S.beta[k - 1] : 0.0;
             // own elements of v_k and v_{k-1} (u1 when k = 0: bk = 0)
             const double* vp = B.row(k);
-            for (int i = tid; i < nr; i += CL_THREADS) yn[i] = (yn[i] - a1 * vk[i]) - bk * vp[i];
-        }
-        __syncthreads();
-        CL_PHASE(2);
-        cl_partial_dots(S, yn, B, rows, nr);
-        cl_sync<C>(cl);
-        const double* hsrc = S.hpart;               // one CTA per node: its partial dots are the coefficients
-        if (C > 1) { cl_reduce_h<C>(cl, S, rows, 1); hsrc = S.hs; }
-        const double a2 = hsrc[rows - 1];
-        CL_PHASE(4);
-        // ---- update, squared norm, z = S y for the next matvec ----
-        double q = cl_update_norm(hsrc, yn, B, rows, nr);
-        // z = S y for the next matvec: every CTA PUSHES its slice into the z vector of all CTAs of the cluster through
-        // distributed shared memory (every matvec of this step has ended before the barrier of the Gram-Schmidt exchange
-        // above, so the peers' z is free; the barrier of the norm exchange below publishes the stores).  Round 1 went through
-        // global memory: slice written, barrier, whole vector read back from L2 by every CTA.
-        if (C > 1) {
             for (int i = tid; i < nr; i += CL_THREADS) {
-                const double zv = S.sv[i] * yn[i];
-#pragma unroll
-                for (int r = 0; r < C; ++r) cl.map_shared_rank(zs, r)[r0 + i + pad] = zv;
+                const double y = (yn[i] - a1 * vk[i]) - bk * vp[i];
+                yn[i] = y;
+                q = fma(y, y, q);
+                cl_put_z<C>(cl, zs, r0 + i + pad, S.sv[i] * y);
             }
-        } else {
-            for (int i = tid; i < nr; i += CL_THREADS) zs[i + pad] = S.sv[i] * yn[i];
         }
         q = cl_block_sum1(S, q);
-        CL_PHASE(5);
-        double nn = q;
-        if (C > 1) {
-            if (tid == 0) S.npart[0] = q;
-            cl.sync();
-            nn = 0.0;
-#pragma unroll
-            for (int r = 0; r < C; ++r) nn += cl.map_shared_rank(&S.npart[0], r)[0];
+        CL_PHASE(2);
+        double beta = cl_norm_exchange<C>(cl, S, q);
+        // ---- partial re-orthogonalisation (Simon 1984, as in PROPACK): the omega recurrence estimates v_{k+1} . v_i of
+        //      the new vector against every Lanczos vector from alpha and beta alone, O(k) per step.  The full classical
+        //      Gram-Schmidt pass against u1 and the whole basis runs only when an estimate passes sqrt(eps), and on the step
+        //      after one (the pair v_{k+1}, v_{k+2} is made orthogonal); a pass resets the estimates to eps.  u1 = D^1/2 1 is
+        //      an exact eigenvector of M (eigenvalue 1), so its own estimate follows
+        //      beta_k w' = (1 - alpha_k) w_k - beta_{k-1} w_{k-1}, and it too is removed only by the full passes.
+        //      Every CTA evaluates the recurrence from its bit-identical alpha / beta in the same order, so the decision is
+        //      the same in the whole cluster without an exchange.  numpy model (tests/test_partial_reorth.py): the same
+        //      steps and the same Ritz vector to 1e-9 as the pass on every step, with the pass on ~5 % of the steps. ----
+        {
+            constexpr double EPS = 0x1p-52;
+            const double bn = beta;
+            const double bkm = (k > 0) ? S.beta[k - 1] : 0.0;
+            // thread i: omega_{k+1, i} from omega_{k, i-1 .. i+1} (S.om, own entry om_c) and omega_{k-1, i} (om_p)
+            float om_new = 0.0f;
+            bool hi = false;
+            if (tid < k) {                               // one estimate per thread (k <= CL_KMAX < CL_THREADS)
+                const double bi = S.beta[tid];
+                double t = bi * (double)S.om[tid + 1] + (S.alpha[tid] - a1) * (double)om_c - bkm * (double)om_p;
+                if (tid > 0) t += S.beta[tid - 1] * (double)S.om[tid - 1];
+                const double noise = 0.6 * EPS * (fabs(bi) + bn);       // rounding of the step's products, as in the model
+                t = (t + (t < 0.0 ? -noise : noise)) / bn;
+                om_new = (float)t;
+                hi = !(fabs(t) <= CL_REORTH_TOL);         // NaN (beta = 0 at a breakdown) takes the pass too
+            } else if (tid == k) {
+                om_new = (float)(EPS * 0.5 * (double)n);
+            } else if (tid == k + 1) {
+                om_new = 1.0f;
+            }
+            {
+                double t = (1.0 - a1) * om_u - bkm * om_u_prev;
+                t = (t + (t < 0.0 ? -2.0 * EPS * bn : 2.0 * EPS * bn)) / bn;
+                om_u_prev = om_u;
+                om_u = t;
+            }
+            const bool full = __syncthreads_or(hi) || reorth_next || !(fabs(om_u) <= CL_REORTH_TOL);
+            // every thread has read S.om (the barrier above): the new row replaces it
+            if (full) {
+                if (tid <= k) om_new = (float)EPS;
+                om_u = EPS;
+            }
+            om_p = om_c;
+            om_c = om_new;
+            if (tid <= k + 1) S.om[tid] = om_new;
+            CL_PHASE(6);
+            if (full) {
+                reorth_next = !reorth_next;
+                nfull += 1;
+                // ---- the full pass on y: ONE classical Gram-Schmidt pass against u1 and every Lanczos vector (rows
+                //      0 .. k+1).  After the three-term part it only removes small components, so one pass is as good as
+                //      two (test_design_choices.py).  The pass leaves alpha v_k to the three-term part: a pass that also
+                //      had to remove it loses orthogonality within dozens of steps; its own coefficient corrects alpha. ----
+                const int rows = k + 2;
+                cl_partial_dots(S, yn, B, rows, nr);      // yn is complete: the barrier of the norm sum ordered its stores
+                cl_sync<C>(cl);
+                const double* hsrc = S.hpart;             // one CTA per node: its partial dots are the coefficients
+                if (C > 1) { cl_reduce_h<C>(cl, S, rows, 1); hsrc = S.hs; }
+                a1 += hsrc[rows - 1];
+                CL_PHASE(4);
+                q = cl_update_norm(hsrc, yn, B, rows, nr);
+                cl_push_z<C>(cl, zs, S.sv, yn, r0, nr, pad);
+                q = cl_block_sum1(S, q);
+                beta = cl_norm_exchange<C>(cl, S, q);
+                CL_PHASE(5);
+            }
         }
-        const double beta = sqrt(nn);
-        if (tid == 0) { S.alpha[k] = a1 + a2; S.beta[k] = beta; }
+        if (tid == 0) { S.alpha[k] = a1; S.beta[k] = beta; }
         bprev = beta;
         k += 1;
         { double* t_ = yc; yc = yn; yn = t_; }
-        // no barrier here: what the next step reads of this one -- yc, z, alpha / beta -- is separated from its writes by the
-        // barrier of the norm reduction above or by the one that ends the next matvec (S.wred / S.wred2 are separate arrays)
-        CL_PHASE(6);
+        // no barrier here: what the next step reads of this one -- yc, z, alpha / beta, omega -- is separated from its writes
+        // by the barriers of the norm exchange and the decision above or by the one that ends the next matvec (S.wred /
+        // S.wred2 are separate arrays)
         const bool breakdown = beta < 1e-13;
         if (breakdown || k >= kcap || k == S.next_check) {
             __syncthreads();                 // alpha[k-1], beta[k-1] of thread 0
@@ -1157,6 +1235,10 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
         for (int i = 0; i < 8; ++i) atomicAdd(&e.dbg[ci * 8 + i], (unsigned long long)tph[i]);
     }
 #undef CL_PHASE
+    if (rank == 0 && tid == 0) {             // share of the steps that took the full Gram-Schmidt pass
+        atomicAdd(&e.acct[SG_CL_STEPS], (unsigned long long)k);
+        atomicAdd(&e.acct[SG_CL_FULL], (unsigned long long)nfull);
+    }
     // ---- Ritz vector of the slice, statistics for the cut kernels ----
     if (conv) {
         const bool fuse = SP && sp.ptr != nullptr && e.fuse_cut != 0;

@@ -257,6 +257,9 @@ int ancuts_set_option(ancuts_handle* h, int option, int value);
 /* Shared-memory sparse matvec form (ANCUTS_OPT_MATVEC = 0), last segment call: out2[0] = sum over the nodes it ran of
  * Lanczos steps x stored entries (what the sparse lower bound of SURVEY.md §8d multiplies by 8 bytes), out2[1] = entries. */
 int ancuts_last_sparse_accounting(ancuts_handle* h, double* out2);
+/* Persistent Lanczos kernel, last segment call: out2[0] = Lanczos steps of the nodes it ran, out2[1] = steps among them
+ * that took the full Gram-Schmidt pass (partial re-orthogonalisation, DESIGN.md §4.3). */
+int ancuts_last_reorth_accounting(ancuts_handle* h, double* out2);
 
 /* Counter for bench.py (`gpu_launches`): kernels launched by this handle since the last reset. */
 int64_t ancuts_launch_count(ancuts_handle* h, int reset);
@@ -271,8 +274,8 @@ int ancuts_set_stage_timing(ancuts_handle* h, int on);
  * kernels of the level, [3..8] nodes per size bin, [9..14] cluster size used per bin.  Returns the row count. */
 int ancuts_last_levels(ancuts_handle* h, double* out, int cap_rows);
 /* Debug (handle created with ANCUTS_PHASES=1 in the environment): cycles spent by the persistent Lanczos kernel per
- * phase, [cluster size 1,2,4,8][basis write, matvec, alpha + three-term, multisection of the check, dots, update + norm, z exchange,
- * rest of the check]. */
+ * phase, [cluster size 1,2,4,8][basis write, matvec, alpha + three-term pass with norm and z push, multisection of the check,
+ * dots of the full Gram-Schmidt pass, its update + norm, norm exchange + omega recurrence, rest of the check]. */
 int ancuts_debug_phases(ancuts_handle* h, double* out32, int reset);
 
 #ifdef __cplusplus

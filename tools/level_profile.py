@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Per-level trace of one bench step: active nodes per size bin, cluster sizes, time of the concurrent
-cluster kernels, and per-level node statistics (sum n^2, steps) from the node table.
+cluster kernels, and per-level node statistics (sum n^2, steps) from the node table; the Lanczos steps of the
+persistent kernel and how many of them took the full Gram-Schmidt pass.
 
     python tools/level_profile.py --batch 64 --out gpurun_out/levels_b64.json
 """
@@ -54,6 +55,9 @@ def main():
             print("cluster size", c, {k: round(100 * v / tot, 1) for k, v in d.items()}, "Mcycles %.1f" % (tot / 1e6), flush=True)
     res = api.segment_packed(packed, device=dev, want_stats=True, **kw)
     st = res.stats
+    ra = hd.reorth_accounting()
+    print("cluster kernel: Lanczos steps %d, steps with the full Gram-Schmidt pass %d (%.1f %%)"
+          % (ra["steps"], ra["full_passes"], 100.0 * ra["full_passes"] / max(ra["steps"], 1)), flush=True)
     rows = []
     for i, l in enumerate(lv):
         m = st[st["level"] == i + 1] if (st["level"].min() >= 1) else st[st["level"] == i]
@@ -69,7 +73,7 @@ def main():
         rows.append(l)
         print(json.dumps(l), flush=True)
     out = dict(batch=args.batch, n_target=args.n_target, levels=rows, matvec_ms=acc["matvec"]["ms"],
-               stat_levels=sorted(set(int(x) for x in st["level"])), phases=phases)
+               stat_levels=sorted(set(int(x) for x in st["level"])), phases=phases, reorth=ra)
     os.makedirs(os.path.dirname(args.out), exist_ok=True)
     json.dump(out, open(args.out, "w"), indent=1)
     print("total matvec ms", acc["matvec"]["ms"], "levels", out["stat_levels"])
