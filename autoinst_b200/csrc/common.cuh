@@ -106,6 +106,27 @@ __device__ __forceinline__ void mbarrier_wait(uint64_t* bar, uint32_t parity) {
         if (mbarrier_try_wait(bar, parity)) return;
     __trap();
 }
+// ---- one-way cluster exchange: a CTA stores into a peer's shared memory with st.async and the bytes are counted on the
+// peer's mbarrier (complete_tx, release at cluster scope); the peer waits on its own barrier (acquire at cluster scope)
+// shared::cluster address of `a` (a shared::cta address of this CTA) in the CTA of the given cluster rank
+__device__ __forceinline__ uint32_t mapa_u32(uint32_t a, int rank) {
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(rank));
+    return r;
+}
+__device__ __forceinline__ void st_async_f64(uint32_t dst, double v, uint32_t bar) {
+    asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.f64 [%0], %1, [%2];"
+                 ::"r"(dst), "d"(v), "r"(bar) : "memory");
+}
+__device__ __forceinline__ bool mbarrier_try_wait_cluster(uint64_t* bar, uint32_t parity) {
+    uint32_t ok;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(ok) : "r"(smem_addr_u32(bar)), "r"(parity) : "memory");
+    return ok != 0;
+}
 // 1-D bulk copy global -> shared memory of this CTA, completion counted in bytes on `bar`
 // (16-byte aligned addresses, size a multiple of 16)
 __device__ __forceinline__ void bulk_copy_g2s(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
@@ -176,6 +197,7 @@ struct Eng {
                           // [16]=eigensolver nodes that stopped unconverged (whole call, never reset between levels)
                           // [17]=nodes of the level whose cut was decided inside the cluster kernel (cl_fused_cut)
                           // [18]=nodes of the level the cluster kernels ran but left to the cut kernels (Eng::unfused)
+                          // [19]=cluster-exchange waits that gave up (ANCUTS_EXCHANGE_GUARD builds only; an error)
     unsigned long long* acct;   // [SG_COUNT] algorithmic bytes
     ancuts_node_stat* stats; int stats_cap;
     int w_own;            // 1 = W holds the library's own affinities (0 or [2^-126, 2)): the matvec may widen on the integer pipe

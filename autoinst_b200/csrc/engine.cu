@@ -297,6 +297,12 @@ static int set_attrs(ancuts_handle* h, int KS) {
 static int read_ctr(ancuts_handle* h, const Eng& e, cudaStream_t st) {
     ANCUTS_CUDA(cudaMemcpyAsync(h->h_ctr, e.ctr, CTR_COUNT * sizeof(int), cudaMemcpyDeviceToHost, st));
     ANCUTS_CUDA(cudaStreamSynchronize(st));
+#ifdef ANCUTS_EXCHANGE_GUARD
+    if (h->h_ctr[19]) {
+        set_error("internal: %d cluster-exchange waits of the Lanczos kernel gave up", h->h_ctr[19]);
+        return ANCUTS_EINVAL;
+    }
+#endif
     return ANCUTS_OK;
 }
 

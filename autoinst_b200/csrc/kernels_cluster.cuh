@@ -5,12 +5,13 @@
 //
 // The C CTAs of a cluster own C row slices of the node's block.  Per step:
 //   matvec of the slice (W streamed from L2/HBM, z = S v for the whole node in shared memory), alpha out of its
-//   epilogue and exchanged (cluster barrier 1), the three-term recurrence with the squared norm and the z push in the
-//   same pass, the norm exchanged (cluster barrier 2), then partial re-orthogonalisation: the omega recurrence decides
-//   whether this step also takes ONE classical Gram-Schmidt pass against u1 = D^1/2 1 and every Lanczos vector (partial
-//   dots over the slice exchanged through distributed shared memory, update, norm exchanged again).  Every exchange is
-//   summed by every CTA in rank order, so all CTAs hold bit-identical alpha/beta and take identical decisions.  A step
-//   without the pass: two cluster barriers and three block barriers, no sweep over the basis.
+//   epilogue and exchanged (pushed into every CTA, mbarrier bar_a), the three-term recurrence with the squared norm and
+//   the z push in the same pass, the norm exchanged (pushed, bar_n, which also counts the z rows), then partial
+//   re-orthogonalisation: the omega recurrence decides whether this step also takes ONE classical Gram-Schmidt pass
+//   against u1 = D^1/2 1 and every Lanczos vector (partial dots over the slice exchanged through a cluster barrier and
+//   remote reads, update, z and norm pushed again).  Every exchange is summed by every CTA in rank order, so all CTAs hold
+//   bit-identical alpha/beta and take identical decisions.  A step without the pass: no cluster barrier, two mbarrier
+//   waits and three block barriers, no sweep over the basis.
 // MODE 7 (default) keeps the slice as CSR in shared memory instead of streaming W, and a node that converged there also
 // takes its N-cut decision in the epilogue (cl_fused_cut).
 // Every sum is float64 and evaluated in a fixed order: results do not depend on scheduling.
@@ -39,7 +40,10 @@ constexpr int CL_DYN_SMEM = 194 * 1024;  // z for the whole node + as many basis
 
 struct ClusterShared {
     double hpart[CL_KS];         // this CTA's partial dots of the Gram-Schmidt pass, read by the peers
-    double npart[2];             // partial squared norm of the slice
+    double npart[2];             // set-up: [1] = this CTA's "slice does not fit" flag, read by the peers
+    double apart[8];             // step exchanges, slot [r] written by rank r with st.async: partials of alpha ...
+    double nslot[8];             // ... and of the squared norm
+    uint64_t bar_a, bar_n;       // their mbarriers (arrival count 1); bar_n also counts the z rows the peers push
     double spart[4];             // at the end: partial (sum, min, max, sum of squares) of the Ritz vector
     double hs[CL_KS];            // reduced projection coefficients
     double alpha[CL_KS], beta[CL_KS];
@@ -66,6 +70,7 @@ struct ClusterShared {
     double prev_res;             // adaptive check schedule: residual estimate and step of the last check
     int prev_k;
     int next_check;
+    int sp_nnz;                  // MODE 7: stored entries of the CSR slice (accounting)
 };
 
 // Adaptive convergence checks.  The fixed schedule (every 16 steps) runs 8 steps past convergence on average
@@ -415,20 +420,69 @@ __device__ __forceinline__ double cl_update_norm(const double* __restrict__ hs, 
     return q;
 }
 
-// z = S y for the next matvec: element j of the node's z vector into the z buffer of every CTA of the cluster
+// ---- the two exchanges of a Lanczos step (C > 1) are one-way pushes onto mbarriers, no cluster barrier:
+//   alpha: thread 0 posts expect_tx(8 C) on its bar_a and st.async's its partial into apart[rank] of every CTA, itself
+//          included; every thread waits for the phase and sums apart[0 .. C) in rank order.
+//   norm:  the three-term pass st.async's z into the peers' z buffers, counted on their bar_n; thread 0 posts
+//          expect_tx(8 (n - nr + C)) -- the z rows of all peers plus the C norm partials -- and pushes its partial into
+//          nslot[rank] of every CTA.  A full Gram-Schmidt pass pushes z and the norm again in a phase of its own.
+// Ordering (why no push lands in a phase it does not belong to, and no slot or z element is overwritten before it is read):
+//   a peer's alpha push of step k+1 follows its matvec k+1, which waited for OUR z of step k, which we push after our
+//   bar_a wait of step k; its z / norm push of step k+1 needs our alpha of step k+1, which we push after our last bar_n wait
+//   of step k; its pushes of a full pass follow the pass's cluster barrier, which we enter after our first bar_n wait of the
+//   step.  So every phase completes before a push of the next phase of the same barrier can arrive (a push that arrives
+//   before the local expect_tx only makes the transaction count negative for a while; the phase cannot complete before
+//   that arrival).  A peer rewrites our apart slots only after our next norm push, and our nslot slots only after our
+//   next alpha push or the full pass's cluster barrier; a block barrier separates every thread's read of the slots from
+//   each of these.  Our z pushes follow the peers' alpha partials of the step, so their matvec, the only reader of z, has
+//   ended.  The phase parities follow from the step count: bar_a completes once per step (k & 1), bar_n once more per full
+//   pass ((k + full passes) & 1).
+// The sums start at 0.0 and add the ranks in order, as the cluster-barrier form with remote reads did: the same bits.
+// ANCUTS_EXCHANGE_GUARD (debug builds): a wait gives up after a bounded number of polls and the step loop stops with
+// e.ctr[19] counted, so a protocol error fails the call instead of hanging the GPU.
+__device__ __forceinline__ bool cl_wait(uint64_t* bar, uint32_t parity) {
+#ifdef ANCUTS_EXCHANGE_GUARD
+    bool ok = false;
+    for (uint32_t it = 0; it < (1u << 22) && !ok; ++it) ok = mbarrier_try_wait_cluster(bar, parity);
+    return !__syncthreads_or(!ok);
+#else
+    while (!mbarrier_try_wait_cluster(bar, parity)) {}
+    return true;
+#endif
+}
+// x = sum over the cluster of every CTA's x, through `slots` and `bar` (bytes: what this CTA receives in the phase)
 template <int C>
-__device__ __forceinline__ void cl_put_z(cg::cluster_group& cl, double* zs, int j, double zv) {
-    if (C > 1) {
+__device__ __forceinline__ bool cl_exchange(double* slots, uint64_t* bar, uint32_t parity, uint32_t bytes, int rank, double& x) {
+    if (threadIdx.x == 0) {
+        mbarrier_expect_tx(bar, bytes);
+        const uint32_t sa = smem_addr_u32(slots + rank), ba = smem_addr_u32(bar);
+#pragma unroll 1
+        for (int r = 0; r < C; ++r) st_async_f64(mapa_u32(sa, r), x, mapa_u32(ba, r));
+    }
+    const bool ok = cl_wait(bar, parity);
+    double t = 0.0;
 #pragma unroll
-        for (int r = 0; r < C; ++r) cl.map_shared_rank(zs, r)[j] = zv;
-    } else {
-        zs[j] = zv;
+    for (int r = 0; r < C; ++r) t += slots[r];
+    x = t;
+    return ok;
+}
+
+// z = S y for the next matvec: element j of the node's z vector into the z buffer of every CTA of the cluster.  The own
+// copy is a plain store (the block barrier of the norm sum orders it before the next matvec), the peers' copies are
+// counted on their bar_n.
+template <int C>
+__device__ __forceinline__ void cl_put_z(ClusterShared& S, double* zs, int rank, int j, double zv) {
+    zs[j] = zv;
+    if (C > 1) {
+        const uint32_t za = smem_addr_u32(zs + j), ba = smem_addr_u32(&S.bar_n);
+#pragma unroll 1
+        for (int r = 0; r < C; ++r)
+            if (r != rank) st_async_f64(mapa_u32(za, r), zv, mapa_u32(ba, r));
     }
 }
 template <int C>
-__device__ __forceinline__ void cl_push_z(cg::cluster_group& cl, double* zs, const double* sv, const double* y, int r0, int nr,
-                                          int pad) {
-    for (int i = threadIdx.x; i < nr; i += CL_THREADS) cl_put_z<C>(cl, zs, r0 + i + pad, sv[i] * y[i]);
+__device__ __forceinline__ void cl_push_z(ClusterShared& S, double* zs, int rank, const double* y, int r0, int nr, int pad) {
+    for (int i = threadIdx.x; i < nr; i += CL_THREADS) cl_put_z<C>(S, zs, rank, r0 + i + pad, S.sv[i] * y[i]);
 }
 
 // sum over the CTA of one value per thread: warp partials in S.wred2, ONE block barrier, fixed order
@@ -442,19 +496,13 @@ __device__ __forceinline__ double cl_block_sum1(ClusterShared& S, double v) {
     return t;
 }
 
-// norm of the node's vector from the CTAs' squared partial norms q (one cluster barrier; every CTA sums in rank order, so all
-// hold the same bits).  The barrier also publishes the z stores of cl_put_z.
+// norm of the node's vector from the CTAs' squared partial norms q; the phase also completes the peers' z pushes
 template <int C>
-__device__ __forceinline__ double cl_norm_exchange(cg::cluster_group& cl, ClusterShared& S, double q) {
-    double nn = q;
-    if (C > 1) {
-        if (threadIdx.x == 0) S.npart[0] = q;
-        cl.sync();
-        nn = 0.0;
-#pragma unroll
-        for (int r = 0; r < C; ++r) nn += cl.map_shared_rank(&S.npart[0], r)[0];
-    }
-    return sqrt(nn);
+__device__ __forceinline__ bool cl_norm_exchange(ClusterShared& S, uint32_t parity, int n, int nr, int rank, double& q) {
+    bool ok = true;
+    if (C > 1) ok = cl_exchange<C>(S.nslot, &S.bar_n, parity, 8u * (uint32_t)(n - nr + C), rank, q);
+    q = sqrt(q);
+    return ok;
 }
 
 // float -> double widening on the integer pipe, for weights in {0} U [2^-126, 2): the bits move 29 places and the
@@ -659,7 +707,7 @@ __device__ __forceinline__ double cl_matvec_ring(ClusterShared& S, const double*
 // the dense kernels' order, so alpha/beta differ from the dense form in the last bits (parity is against the oracle).
 // A slice that does not fit (dense little nodes far above 100 entries per row) sends the node to the grid-wide path.
 struct SparseSlice {
-    const float* val; const unsigned short* col; const int* ptr; int nnz;
+    const float* val; const unsigned short* col; const int* ptr;
     // col holds the BYTE offset of the entry's z value inside the CTA's z buffer, 8 * (column + pad) <= 8 * 4099: the matvec
     // adds it to the buffer's address and loads (two integer instructions per entry less than index -> address)
     __device__ __forceinline__ int column(int q, int pad) const { return (int)(col[q] >> 3) - pad; }
@@ -958,7 +1006,7 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
     constexpr bool SP = (MODE == 7);
     const int nz = (n + 8 + 3) & ~3;                   // doubles used by zs
     SparseSlice sp;
-    sp.val = nullptr; sp.col = nullptr; sp.ptr = nullptr; sp.nnz = 0;
+    sp.val = nullptr; sp.col = nullptr; sp.ptr = nullptr;
     int sp_doubles = 0;
     if (SP) {
         // ---- build the CSR slice: entries per row (counted by k_degree on its pass over the block), scan, fill ----
@@ -1007,7 +1055,8 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
                 sp_fill_rows(v.W + (size_t)(v.ro + r0 + i) * v.ld, i2 < nr ? v.W + (size_t)(v.ro + r0 + i2) * v.ld : nullptr, a0,
                              c_lo, c_hi, lane, val, col, ptr[i], i2 < nr ? ptr[i2] : 0, pad);
             }
-            sp.val = val; sp.col = col; sp.ptr = ptr; sp.nnz = total - fill;
+            sp.val = val; sp.col = col; sp.ptr = ptr;
+            if (tid == 0) S.sp_nnz = total - fill;       // accounting only: shared memory, not a register across the steps
             __syncthreads();
         }
     }
@@ -1066,6 +1115,14 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
         S.sv[i] = e.sinv[v.start + j];
     }
     __syncthreads();
+    if (C > 1) {                                         // the mbarriers of the step exchanges, initialised before any peer pushes
+        if (tid == 0) {
+            mbarrier_init(&S.bar_a, 1);
+            mbarrier_init(&S.bar_n, 1);
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        }
+        cl.sync();
+    }
 
     float om_c = (tid == 0) ? 1.0f : 0.0f, om_p = 0.0f;  // omega_{k, tid}, omega_{k-1, tid}; omega_{0,0} = v_0 . v_0 = 1
     if (tid == 0) S.om[0] = 1.0f;
@@ -1083,6 +1140,8 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
     long long tph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     long long tlast = prof ? clock64() : 0;
 #define CL_PHASE(i) do { if (prof) { long long t_ = clock64(); tph[i] += t_ - tlast; tlast = t_; } } while (0)
+    // a guard build's wait gave up (cl_wait): count it and leave the step loop
+#define CL_EXCHANGE_FAILED() do { if (tid == 0) atomicAdd(&e.ctr[19], 1); } while (0)
     while (true) {
         const double invb = 1.0 / bprev;
         // basis row k+1 = current vector (slice).  The matvec below only reads yc and writes yn: no barrier in between.
@@ -1100,17 +1159,11 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
         double a1 = 0.0;
 #pragma unroll
         for (int i = 0; i < CL_WARPS; ++i) a1 += S.wred[i];
-        if (C > 1) {
-            if (tid == 0) S.npart[1] = a1;
-            cl.sync();
-            a1 = 0.0;
-#pragma unroll
-            for (int r = 0; r < C; ++r) a1 += cl.map_shared_rank(&S.npart[0], r)[1];      // rank order
-        }
+        if (C > 1 && !cl_exchange<C>(S.apart, &S.bar_a, (uint32_t)k & 1u, 8u * C, rank, a1)) { CL_EXCHANGE_FAILED(); break; }
         // ---- three-term recurrence y = M v_k - alpha v_k - beta v_{k-1}; its squared norm and z = S y for the next matvec
         //      ride on the same pass.  z: every CTA PUSHES its slice into the z vector of all CTAs of the cluster through
-        //      distributed shared memory (every matvec of this step has ended before the alpha exchange above, so the peers'
-        //      z is free; the barrier of the norm exchange below publishes the stores). ----
+        //      distributed shared memory (every matvec of this step has ended before its alpha partial was pushed, so the
+        //      peers' z is free; the stores complete the phase of the norm exchange below). ----
         double q = 0.0;
         {
             const double bk = (k > 0) ? S.beta[k - 1] : 0.0;
@@ -1120,12 +1173,13 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
                 const double y = (yn[i] - a1 * vk[i]) - bk * vp[i];
                 yn[i] = y;
                 q = fma(y, y, q);
-                cl_put_z<C>(cl, zs, r0 + i + pad, S.sv[i] * y);
+                cl_put_z<C>(S, zs, rank, r0 + i + pad, S.sv[i] * y);
             }
         }
         q = cl_block_sum1(S, q);
         CL_PHASE(2);
-        double beta = cl_norm_exchange<C>(cl, S, q);
+        double beta = q;
+        if (!cl_norm_exchange<C>(S, (uint32_t)(k + nfull) & 1u, n, nr, rank, beta)) { CL_EXCHANGE_FAILED(); break; }
         // ---- partial re-orthogonalisation (Simon 1984, as in PROPACK): the omega recurrence estimates v_{k+1} . v_i of
         //      the new vector against every Lanczos vector from alpha and beta alone, O(k) per step.  The full classical
         //      Gram-Schmidt pass against u1 and the whole basis runs only when an estimate passes sqrt(eps), and on the step
@@ -1186,9 +1240,10 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
                 a1 += hsrc[rows - 1];
                 CL_PHASE(4);
                 q = cl_update_norm(hsrc, yn, B, rows, nr);
-                cl_push_z<C>(cl, zs, S.sv, yn, r0, nr, pad);
-                q = cl_block_sum1(S, q);
-                beta = cl_norm_exchange<C>(cl, S, q);
+                cl_push_z<C>(S, zs, rank, yn, r0, nr, pad);
+                beta = cl_block_sum1(S, q);
+                // a bar_n phase of its own (nfull already counts this pass): z and the norm arrive as after the three-term pass
+                if (!cl_norm_exchange<C>(S, (uint32_t)(k + nfull) & 1u, n, nr, rank, beta)) { CL_EXCHANGE_FAILED(); break; }
                 CL_PHASE(5);
             }
         }
@@ -1197,8 +1252,8 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
         k += 1;
         { double* t_ = yc; yc = yn; yn = t_; }
         // no barrier here: what the next step reads of this one -- yc, z, alpha / beta, omega -- is separated from its writes
-        // by the barriers of the norm exchange and the decision above or by the one that ends the next matvec (S.wred /
-        // S.wred2 are separate arrays)
+        // by the block barriers of the norm sum and the decision above or by the one that ends the next matvec (S.wred /
+        // S.wred2 are separate arrays); the peers' z arrived with the bar_n phase
         const bool breakdown = beta < 1e-13;
         if (breakdown || k >= kcap || k == S.next_check) {
             __syncthreads();                 // alpha[k-1], beta[k-1] of thread 0
@@ -1235,6 +1290,7 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
         for (int i = 0; i < 8; ++i) atomicAdd(&e.dbg[ci * 8 + i], (unsigned long long)tph[i]);
     }
 #undef CL_PHASE
+#undef CL_EXCHANGE_FAILED
     if (rank == 0 && tid == 0) {             // share of the steps that took the full Gram-Schmidt pass
         atomicAdd(&e.acct[SG_CL_STEPS], (unsigned long long)k);
         atomicAdd(&e.acct[SG_CL_FULL], (unsigned long long)nfull);
@@ -1290,8 +1346,8 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
         }
         if (SP && sp.ptr && tid == 0) {      // what this form really moves: the slice once from HBM, then k sweeps over its entries
             atomicAdd(&e.acct[SG_MATVEC], 4ull * (unsigned long long)nr * n);
-            atomicAdd(&e.acct[SG_SPARSE_STEPS], (unsigned long long)k * (unsigned long long)sp.nnz);
-            atomicAdd(&e.acct[SG_SPARSE_NNZ], (unsigned long long)sp.nnz);
+            atomicAdd(&e.acct[SG_SPARSE_STEPS], (unsigned long long)k * (unsigned long long)S.sp_nnz);
+            atomicAdd(&e.acct[SG_SPARSE_NNZ], (unsigned long long)S.sp_nnz);
         }
         if (fuse) cl_fused_cut<C>(cl, S, e, zs, sp, v, a, rank, r0, nr, pad, k, th);
         else if (rank == 0 && tid == 0 && e.unfused) e.unfused[atomicAdd(&e.ctr[18], 1)] = a;     // the cut kernels take it
