@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("ANCUTS_LIB_PATH") or os.path.join(_HERE, "lib", "liba
 CSRC = os.path.join(_HERE, "csrc")
 
 NUM_CUTS = 10
+EINVAL = -1         # ANCUTS_EINVAL: bad argument (also a caller graph that breaks the contract of ancuts_segment_csr_f32)
 
 # every symbol include/autoinst_ncuts.h declares
 EXPORTS = [
@@ -26,7 +27,7 @@ EXPORTS = [
     "ancuts_last_unconverged", "ancuts_set_option",
     "ancuts_merge_chunks", "ancuts_remove_semantics", "ancuts_instance_metrics", "ancuts_map_labels",
     "ancuts_last_sparse_accounting", "ancuts_dino_view_pixels", "ancuts_dino_mean",
-    "ancuts_last_reorth_accounting",
+    "ancuts_last_reorth_accounting", "ancuts_segment_csr_f32",
 ]
 
 # ancuts_set_option (include/autoinst_ncuts.h)
@@ -114,6 +115,8 @@ def load():
                                                C.c_int32, i32p, vp]
     lib.ancuts_segment_dense_f32.argtypes = [vp, C.c_int, vp, C.c_int64, C.c_int, pp, vp, i32p, sp,
                                              C.c_int32, i32p, vp]
+    lib.ancuts_segment_csr_f32.argtypes = [vp, C.c_int, i64p, vp, vp, vp, C.c_int64, i32p, pp, vp, i32p, sp,
+                                           C.c_int32, i32p, vp]
     lib.ancuts_nn_reproject.argtypes = [vp, C.c_int, vp, C.c_int, vp, vp, C.c_double, C.c_int32, vp, vp, vp]
     lib.ancuts_feature_pool_workspace_bytes.argtypes = [C.c_int]
     lib.ancuts_feature_pool_workspace_bytes.restype = C.c_int64

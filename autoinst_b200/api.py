@@ -880,3 +880,136 @@ def segment_dense(W, num_points_orig=None, *, T=0.01, split_lim=0.01, want_stats
     _report_unconverged(hd, strict)
     out = labels.cpu().numpy()
     return (out, stats[:nstats.value].copy()) if want_stats else out
+
+
+# ------------------------------------------------------------------------------------------------
+# caller-supplied sparse affinity graphs (ancuts_segment_csr_f32)
+# ------------------------------------------------------------------------------------------------
+@dataclass
+class PackedGraphs:
+    """A batch of graphs as one CSR: global int64 row pointers (P + 1), int32 columns local to each graph, float32 values."""
+    sizes: list
+    off: np.ndarray         # int64 [B + 1] first row of every graph
+    row_ptr: torch.Tensor
+    col: torch.Tensor
+    val: torch.Tensor
+
+    @property
+    def nnz(self) -> int:
+        return int(self.col.numel())
+
+    def to(self, device) -> "PackedGraphs":
+        return PackedGraphs(self.sizes, self.off, self.row_ptr.to(device), self.col.to(device), self.val.to(device))
+
+
+def _graph_shape(g):
+    shape = tuple(int(s) for s in g.shape)
+    if len(shape) != 2 or shape[0] != shape[1]:
+        raise ValueError(f"a graph must be a square matrix, got shape {shape}")
+    if shape[0] == 0:
+        raise ValueError("a graph must have at least one point")
+    return shape[0]
+
+
+def pack_graphs(graphs) -> PackedGraphs:
+    """Concatenate sparse affinity graphs into the CSR layout of ancuts_segment_csr_f32; needs no GPU.
+
+    scipy sparse input is made canonical the way `toarray()` reads it: duplicates are summed in the input dtype, then the
+    values are rounded to float32 (what `toarray().astype(np.float32)` holds); explicit zeros stay (a stored 0 is no edge).
+    torch sparse-CSR input is taken as it is (the library validates it) and stays on its device: the row pointers are offset
+    and the columns narrowed there, without a round trip through the host.  Non-square and empty graphs raise ValueError."""
+    graphs = list(graphs)
+    if not graphs:
+        raise ValueError("no graphs")
+    sizes = [_graph_shape(g) for g in graphs]
+    parts = []
+    dev = None
+    for g in graphs:
+        if isinstance(g, torch.Tensor):
+            if g.layout != torch.sparse_csr:
+                raise TypeError("torch graphs must be sparse-CSR tensors (Tensor.to_sparse_csr())")
+            if g.is_cuda:
+                dev = dev or g.device
+            parts.append((g.crow_indices().to(torch.int64), g.col_indices().to(torch.int32), g.values().to(torch.float32)))
+        elif hasattr(g, "tocsr"):
+            m = g.tocsr(copy=True)
+            m.sum_duplicates()
+            parts.append((torch.from_numpy(np.asarray(m.indptr, dtype=np.int64)),
+                          torch.from_numpy(np.asarray(m.indices, dtype=np.int32)),
+                          torch.from_numpy(np.asarray(m.data).astype(np.float32))))
+        else:
+            raise TypeError("graphs must be scipy sparse matrices or torch sparse-CSR tensors")
+    dev = dev or torch.device("cpu")
+    rows, cols, vals = [], [], []
+    e0 = 0
+    for rp, cl, vl in parts:
+        rp, cl, vl = rp.to(dev), cl.to(dev), vl.to(dev)
+        rows.append(rp[:-1] + e0)
+        cols.append(cl)
+        vals.append(vl)
+        e0 += int(cl.numel())
+    rows.append(torch.full((1,), e0, dtype=torch.int64, device=dev))
+    off = np.zeros(len(sizes) + 1, dtype=np.int64)
+    off[1:] = np.cumsum(sizes)
+    return PackedGraphs(sizes, off, torch.cat(rows).contiguous(), torch.cat(cols).contiguous(), torch.cat(vals).contiguous())
+
+
+def _run_graphs(hd, pk: PackedGraphs, norig, p, want_stats, device):
+    B = len(pk.sizes)
+    off = np.ascontiguousarray(pk.off, dtype=np.int64)
+    nseg = np.zeros(B, dtype=np.int32)
+    cap = 128 * B + 64 if want_stats else 0
+    stats = np.zeros(max(cap, 1), dtype=_STAT_DTYPE)
+    nstats = C.c_int32(0)
+    labels = torch.empty(int(off[-1]), dtype=torch.int32, device=device)
+    no = None if norig is None else np.ascontiguousarray(norig, dtype=np.int32)
+    with torch.cuda.device(device):
+        check(hd.lib.ancuts_segment_csr_f32(
+            hd.h, B, off.ctypes.data_as(C.POINTER(C.c_int64)), _ptr(pk.row_ptr), _ptr(pk.col), _ptr(pk.val), pk.nnz,
+            no.ctypes.data_as(C.POINTER(C.c_int32)) if no is not None else None, C.byref(p), _ptr(labels),
+            nseg.ctypes.data_as(C.POINTER(C.c_int32)), stats.ctypes.data_as(C.POINTER(NodeStat)) if want_stats else None,
+            cap, C.byref(nstats), _stream(device)))
+    arr = labels.cpu().numpy()
+    return [arr[a:b].copy() for a, b in zip(off[:-1], off[1:])], nseg, (stats[:nstats.value].copy() if want_stats else None)
+
+
+def segment_graphs(graphs, *, num_points_orig=None, T=0.01, split_lim=0.01, device=None, want_stats=False, max_steps=0,
+                   tol=0.0, strict: bool = False, memory_budget=None, lane: int = 0) -> SegmentResult:
+    """normalized_cut(w, num_points_orig, labels, T, split_lim) (normalized_cut.py:37-63) for a list of sparse affinity
+    graphs (scipy sparse matrices or torch sparse-CSR tensors, host or device), batched to fit device memory like
+    `segment_chunks`.  Every graph must be symmetric with a unit diagonal (stored diagonal entries exactly 1, absent ones
+    taken as 1) and finite; a violation raises naming the graph and the row.  The labels equal `segment_dense` on the
+    densified graph.  num_points_orig: None (each graph's own size), one int for all graphs, or one per graph."""
+    device = _dev(device)
+    hd = Handle.get(device, lane)
+    graphs = list(graphs)
+    sizes = [_graph_shape(g) for g in graphs]
+    if num_points_orig is None:
+        norig = None
+    elif np.ndim(num_points_orig) == 0:
+        norig = [int(num_points_orig)] * len(graphs)
+    else:
+        norig = [int(x) for x in num_points_orig]
+        if len(norig) != len(graphs):
+            raise ValueError("num_points_orig needs one value per graph")
+    if memory_budget is None:
+        free, _total = torch.cuda.mem_get_info(device)
+        memory_budget = int(free * 0.7)
+    p = make_params(T=T, split_lim=split_lim, max_steps=max_steps, tol=tol)
+    labels = [None] * len(sizes)
+    nseg = np.zeros(len(sizes), dtype=np.int32)
+    stats_all = []
+    unconv = 0
+    for batch in plan_batches(sizes, memory_budget, max_steps):
+        pk = pack_graphs([graphs[i] for i in batch]).to(device)
+        lab, ns, st = _run_graphs(hd, pk, None if norig is None else [norig[i] for i in batch], p, want_stats, device)
+        unconv += _report_unconverged(hd, strict)
+        for j, i in enumerate(batch):
+            labels[i] = lab[j]
+            nseg[i] = ns[j]
+        if want_stats and st is not None:
+            st = st.copy()
+            st["chunk"] = np.asarray(batch, dtype=np.int32)[st["chunk"]]
+            stats_all.append(st)
+    stats = np.concatenate(stats_all) if stats_all else None
+    return SegmentResult(labels=labels, num_segments=nseg, stats=stats, unconverged=unconv)

@@ -13,6 +13,7 @@
 #include "kernels_cluster.cuh"
 #include "kernels_pool.cuh"
 #include "kernels_dino.cuh"
+#include "kernels_csr.cuh"
 
 namespace ancuts {
 
@@ -80,6 +81,8 @@ struct Plan {
     int* c_tile0 = nullptr; double* tbox = nullptr; long long* d_qoff = nullptr; int* d_qcap = nullptr;          // cell-sorted sweep
     std::vector<int> tile0; int max_tiles = 0;
     bool grid_pairs = false;
+    bool csr = false;                      // caller graphs in CSR form (ancuts_segment_csr_f32)
+    unsigned long long* csr_err = nullptr; int* csr_out = nullptr;      // k_csr_validate: first violation per graph, range flag
     ancuts_node_stat* stats;
     Eng e{};            // zero: optional pointers (sel, unfused, dbg, stats) are NULL unless a call sets them
 };
@@ -183,6 +186,8 @@ static size_t layout(Plan& pl, char* base, int stats_cap, int tdim, int ddim, bo
             pl.d_qcap = ar.take<int>((size_t)B);
         }
     }
+    pl.csr_err = nullptr; pl.csr_out = nullptr;
+    if (pl.csr) { pl.csr_err = ar.take<unsigned long long>(B); pl.csr_out = ar.take<int>(1); }
     pl.hW0.assign(B, nullptr); pl.hW1.assign(B, nullptr);
     if (pl.own_w0) for (int c = 0; c < B; ++c) pl.hW0[c] = ar.take<float>((size_t)pl.n[c] * pl.ld[c]);
     if (pl.own_w1) for (int c = 0; c < B; ++c) pl.hW1[c] = ar.take<float>((size_t)pl.n[c] * pl.ld[c]);
@@ -654,6 +659,10 @@ struct DeferredAffinity {
     const int64_t* chunk_off;
     const cudaEvent_t* feat_ev;    // host entry with the batched pair stage: chunk c's features have arrived at feat_ev[c]
     const int* order;              // batched pair stage: the queue holds cell-sorted ranks, order[base + rank] = input index
+    // caller graphs (ancuts_segment_csr_f32): the stored entries take the place of the queued pairs
+    const int64_t* row_ptr = nullptr;
+    const int32_t* col = nullptr;
+    const float* val = nullptr;
 };
 
 static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int max_split_n, bool components,
@@ -706,6 +715,16 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
         // and scatter the queued pairs of every chunk to the positions their points have now.
         LAUNCH(SG_AFFINITY, k_zero_blocks<<<dim3(ZB_BLOCKS, num_active), 256, 0, st>>>(e, cur));
         LAUNCH(SG_PARTITION, k_inverse_positions<<<gP, tb, 0, st>>>(e, e.val));
+        if (df->row_ptr) {
+            // caller graphs: one pass over every graph's rows in input order
+            int nmax = 0;
+            for (int c = 0; c < e.B; ++c) nmax = std::max(nmax, pl.n[c]);
+            dim3 g((nmax + 256 / CSR_LANES - 1) / (256 / CSR_LANES), e.B);
+            LAUNCH(SG_AFFINITY, k_csr_scatter<<<g, 256, 0, st>>>(e, cur, df->row_ptr, df->col, df->val, e.val));
+            ANCUTS_CUDA(cudaGetLastError());
+            cur ^= 1;
+            return ANCUTS_OK;
+        }
         const ancuts_params* p = df->p;
         const bool use_tarl = p->theta != 0.0 && df->tarl, use_dino = p->gamma != 0.0 && df->dino;
         for (int c = 0; c < e.B; ++c) {
@@ -1429,10 +1448,73 @@ int ancuts_dino_mean(ancuts_handle* h, int num_major, int num_views, const int32
     return ANCUTS_OK;
 }
 
+// caller graphs of ancuts_segment_csr_f32 (one concatenated CSR, columns local to the row's graph)
+struct CsrInput {
+    const int64_t* row_ptr;
+    const int32_t* col;
+    const float* val;
+    int64_t nnz;
+    const int32_t* norig;      // per graph, or NULL
+};
+
+static const char* csr_rule(int kind) {
+    switch (kind) {
+        case CSR_ROWPTR: return "row_ptr decreases or leaves [0, nnz]";
+        case CSR_ROWPTR_ENDS: return "row_ptr[0] != 0 or row_ptr[P] != nnz";
+        case CSR_COLUMN: return "column outside [0, n)";
+        case CSR_UNSORTED: return "columns not in increasing order";
+        case CSR_DUPLICATE: return "duplicate column";
+        case CSR_NONFINITE: return "non-finite value";
+        case CSR_DIAGONAL: return "stored diagonal entry is not 1";
+        case CSR_NO_MIRROR: return "not symmetric: entry (i, j) without entry (j, i)";
+        case CSR_ASYMMETRIC: return "not symmetric: value of (i, j) differs from (j, i)";
+        default: return "unknown";
+    }
+}
+
+// Input stage of a CSR call: validation, the w_own rule, root-level components.  The points path's pair stage ends at
+// the same state (forest in e.parent, W written after the root split by run_rebuild's deferred branch).
+static int run_csr_front(ancuts_handle* h, Plan& pl, const CsrInput& csr, cudaStream_t st) {
+    const int B = pl.B;
+    int nmax = 0;
+    for (int c = 0; c < B; ++c) nmax = std::max(nmax, pl.n[c]);
+    const dim3 g((nmax + 256 / CSR_LANES - 1) / (256 / CSR_LANES), B);
+    ANCUTS_CUDA(cudaMemsetAsync(pl.csr_err, 0xff, (size_t)B * sizeof(unsigned long long), st));
+    ANCUTS_CUDA(cudaMemsetAsync(pl.csr_out, 0, sizeof(int), st));
+    LAUNCH(SG_AFFINITY, k_csr_validate<<<g, 256, 0, st>>>(pl.c_base, pl.c_n, pl.P, csr.row_ptr, csr.col, csr.val,
+                                                          (long long)csr.nnz, pl.csr_err, pl.csr_out));
+    ANCUTS_CUDA(cudaGetLastError());
+    std::vector<unsigned long long> herr(B);
+    int outside = 0;
+    ANCUTS_CUDA(cudaMemcpyAsync(herr.data(), pl.csr_err, (size_t)B * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    ANCUTS_CUDA(cudaMemcpyAsync(&outside, pl.csr_out, sizeof(int), cudaMemcpyDeviceToHost, st));
+    ANCUTS_CUDA(cudaStreamSynchronize(st));
+    for (int c = 0; c < B; ++c) {
+        if (herr[c] == ~0ull) continue;
+        const int kind = (int)(herr[c] & 0xff), row = (int)((herr[c] >> 8) & 0x3fffffffu);
+        set_error("graph %d, row %d: %s", c, row, csr_rule(kind));
+        return ANCUTS_EINVAL;
+    }
+    // Every stored value in {0} U [2^-126, 2), the range of the library's own affinities: the default forms of the points
+    // path apply (shared-memory CSR slices, fused cut, integer widening).  The widening is exact for +0 and positive
+    // normal floats; the fixed-point cut sums need non-negative weights (a node's volume bounds its cut weights).
+    // Otherwise the plain widening and separate cut kernels, as segment_dense.
+    pl.e.w_own = outside ? 0 : 1;
+    LAUNCH(SG_PARTITION, k_cc_init<<<(pl.P + 255) / 256, 256, 0, st>>>(pl.e));
+    LAUNCH(SG_AFFINITY, k_csr_unions<<<g, 256, 0, st>>>(pl.c_base, pl.c_n, csr.row_ptr, csr.col, csr.val, pl.e.parent));
+    ANCUTS_CUDA(cudaGetLastError());
+    // algorithmic bytes of validation, unions and scatter: row pointers 8 B per row three times; per stored entry its column
+    // and value (8 B) in each of the three passes, the mirror entry's (8 B) in the validation, the position of the column's
+    // point (4 B) and the store (4 B) in the scatter
+    h->stage_bytes[SG_AFFINITY] = 24.0 * pl.P + 40.0 * (double)csr.nnz;
+    return ANCUTS_OK;
+}
+
 static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off, const double* d_points,
                           const float* d_tarl, const float* d_dino, const float* d_W_dense, int64_t ld_dense,
                           int num_points_orig, const ancuts_params* p, int32_t* d_labels, int32_t* h_num_segments,
-                          ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats, cudaStream_t st) {
+                          ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats, cudaStream_t st,
+                          const CsrInput* csr = nullptr) {
     const cudaEvent_t* wait_ev = h ? h->wait_ev : nullptr;      // per-chunk "inputs have arrived" events of the host entry point
     if (h) h->wait_ev = nullptr;                                 // consumed by this call
     struct EvReset { ancuts_handle* h; ~EvReset() { if (h) { h->ev_points = nullptr; h->feat_ev = nullptr; } } } ev_reset{h};
@@ -1446,22 +1528,27 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
         if (d <= 0 || d > (1 << 28)) { set_error("chunk %d has %lld points", c, (long long)d); return ANCUTS_EINVAL; }
         n[c] = (int)d;
         norig[c] = (d_W_dense && num_points_orig > 0) ? num_points_orig : (int)d;
+        if (csr && csr->norig) {
+            if (csr->norig[c] <= 0) { set_error("graph %d: num_points_orig %d must be positive", c, csr->norig[c]); return ANCUTS_EINVAL; }
+            norig[c] = csr->norig[c];
+        }
     }
     if (h_chunk_off[num_chunks] - h_chunk_off[0] > 0x7fffffffLL / 4) { set_error("batch too large"); return ANCUTS_EINVAL; }
     const int kmax = resolve_kmax(p);
     Plan pl;
     make_plan(pl, num_chunks, n.data(), norig.data(), nullptr, kmax, 0);
     if (stats_cap < 0) stats_cap = 0;
-    const bool need_tc = (p->affinity_impl == 1) && !d_W_dense;
+    const bool need_tc = (p->affinity_impl == 1) && !d_W_dense && !csr;
     const bool feats = (p->theta != 0.0 && d_tarl) || (p->gamma != 0.0 && d_dino);
     const int aform = h->opt[ANCUTS_OPT_AFFINITY_FORM];        // 0 deferred (default), 1 dense two-pass, 2 dense one-kernel
     (void)feats;                                               // spatial-only configs take the deferred form too (pass 2 = exp(-alpha d))
-    pl.want_pairq = !d_W_dense && p->affinity_impl == 0 && aform != 2;
+    pl.want_pairq = !d_W_dense && !csr && p->affinity_impl == 0 && aform != 2;
+    pl.csr = csr != nullptr;
     pl.deferred = pl.want_pairq && aform == 0;                 // W written block by block after the root split
     pl.grid_pairs = pl.deferred && h->opt[ANCUTS_OPT_PAIR_SEARCH] == 0;     // cell-sorted, batched sweep (default) or the shuffled one
     if (pl.grid_pairs) ANCUTS_CUDA(cudaFuncSetAttribute(k_pair_grid_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(PG_CELLS * sizeof(int))));
-    bool root_forest = pl.want_pairq;
-    bool deferred = pl.deferred;
+    bool root_forest = pl.want_pairq || pl.csr;     // CSR: k_csr_unions builds the forest, W is written after the root split
+    bool deferred = pl.deferred || pl.csr;
     size_t bytes = layout(pl, nullptr, stats_cap, p->tarl_dim, p->dino_dim, need_tc);
     rc = ensure_ws(h, bytes);
     if (rc) return rc;
@@ -1470,9 +1557,9 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     if (rc) return rc;
     fill_params(pl.e, p, kmax);
     pl.e.dbg = h->dbg;
-    pl.e.pts = d_W_dense ? nullptr : d_points;
+    pl.e.pts = (d_W_dense || csr) ? nullptr : d_points;      // caller weights: hash start vector
     pl.e.w_guard = 0;                         // every node block is written by k_gather_blocks_cur (fringe zeroed)
-    pl.e.w_own = d_W_dense ? 0 : 1;           // caller-provided weights may be negative or denormal: plain widening
+    pl.e.w_own = d_W_dense ? 0 : 1;           // caller-provided weights may be negative or denormal: plain widening (CSR: run_csr_front)
     pl.e.stats = (h_stats && stats_cap > 0) ? pl.stats : nullptr;
     pl.e.stats_cap = stats_cap;
     rc = set_attrs(h, pl.KS);
@@ -1483,6 +1570,9 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     if (d_W_dense) {
         ANCUTS_CUDA(cudaMemcpy2DAsync(pl.hW0[0], (size_t)pl.ld[0] * 4, d_W_dense, (size_t)ld_dense * 4, (size_t)n[0] * 4,
                                       n[0], cudaMemcpyDeviceToDevice, st));
+    } else if (csr) {
+        rc = run_csr_front(h, pl, *csr, st);
+        if (rc) return rc;
     } else {
         double aff_bytes = 0.0;
         if (pl.qctr) {
@@ -1535,6 +1625,7 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     }
     DeferredAffinity df{p, d_tarl, d_dino, h_chunk_off, (deferred && pl.grid_pairs) ? h->feat_ev : nullptr,
                         (deferred && pl.grid_pairs) ? pl.pg_sorted : nullptr};
+    if (csr) { df.row_ptr = csr->row_ptr; df.col = csr->col; df.val = csr->val; }
     rc = run_levels(h, pl, p, 0, d_labels, h_num_segments, st, root_forest, deferred ? &df : nullptr);
     if (rc) return rc;
     rc = copy_stats(h, pl, h_stats, stats_cap, h_num_stats, st);
@@ -1560,6 +1651,17 @@ int ancuts_segment_dense_f32(ancuts_handle* h, int n, const float* d_W, int64_t 
     int64_t off[2] = {0, n};
     return segment_common(h, 1, off, nullptr, nullptr, nullptr, d_W, ld, num_points_orig, p, d_labels,
                           h_num_segments, h_stats, stats_cap, h_num_stats, (cudaStream_t)stream);
+}
+
+int ancuts_segment_csr_f32(ancuts_handle* h, int num_graphs, const int64_t* h_graph_off, const int64_t* d_row_ptr,
+                           const int32_t* d_col, const float* d_val, int64_t nnz, const int32_t* h_num_points_orig,
+                           const ancuts_params* p, int32_t* d_labels, int32_t* h_num_segments, ancuts_node_stat* h_stats,
+                           int32_t stats_cap, int32_t* h_num_stats, void* stream) {
+    if (!d_row_ptr || nnz < 0 || (nnz > 0 && (!d_col || !d_val))) { set_error("bad argument to ancuts_segment_csr_f32"); return ANCUTS_EINVAL; }
+    if (h_graph_off && h_graph_off[0] != 0) { set_error("h_graph_off[0] must be 0"); return ANCUTS_EINVAL; }
+    CsrInput csr{d_row_ptr, d_col, d_val, nnz, h_num_points_orig};
+    return segment_common(h, num_graphs, h_graph_off, nullptr, nullptr, nullptr, nullptr, 0, 0, p, d_labels, h_num_segments,
+                          h_stats, stats_cap, h_num_stats, (cudaStream_t)stream, &csr);
 }
 
 int ancuts_segment_chunks_host(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off, const double* h_points,

@@ -145,6 +145,24 @@ int ancuts_segment_dense_f32(ancuts_handle* h, int n, const float* d_W, int64_t 
                              int32_t* h_num_segments, ancuts_node_stat* h_stats, int32_t stats_cap,
                              int32_t* h_num_stats, void* stream);
 
+/* normalized_cut(w, num_points_orig, labels, T, split_lim) (normalized_cut.py:37-63) for a BATCH of sparse
+ * affinity graphs in CSR form on the device -- the scipy CSR `w` that ncuts_utils.py:167-174 passes, or any
+ * affinity a caller builds.  Graph c owns rows [h_graph_off[c], h_graph_off[c+1]) of one concatenated CSR
+ * (h_graph_off[0] = 0): d_row_ptr has P + 1 global entry offsets (d_row_ptr[0] = 0, d_row_ptr[P] = nnz), d_col
+ * the column LOCAL to the row's graph (0 .. n_c - 1), d_val the float32 value.  The CSR is read in place.
+ * Each graph must be symmetric bit for bit (an absent entry counts as 0), have a unit diagonal (a stored diagonal
+ * entry is exactly 1.0f, an absent one is taken as 1), strictly increasing columns per row and finite values; a
+ * stored 0 is no edge.  A violation returns ANCUTS_EINVAL naming the graph, the row and the rule; no malformed
+ * d_row_ptr / d_col makes any kernel read outside the arrays.  The result is the one ancuts_segment_dense_f32
+ * gives on the densified graph.  h_num_points_orig: per-graph num_points_orig, or NULL for each graph's own
+ * size.  Of p only T, split_lim and the lanczos_* fields are read.  d_labels, h_num_segments and the stats are
+ * as in ancuts_segment_chunks (`chunk` of a record = graph index).  Blocks. */
+int ancuts_segment_csr_f32(ancuts_handle* h, int num_graphs, const int64_t* h_graph_off,
+                           const int64_t* d_row_ptr, const int32_t* d_col, const float* d_val, int64_t nnz,
+                           const int32_t* h_num_points_orig, const ancuts_params* p, int32_t* d_labels,
+                           int32_t* h_num_segments, ancuts_node_stat* h_stats, int32_t stats_cap,
+                           int32_t* h_num_stats, void* stream);
+
 /* "Next" row N1 — replaces kDTree_1NN_feature_reprojection (point_cloud_utils.py:144-174, called at
  * ncuts_utils.py:185-189): every query point (5 cm cloud) takes the label of its nearest source point
  * (0.35 m cloud).  d_source_label may be NULL (the source index is returned as label).  max_radius <= 0
