@@ -30,8 +30,8 @@ EXPORTS = [
     "ancuts_last_reorth_accounting", "ancuts_segment_csr_f32",
 ]
 
-# ancuts_set_option (include/autoinst_ncuts.h)
-OPT_AFFINITY_FORM, OPT_PAIR_SEARCH, OPT_MATVEC, OPT_CLUSTER_MAP, OPT_FUSED_CUT = 0, 1, 2, 3, 4
+# ancuts_set_option (include/autoinst_ncuts.h; option 0 is retired)
+OPT_PAIR_SEARCH, OPT_MATVEC, OPT_CLUSTER_MAP, OPT_FUSED_CUT = 1, 2, 3, 4
 PAIRS_SORTED, PAIRS_SHUFFLED = 0, 1
 MATVEC_SPARSE, MATVEC_DENSE = 0, 1
 

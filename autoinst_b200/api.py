@@ -55,10 +55,10 @@ class Handle:
         return cls._cache[key]
 
     def set_option(self, option: int, value: int):
-        """Alternative implementations behind the same results (`ancuts_set_option`): _lib.OPT_AFFINITY_FORM
-        (0 deferred, 1 dense two-pass, 2 dense one-kernel), OPT_PAIR_SEARCH (0 cell-sorted sweep, 1 shuffled sweep),
-        OPT_MATVEC (0 slices compressed into shared memory, 1 dense blocks from HBM), OPT_CLUSTER_MAP (tuning),
-        OPT_FUSED_CUT (0 the cut decision inside the sparse-form eigensolver kernel, 1 as its own kernels)."""
+        """Alternative implementations behind the same results (`ancuts_set_option`): _lib.OPT_PAIR_SEARCH
+        (0 cell-sorted sweep, 1 shuffled sweep), OPT_MATVEC (0 slices compressed into shared memory, 1 dense blocks
+        from HBM), OPT_CLUSTER_MAP (tuning), OPT_FUSED_CUT (0 the cut decision inside the sparse-form eigensolver kernel,
+        1 as its own kernels).  Option 0 is retired and raises."""
         check(self.lib.ancuts_set_option(self.h, int(option), int(value)))
 
     def sparse_accounting(self) -> dict:

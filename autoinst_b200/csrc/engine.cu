@@ -72,9 +72,9 @@ struct Plan {
     uint8_t* tarl_zero;
     void* cub_tmp;
     void* tc_scratch; size_t tc_scratch_bytes = 0;
-    PairQ* pairq = nullptr; int qcap = 0; int* qctr = nullptr;     // two-pass affinity: pair queue, [2c]=count [2c+1]=overflow
-    bool want_pairq = false;
-    bool deferred = false;                 // per-chunk pair queues kept until the root split (deferred affinity)
+    PairQ* pairq = nullptr; int* qctr = nullptr;     // pair queue, [2c]=count [2c+1]=overflow
+    int qcap = 0;                          // stage entry (ancuts_affinity_f32): capacity of its single queue
+    bool deferred = false;                 // points input: per-chunk pair queues kept until the root split (deferred affinity)
     std::vector<size_t> qoff;              // deferred: first queue entry of chunk c
     std::vector<int> qcap_c;               // deferred: queue capacity of chunk c
     int* pg_cells = nullptr; int* pg_sorted = nullptr; int* pg_tmp = nullptr; double* pg_spts = nullptr; PairGrid* pg_grid = nullptr;   // deferred: cell grids of the pair search
@@ -149,42 +149,34 @@ static size_t layout(Plan& pl, char* base, int stats_cap, int tdim, int ddim, bo
         pl.tc_scratch_bytes = affinity_tc_scratch_bytes(nmax, tdim, ddim);
         pl.tc_scratch = ar.take<char>(pl.tc_scratch_bytes);
     }
-    pl.pairq = nullptr; pl.qcap = 0; pl.qctr = nullptr;
-    if (pl.want_pairq) {
-        int nmax = 0;
-        for (int c = 0; c < B; ++c) nmax = std::max(nmax, pl.n[c]);
-        pl.qcap = (int)std::min<long long>(96ll * nmax, (long long)nmax * (nmax - 1) / 2 + 1);
-        size_t total = (size_t)pl.qcap;
-        pl.qoff.assign(B, 0); pl.qcap_c.assign(B, pl.qcap);
-        if (pl.deferred) {
-            total = 0;
-            for (int c = 0; c < B; ++c) {
-                const long long nc = pl.n[c];
-                pl.qoff[c] = total;
-                pl.qcap_c[c] = (int)std::min<long long>(96ll * nc, nc * (nc - 1) / 2 + 1);
-                total += (size_t)pl.qcap_c[c];
-            }
+    pl.pairq = nullptr; pl.qctr = nullptr;
+    if (pl.deferred) {
+        size_t total = 0;
+        pl.qoff.assign(B, 0); pl.qcap_c.assign(B, 0);
+        for (int c = 0; c < B; ++c) {
+            const long long nc = pl.n[c];
+            pl.qoff[c] = total;
+            pl.qcap_c[c] = (int)std::min<long long>(96ll * nc, nc * (nc - 1) / 2 + 1);
+            total += (size_t)pl.qcap_c[c];
         }
         pl.pairq = ar.take<PairQ>(total);
         pl.qctr = ar.take<int>(2 * (size_t)B);
-        if (pl.deferred) {
-            pl.pg_cells = ar.take<int>((size_t)B * PG_STRIDE);
-            pl.pg_sorted = ar.take<int>((size_t)P);
-            pl.pg_tmp = ar.take<int>((size_t)P);
-            pl.pg_spts = ar.take<double>((size_t)P * 3);
-            pl.pg_grid = ar.take<PairGrid>((size_t)B);
-            pl.tile0.assign(B + 1, 0);
-            pl.max_tiles = 0;
-            for (int c = 0; c < B; ++c) {
-                const int t = (pl.n[c] + PS_T - 1) / PS_T;
-                pl.tile0[c + 1] = pl.tile0[c] + t;
-                pl.max_tiles = std::max(pl.max_tiles, t);
-            }
-            pl.c_tile0 = ar.take<int>((size_t)B + 1);
-            pl.tbox = ar.take<double>((size_t)pl.tile0[B] * 6);
-            pl.d_qoff = ar.take<long long>((size_t)B);
-            pl.d_qcap = ar.take<int>((size_t)B);
+        pl.pg_cells = ar.take<int>((size_t)B * PG_STRIDE);
+        pl.pg_sorted = ar.take<int>((size_t)P);
+        pl.pg_tmp = ar.take<int>((size_t)P);
+        pl.pg_spts = ar.take<double>((size_t)P * 3);
+        pl.pg_grid = ar.take<PairGrid>((size_t)B);
+        pl.tile0.assign(B + 1, 0);
+        pl.max_tiles = 0;
+        for (int c = 0; c < B; ++c) {
+            const int t = (pl.n[c] + PS_T - 1) / PS_T;
+            pl.tile0[c + 1] = pl.tile0[c] + t;
+            pl.max_tiles = std::max(pl.max_tiles, t);
         }
+        pl.c_tile0 = ar.take<int>((size_t)B + 1);
+        pl.tbox = ar.take<double>((size_t)pl.tile0[B] * 6);
+        pl.d_qoff = ar.take<long long>((size_t)B);
+        pl.d_qcap = ar.take<int>((size_t)B);
     }
     pl.csr_err = nullptr; pl.csr_out = nullptr;
     if (pl.csr) { pl.csr_err = ar.take<unsigned long long>(B); pl.csr_out = ar.take<int>(1); }
@@ -377,11 +369,8 @@ static int resolve_kmax(const ancuts_params* p) {
     return std::min(std::max(k, 2), KMAX_LIMIT);
 }
 
-// qctr != NULL selects the two-pass form (feature terms only); parent != NULL additionally records the root-level
-// connected components (positions pos0 + i) while the pairs are at hand
-static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, const float* tarl, const float* dino,
-                        const ancuts_params* p, float* W, long long ld, uint8_t* tarl_zero, cudaStream_t st,
-                        int* qctr = nullptr, int* parent = nullptr, int pos0 = 0, int defer_chunk = -1) {
+// feature inputs of an affinity call (stage entry, points input of the segment path)
+static int check_features(const ancuts_params* p, const float* tarl, const float* dino) {
     const bool use_tarl = p->theta != 0.0 && tarl != nullptr;
     const bool use_dino = p->gamma != 0.0 && dino != nullptr;
     if (p->theta != 0.0 && tarl == nullptr) { set_error("theta != 0 but no TARL features"); return ANCUTS_EINVAL; }
@@ -393,6 +382,16 @@ static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, co
         set_error("feature dimensions must be positive multiples of 4 (got %d, %d)", p->tarl_dim, p->dino_dim);
         return ANCUTS_EUNSUPPORTED;
     }
+    return ANCUTS_OK;
+}
+
+// W of one chunk written whole (inputs checked by check_features).  qctr != NULL selects the two-pass form of the stage
+// entry (feature terms only): pairs into the single queue pl.pairq, then the feature pass.
+static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, const float* tarl, const float* dino,
+                        const ancuts_params* p, float* W, long long ld, uint8_t* tarl_zero, cudaStream_t st,
+                        int* qctr = nullptr) {
+    const bool use_tarl = p->theta != 0.0 && tarl != nullptr;
+    const bool use_dino = p->gamma != 0.0 && dino != nullptr;
     if (use_tarl)
         LAUNCH(SG_AFFINITY, k_zero_rows<<<(n + 7) / 8, 256, 0, st>>>(n, tarl, p->tarl_dim, tarl_zero));
     if (p->affinity_impl == 1 && (use_tarl || use_dino)) {
@@ -404,16 +403,8 @@ static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, co
     } else if (qctr) {
         // two-pass form: distances + zero fill + pair queue, then the queued pairs spread over the whole grid
         dim3 grid((unsigned)((ld + AT - 1) / AT), (n + AT - 1) / AT);
-        if (defer_chunk >= 0) {
-            // deferred: pairs and root-level components only; W is written after the root split (run_rebuild)
-            LAUNCH(SG_AFFINITY, k_affinity_pairs<<<grid, 256, 0, st>>>(n, pts, p->alpha, p->proximity, nullptr, ld,
-                                                                       pl.pairq + pl.qoff[defer_chunk], pl.qcap_c[defer_chunk],
-                                                                       qctr, parent, pos0));
-            ANCUTS_CUDA(cudaGetLastError());
-            return ANCUTS_OK;
-        }
         LAUNCH(SG_AFFINITY, k_affinity_pairs<<<grid, 256, 0, st>>>(n, pts, p->alpha, p->proximity, W, ld, pl.pairq, pl.qcap, qctr,
-                                                                   parent, pos0));
+                                                                   nullptr, 0));
         LAUNCH(SG_AFFINITY, k_affinity_feats<<<148 * 4, 256, 0, st>>>(pl.pairq, qctr, pl.qcap, use_tarl ? tarl : nullptr, p->tarl_dim,
                                                                         use_dino ? dino : nullptr, p->dino_dim, tarl_zero, p->theta,
                                                                         p->gamma, W, ld));
@@ -657,7 +648,7 @@ struct DeferredAffinity {
     const float* tarl;      // all chunks, input order
     const float* dino;
     const int64_t* chunk_off;
-    const cudaEvent_t* feat_ev;    // host entry with the batched pair stage: chunk c's features have arrived at feat_ev[c]
+    const cudaEvent_t* feats;      // host entry: chunk c's features have arrived at feats[c], else NULL
     const int* order;              // batched pair stage: the queue holds cell-sorted ranks, order[base + rank] = input index
     // caller graphs (ancuts_segment_csr_f32): the stored entries take the place of the queued pairs
     const int64_t* row_ptr = nullptr;
@@ -666,13 +657,14 @@ struct DeferredAffinity {
 };
 
 static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int max_split_n, bool components,
-                       cudaStream_t st, int* class_cnt = nullptr, int* big_cnt = nullptr, bool forest_ready = false,
+                       cudaStream_t st, int* class_cnt = nullptr, int* big_cnt = nullptr,
                        const DeferredAffinity* df = nullptr, bool forest_inited = false) {
     Eng& e = pl.e;
     const int P = e.P;
     const int tb = 256, gP = (P + tb - 1) / tb;
-    // forest_ready: the affinity pass already joined every in-mask pair of the (root) ranges in e.parent
+    // forest_ready (deferred affinity): the input stage already joined every in-mask pair of the root ranges in e.parent
     // forest_inited: the level loop reset the forest before the Lanczos launch (the fused cut joins components into it)
+    const bool forest_ready = df != nullptr;
     if (!forest_ready && !forest_inited) LAUNCH(SG_PARTITION, k_cc_init<<<gP, tb, 0, st>>>(e));
     if (!forest_ready && components && num_split > 0) {
         dim3 g((max_split_n + 7) / 8, num_split);
@@ -730,8 +722,8 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
         for (int c = 0; c < e.B; ++c) {
             const size_t o = (size_t)df->chunk_off[c];
             float* dst = cur ? pl.hW0[c] : pl.hW1[c];
-            if (df->feat_ev) {
-                ANCUTS_CUDA(cudaStreamWaitEvent(st, df->feat_ev[c], 0));
+            if (df->feats) {
+                ANCUTS_CUDA(cudaStreamWaitEvent(st, df->feats[c], 0));
                 if (use_tarl)
                     LAUNCH(SG_AFFINITY, k_zero_rows<<<(pl.n[c] + 7) / 8, 256, 0, st>>>(pl.n[c], df->tarl + o * p->tarl_dim, p->tarl_dim,
                                                                                       pl.tarl_zero + (o - (size_t)df->chunk_off[0])));
@@ -753,10 +745,10 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
     return ANCUTS_OK;
 }
 
-// the whole recursion for the chunks described by the plan; W of every chunk is in buffer `cur`
+// the whole recursion for the chunks described by the plan; W of every chunk is in buffer `cur`, or, with df, written
+// after the root split from the root-level forest the input stage built
 static int run_levels(ancuts_handle* h, Plan& pl, const ancuts_params* p, int cur, int32_t* d_labels,
-                      int32_t* h_num_segments, cudaStream_t st, bool root_forest_ready = false,
-                      const DeferredAffinity* df = nullptr) {
+                      int32_t* h_num_segments, cudaStream_t st, const DeferredAffinity* df = nullptr) {
     Eng& e = pl.e;
     const int P = e.P, B = e.B;
     ANCUTS_CUDA(cudaMemsetAsync(e.ctr, 0, CTR_COUNT * sizeof(int), st));
@@ -775,8 +767,8 @@ static int run_levels(ancuts_handle* h, Plan& pl, const ancuts_params* p, int cu
     bool all_fused = false;            // previous level: every node joined its components inside the cluster kernel
     while (num_split > 0) {
         int class_cnt[CL_CLASSES] = {0}, big_cnt = 0;
-        rc = run_rebuild(h, pl, cur, num_split, max_split_n, !all_fused, st, class_cnt, &big_cnt, root_forest_ready && guard == 0,
-                         guard == 0 ? df : nullptr, guard > 0);
+        rc = run_rebuild(h, pl, cur, num_split, max_split_n, !all_fused, st, class_cnt, &big_cnt, guard == 0 ? df : nullptr,
+                         guard > 0);
         if (rc) return rc;
         int num_active = h->h_ctr[1], max_n = h->h_ctr[2];
         if (num_active == 0) break;
@@ -881,6 +873,7 @@ int ancuts_create(int device, ancuts_handle** out) {
     }
     ANCUTS_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     ANCUTS_CUDA(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
+    ANCUTS_CUDA(cudaEventCreateWithFlags(&h->points_ev, cudaEventDisableTiming));
     ANCUTS_CUDA(cudaMallocHost((void**)&h->h_acct, SG_ACCT * sizeof(unsigned long long)));
     *out = h;
     return ANCUTS_OK;
@@ -895,7 +888,7 @@ int ancuts_destroy(ancuts_handle* h) {
     if (h->post_ws) cudaFree(h->post_ws);
     if (h->h_post) cudaFreeHost(h->h_post);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    for (int i = 0; i < 2; ++i) if (h->ev_host[i]) cudaEventDestroy(h->ev_host[i]);
+    if (h->points_ev) cudaEventDestroy(h->points_ev);
     for (auto ev : h->copy_ev) cudaEventDestroy(ev);
     if (h->h_ctr) cudaFreeHost(h->h_ctr);
     if (h->h_acct) cudaFreeHost(h->h_acct);
@@ -911,8 +904,7 @@ int64_t ancuts_segment_workspace_bytes(int num_chunks, const int32_t* h_chunk_n,
     Plan pl;
     int kmax = lanczos_max_steps > 0 ? lanczos_max_steps : KMAX_DEFAULT;
     make_plan(pl, num_chunks, h_chunk_n, nullptr, nullptr, kmax, 0);
-    pl.want_pairq = true;                              // upper bound: tensor-core scratch and pair queue both counted
-    pl.deferred = true;
+    pl.deferred = true;                                // upper bound: tensor-core scratch and pair queues both counted
     return (int64_t)layout(pl, nullptr, 1 << 16, 96, 384, true);
 }
 
@@ -947,6 +939,10 @@ int ancuts_debug_phases(ancuts_handle* h, double* out32, int reset) {
 
 int ancuts_set_option(ancuts_handle* h, int option, int value) {
     if (!h || option < 0 || option >= ANCUTS_OPT_COUNT) { set_error("unknown option %d", option); return ANCUTS_EINVAL; }
+    if (option == 0) {
+        set_error("option 0 is retired (it selected a dense affinity form of the segment path)");
+        return ANCUTS_EINVAL;
+    }
     h->opt[option] = value;
     return ANCUTS_OK;
 }
@@ -987,13 +983,14 @@ int ancuts_affinity_f32(ancuts_handle* h, int n, const double* d_points, const f
                         const ancuts_params* p, float* d_W, int64_t ld, double* d_rowsum, void* stream) {
     if (!h || n <= 0 || !d_points || !d_W || ld < n || (ld % 4)) { set_error("bad argument to ancuts_affinity_f32"); return ANCUTS_EINVAL; }
     int rc = check_params(p);
+    if (!rc) rc = check_features(p, d_tarl, d_dino);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     ANCUTS_CUDA(cudaSetDevice(h->device));
     Plan pl;
     size_t tcb = (p->affinity_impl == 1) ? affinity_tc_scratch_bytes(n, p->tarl_dim, p->dino_dim) : 0;
     const bool feats = (p->theta != 0.0 && d_tarl) || (p->gamma != 0.0 && d_dino);
-    const bool two_pass = p->affinity_impl == 0 && feats && h->opt[ANCUTS_OPT_AFFINITY_FORM] != 2;
+    const bool two_pass = p->affinity_impl == 0 && feats;       // spatial only: the one-kernel form
     const int qcap = two_pass ? (int)std::min<long long>(96ll * n, (long long)n * (n - 1) / 2 + 1) : 0;
     const size_t o_tc = align_up((size_t)n, 256) + 256;
     const size_t o_q = o_tc + align_up(tcb, 256) + 256;
@@ -1377,8 +1374,8 @@ int ancuts_feature_pool(ancuts_handle* h, int num_major, const double* d_major, 
 }
 
 // Pair stage of the deferred affinity for ALL chunks of the call in four launches (ANCUTS_OPT_PAIR_SEARCH = 0, the default):
-// cell sort, tile boxes, tile-pair sweep, root-level unions.  Needs the points only.
-static int run_pairs_batched(ancuts_handle* h, Plan& pl, const double* d_points, const float* d_tarl, const ancuts_params* p,
+// cell sort, tile boxes, tile-pair sweep, root-level unions.  Needs the points only; points_ev (host entry): they have arrived.
+static int run_pairs_batched(ancuts_handle* h, Plan& pl, const double* d_points, const ancuts_params* p, cudaEvent_t points_ev,
                              cudaStream_t st) {
     const int B = pl.B;
     std::vector<long long> qo(B);
@@ -1387,7 +1384,7 @@ static int run_pairs_batched(ancuts_handle* h, Plan& pl, const double* d_points,
     ANCUTS_CUDA(cudaMemcpyAsync(pl.d_qoff, qo.data(), B * sizeof(long long), cudaMemcpyHostToDevice, st));
     ANCUTS_CUDA(cudaMemcpyAsync(pl.d_qcap, pl.qcap_c.data(), B * sizeof(int), cudaMemcpyHostToDevice, st));
     ANCUTS_CUDA(cudaStreamSynchronize(st));              // qo is a local
-    if (h->ev_points) ANCUTS_CUDA(cudaStreamWaitEvent(st, h->ev_points, 0));    // host entry: the coordinates have arrived
+    if (points_ev) ANCUTS_CUDA(cudaStreamWaitEvent(st, points_ev, 0));      // after the synchronise, which so does not wait for the copy
     LAUNCH(SG_AFFINITY, k_pair_grid_b<<<B, 1024, PG_CELLS * sizeof(int), st>>>(pl.c_n, pl.c_base, d_points, p->proximity,
                                                                               pl.pg_cells, pl.pg_sorted, pl.pg_tmp, pl.pg_spts, pl.pg_grid));
     LAUNCH(SG_AFFINITY, k_tile_boxes<<<dim3(pl.max_tiles, B), PS_T, 0, st>>>(pl.c_n, pl.c_base, pl.c_tile0, pl.pg_spts, pl.tbox));
@@ -1395,10 +1392,20 @@ static int run_pairs_batched(ancuts_handle* h, Plan& pl, const double* d_points,
     LAUNCH(SG_AFFINITY, k_pair_sweep<<<dim3(npair, B), 256, 0, st>>>(pl.c_n, pl.c_base, pl.c_tile0, pl.pg_spts, pl.tbox,
                                                                      p->alpha, p->proximity, pl.pairq, pl.d_qoff, pl.d_qcap, pl.qctr));
     LAUNCH(SG_AFFINITY, k_pair_unions<<<dim3(32, B), 256, 0, st>>>(pl.pairq, pl.d_qoff, pl.d_qcap, pl.qctr, pl.c_base, pl.e.parent));
-    // host entry: the features arrive chunk by chunk while this stage and the root split run; the zero-row flags are then
-    // taken per chunk right before its feature pass (run_rebuild)
-    if (!h->feat_ev && p->theta != 0.0 && d_tarl)
-        LAUNCH(SG_AFFINITY, k_zero_rows<<<(pl.P + 7) / 8, 256, 0, st>>>(pl.P, d_tarl, p->tarl_dim, pl.tarl_zero));
+    ANCUTS_CUDA(cudaGetLastError());
+    return ANCUTS_OK;
+}
+
+// The same stage with the shuffled 64 x 64 tile sweep over each chunk's whole upper triangle (ANCUTS_OPT_PAIR_SEARCH = 1),
+// one launch per chunk that also joins the root-level components while the pairs are at hand.  Needs the points only.
+static int run_pairs_shuffled(ancuts_handle* h, Plan& pl, const double* d_points, const ancuts_params* p, cudaStream_t st) {
+    for (int c = 0; c < pl.B; ++c) {
+        const int n = pl.n[c];
+        dim3 grid((unsigned)((pl.ld[c] + AT - 1) / AT), (n + AT - 1) / AT);
+        LAUNCH(SG_AFFINITY, k_affinity_pairs<<<grid, 256, 0, st>>>(n, d_points + (size_t)pl.base[c] * 3, p->alpha, p->proximity,
+                                                                   nullptr, pl.ld[c], pl.pairq + pl.qoff[c], pl.qcap_c[c],
+                                                                   pl.qctr + 2 * c, pl.e.parent, pl.base[c]));
+    }
     ANCUTS_CUDA(cudaGetLastError());
     return ANCUTS_OK;
 }
@@ -1510,15 +1517,20 @@ static int run_csr_front(ancuts_handle* h, Plan& pl, const CsrInput& csr, cudaSt
     return ANCUTS_OK;
 }
 
+// Host entry: the inputs of the call arrive on a copy stream, the coordinates of every chunk first (points), then the
+// features chunk by chunk (feats[c]).
+struct Arrival {
+    cudaEvent_t points;
+    const cudaEvent_t* feats;
+};
+
 static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off, const double* d_points,
                           const float* d_tarl, const float* d_dino, const float* d_W_dense, int64_t ld_dense,
                           int num_points_orig, const ancuts_params* p, int32_t* d_labels, int32_t* h_num_segments,
                           ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats, cudaStream_t st,
-                          const CsrInput* csr = nullptr) {
-    const cudaEvent_t* wait_ev = h ? h->wait_ev : nullptr;      // per-chunk "inputs have arrived" events of the host entry point
-    if (h) h->wait_ev = nullptr;                                 // consumed by this call
-    struct EvReset { ancuts_handle* h; ~EvReset() { if (h) { h->ev_points = nullptr; h->feat_ev = nullptr; } } } ev_reset{h};
+                          const CsrInput* csr = nullptr, const Arrival* arrival = nullptr) {
     int rc = check_params(p);
+    if (!rc && !d_W_dense && !csr) rc = check_features(p, d_tarl, d_dino);
     if (rc) return rc;
     if (!h || num_chunks <= 0 || !h_chunk_off || !d_labels) { set_error("bad argument to segment"); return ANCUTS_EINVAL; }
     ANCUTS_CUDA(cudaSetDevice(h->device));
@@ -1539,20 +1551,20 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     make_plan(pl, num_chunks, n.data(), norig.data(), nullptr, kmax, 0);
     if (stats_cap < 0) stats_cap = 0;
     const bool need_tc = (p->affinity_impl == 1) && !d_W_dense && !csr;
-    const bool feats = (p->theta != 0.0 && d_tarl) || (p->gamma != 0.0 && d_dino);
-    const int aform = h->opt[ANCUTS_OPT_AFFINITY_FORM];        // 0 deferred (default), 1 dense two-pass, 2 dense one-kernel
-    (void)feats;                                               // spatial-only configs take the deferred form too (pass 2 = exp(-alpha d))
-    pl.want_pairq = !d_W_dense && !csr && p->affinity_impl == 0 && aform != 2;
     pl.csr = csr != nullptr;
-    pl.deferred = pl.want_pairq && aform == 0;                 // W written block by block after the root split
+    // points input: the deferred form (spatial-only configs too: pass 2 = exp(-alpha d)) unless the tensor-core form writes W
+    pl.deferred = !d_W_dense && !csr && p->affinity_impl == 0;
     pl.grid_pairs = pl.deferred && h->opt[ANCUTS_OPT_PAIR_SEARCH] == 0;     // cell-sorted, batched sweep (default) or the shuffled one
     if (pl.grid_pairs) ANCUTS_CUDA(cudaFuncSetAttribute(k_pair_grid_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(PG_CELLS * sizeof(int))));
-    bool root_forest = pl.want_pairq || pl.csr;     // CSR: k_csr_unions builds the forest, W is written after the root split
-    bool deferred = pl.deferred || pl.csr;
     size_t bytes = layout(pl, nullptr, stats_cap, p->tarl_dim, p->dino_dim, need_tc);
     rc = ensure_ws(h, bytes);
     if (rc) return rc;
     layout(pl, h->ws, stats_cap, p->tarl_dim, p->dino_dim, need_tc);
+    // deferred != NULL: the input stage builds the root-level forest and W is written after the root split (CSR: from the
+    // stored entries); otherwise W is whole before the level loop
+    DeferredAffinity df{p, d_tarl, d_dino, h_chunk_off, arrival ? arrival->feats : nullptr, pl.grid_pairs ? pl.pg_sorted : nullptr};
+    if (csr) { df.row_ptr = csr->row_ptr; df.col = csr->col; df.val = csr->val; }
+    const DeferredAffinity* deferred = (pl.deferred || pl.csr) ? &df : nullptr;
     rc = upload_tables(pl, st);
     if (rc) return rc;
     fill_params(pl.e, p, kmax);
@@ -1574,59 +1586,50 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
         rc = run_csr_front(h, pl, *csr, st);
         if (rc) return rc;
     } else {
-        double aff_bytes = 0.0;
-        if (pl.qctr) {
+        if (pl.deferred) {
             ANCUTS_CUDA(cudaMemsetAsync(pl.qctr, 0, 2 * (size_t)num_chunks * sizeof(int), st));
             const int gP = (pl.P + 255) / 256;
             LAUNCH(SG_PARTITION, k_cc_init<<<gP, 256, 0, st>>>(pl.e));          // forest of the root-level components
-        }
-        if (pl.grid_pairs) {
-            rc = run_pairs_batched(h, pl, d_points, d_tarl, p, st);
+            if (pl.grid_pairs) {
+                rc = run_pairs_batched(h, pl, d_points, p, arrival ? arrival->points : nullptr, st);
+            } else {
+                if (arrival) ANCUTS_CUDA(cudaStreamWaitEvent(st, arrival->points, 0));
+                rc = run_pairs_shuffled(h, pl, d_points, p, st);
+            }
             if (rc) return rc;
-            for (int c = 0; c < num_chunks; ++c)
-                aff_bytes += 4.0 * n[c] * (double)n[c] +
-                             4.0 * n[c] * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? p->dino_dim : 0));
-        }
-        for (int c = 0; c < num_chunks && !pl.grid_pairs; ++c) {
-            int64_t o = h_chunk_off[c] - off0;
-            const float* tz = d_tarl ? d_tarl + (size_t)(h_chunk_off[c]) * p->tarl_dim : nullptr;
-            const float* dz = d_dino ? d_dino + (size_t)(h_chunk_off[c]) * p->dino_dim : nullptr;
-            if (wait_ev) ANCUTS_CUDA(cudaStreamWaitEvent(st, wait_ev[c], 0));       // this chunk's inputs have arrived
-            rc = run_affinity(h, pl, n[c], d_points + (size_t)h_chunk_off[c] * 3, tz, dz, p, pl.hW0[c], pl.ld[c],
-                              pl.tarl_zero + o, st, pl.qctr ? pl.qctr + 2 * c : nullptr, pl.qctr ? pl.e.parent : nullptr,
-                              pl.base[c], deferred ? c : -1);
-            if (rc) return rc;
-            aff_bytes += 4.0 * n[c] * (double)n[c] +
-                         4.0 * n[c] * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? p->dino_dim : 0));
-        }
-        if (pl.qctr) {
+            // host entry: the features arrive chunk by chunk while the pair stage and the root split run; the zero-row flags
+            // are then taken per chunk right before its feature pass (run_rebuild)
+            if (!arrival && p->theta != 0.0 && d_tarl)
+                LAUNCH(SG_AFFINITY, k_zero_rows<<<(pl.P + 7) / 8, 256, 0, st>>>(pl.P, d_tarl, p->tarl_dim, pl.tarl_zero));
             // a pair queue that overflowed (more than 96 in-mask pairs per point on average) leaves W incomplete:
             // redo the batch with the one-kernel form.  One small read-back per call.
             std::vector<int> hq(2 * (size_t)num_chunks);
             ANCUTS_CUDA(cudaMemcpyAsync(hq.data(), pl.qctr, hq.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
             ANCUTS_CUDA(cudaStreamSynchronize(st));
-            bool overflow = false;
-            for (int c = 0; c < num_chunks; ++c) overflow |= (hq[2 * c + 1] != 0);
-            if (overflow) {
-                root_forest = false;
-                deferred = false;
-                for (int c = 0; c < num_chunks; ++c) {
-                    int64_t o = h_chunk_off[c] - off0;
-                    if (h->feat_ev) ANCUTS_CUDA(cudaStreamWaitEvent(st, h->feat_ev[c], 0));     // batched host path: features
-                    const float* tz = d_tarl ? d_tarl + (size_t)(h_chunk_off[c]) * p->tarl_dim : nullptr;
-                    const float* dz = d_dino ? d_dino + (size_t)(h_chunk_off[c]) * p->dino_dim : nullptr;
-                    rc = run_affinity(h, pl, n[c], d_points + (size_t)h_chunk_off[c] * 3, tz, dz, p, pl.hW0[c], pl.ld[c],
-                                      pl.tarl_zero + o, st);
-                    if (rc) return rc;
-                }
+            for (int c = 0; c < num_chunks; ++c)
+                if (hq[2 * c + 1] != 0) deferred = nullptr;
+        } else if (arrival) {
+            ANCUTS_CUDA(cudaStreamWaitEvent(st, arrival->points, 0));
+        }
+        if (!deferred) {
+            // W of every chunk written whole: the tensor-core form, or the one-kernel form after an overflow
+            for (int c = 0; c < num_chunks; ++c) {
+                int64_t o = h_chunk_off[c] - off0;
+                if (arrival) ANCUTS_CUDA(cudaStreamWaitEvent(st, arrival->feats[c], 0));
+                const float* tz = d_tarl ? d_tarl + (size_t)(h_chunk_off[c]) * p->tarl_dim : nullptr;
+                const float* dz = d_dino ? d_dino + (size_t)(h_chunk_off[c]) * p->dino_dim : nullptr;
+                rc = run_affinity(h, pl, n[c], d_points + (size_t)h_chunk_off[c] * 3, tz, dz, p, pl.hW0[c], pl.ld[c],
+                                  pl.tarl_zero + o, st);
+                if (rc) return rc;
             }
         }
+        double aff_bytes = 0.0;
+        for (int c = 0; c < num_chunks; ++c)
+            aff_bytes += 4.0 * n[c] * (double)n[c] +
+                         4.0 * n[c] * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? p->dino_dim : 0));
         h->stage_bytes[SG_AFFINITY] = aff_bytes;
     }
-    DeferredAffinity df{p, d_tarl, d_dino, h_chunk_off, (deferred && pl.grid_pairs) ? h->feat_ev : nullptr,
-                        (deferred && pl.grid_pairs) ? pl.pg_sorted : nullptr};
-    if (csr) { df.row_ptr = csr->row_ptr; df.col = csr->col; df.val = csr->val; }
-    rc = run_levels(h, pl, p, 0, d_labels, h_num_segments, st, root_forest, deferred ? &df : nullptr);
+    rc = run_levels(h, pl, p, 0, d_labels, h_num_segments, st, deferred);
     if (rc) return rc;
     rc = copy_stats(h, pl, h_stats, stats_cap, h_num_stats, st);
     if (rc) return rc;
@@ -1691,8 +1694,8 @@ int ancuts_segment_chunks_host(ancuts_handle* h, int num_chunks, const int64_t* 
     float* d_dino = use_d ? (float*)(stage + align_up(bp, 256) + align_up(bt, 256)) : nullptr;
     int32_t* d_labels = (int32_t*)(stage + align_up(bp, 256) + align_up(bt, 256) + align_up(bd, 256));
     int rc = ANCUTS_OK;
-    // per-chunk copies on their own stream, one event per chunk: the affinity kernels of chunk c start as soon as its
-    // inputs are there, the copies of the later chunks overlap with them (pinned host memory)
+    // copies on their own stream (pinned host memory): the coordinates of every chunk first in one copy, for the pair stage,
+    // then the features chunk by chunk with one event each, which arrive while the pair stage and the root split run
     while ((int)h->copy_ev.size() < num_chunks + 1) {
         cudaEvent_t ev;
         ANCUTS_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -1700,38 +1703,20 @@ int ancuts_segment_chunks_host(ancuts_handle* h, int num_chunks, const int64_t* 
     }
     cudaError_t ce = cudaEventRecord(h->copy_ev[num_chunks], st);           // earlier work on st may still read the staging area
     if (ce == cudaSuccess) ce = cudaStreamWaitEvent(h->copy_stream, h->copy_ev[num_chunks], 0);
-    const bool feats_on = use_t || use_d;
-    (void)feats_on;
-    const bool batched = p->affinity_impl == 0 && h->opt[ANCUTS_OPT_AFFINITY_FORM] == 0 && h->opt[ANCUTS_OPT_PAIR_SEARCH] == 0;
-    if (batched && ce == cudaSuccess) {
-        // the batched pair stage needs every chunk's coordinates at once and no features: coordinates first (one copy), then
-        // the features, which arrive while the pair stage and the root split run
-        if (!h->ev_host[0]) ANCUTS_CUDA(cudaEventCreateWithFlags(&h->ev_host[0], cudaEventDisableTiming));
-        ce = cudaMemcpyAsync(d_points, h_points, bp, cudaMemcpyHostToDevice, h->copy_stream);
-        if (ce == cudaSuccess) ce = cudaEventRecord(h->ev_host[0], h->copy_stream);
-        for (int c = 0; c < num_chunks && ce == cudaSuccess; ++c) {
-            const size_t o = (size_t)h_chunk_off[c], m = (size_t)(h_chunk_off[c + 1] - h_chunk_off[c]);
-            if (use_t) ce = cudaMemcpyAsync(d_tarl + o * p->tarl_dim, h_tarl + o * p->tarl_dim, m * p->tarl_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
-            if (ce == cudaSuccess && use_d)
-                ce = cudaMemcpyAsync(d_dino + o * p->dino_dim, h_dino + o * p->dino_dim, m * p->dino_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
-            if (ce == cudaSuccess) ce = cudaEventRecord(h->copy_ev[c], h->copy_stream);
-        }
-        if (ce == cudaSuccess) { h->ev_points = h->ev_host[0]; h->feat_ev = h->copy_ev.data(); }
-    }
-    for (int c = 0; c < num_chunks && ce == cudaSuccess && !batched; ++c) {
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_points, h_points, bp, cudaMemcpyHostToDevice, h->copy_stream);
+    if (ce == cudaSuccess) ce = cudaEventRecord(h->points_ev, h->copy_stream);
+    for (int c = 0; c < num_chunks && ce == cudaSuccess; ++c) {
         const size_t o = (size_t)h_chunk_off[c], m = (size_t)(h_chunk_off[c + 1] - h_chunk_off[c]);
-        ce = cudaMemcpyAsync(d_points + o * 3, h_points + o * 3, m * 3 * sizeof(double), cudaMemcpyHostToDevice, h->copy_stream);
-        if (ce == cudaSuccess && use_t)
-            ce = cudaMemcpyAsync(d_tarl + o * p->tarl_dim, h_tarl + o * p->tarl_dim, m * p->tarl_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
+        if (use_t) ce = cudaMemcpyAsync(d_tarl + o * p->tarl_dim, h_tarl + o * p->tarl_dim, m * p->tarl_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
         if (ce == cudaSuccess && use_d)
             ce = cudaMemcpyAsync(d_dino + o * p->dino_dim, h_dino + o * p->dino_dim, m * p->dino_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
         if (ce == cudaSuccess) ce = cudaEventRecord(h->copy_ev[c], h->copy_stream);
     }
     if (ce != cudaSuccess) { set_error("H2D copy failed: %s", cudaGetErrorString(ce)); rc = ANCUTS_ECUDA; cudaStreamSynchronize(h->copy_stream); }
-    if (rc == ANCUTS_OK && !batched) h->wait_ev = h->copy_ev.data();
+    const Arrival arrival{h->points_ev, h->copy_ev.data()};
     if (rc == ANCUTS_OK)
         rc = segment_common(h, num_chunks, h_chunk_off, d_points, d_tarl, d_dino, nullptr, 0, 0, p, d_labels,
-                            h_num_segments, h_stats, stats_cap, h_num_stats, st);
+                            h_num_segments, h_stats, stats_cap, h_num_stats, st, nullptr, &arrival);
     if (rc != ANCUTS_OK) cudaStreamSynchronize(h->copy_stream);        // the caller may release its buffers after an error
     if (rc == ANCUTS_OK) {
         ce = cudaMemcpyAsync(h_labels, d_labels, bl, cudaMemcpyDeviceToHost, st);

@@ -21,7 +21,6 @@ struct ancuts_handle {
     cudaStream_t side[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // one per node size bin
     cudaEvent_t ev_fork = nullptr;
     cudaEvent_t ev_join[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    bool cluster16_ok = true;
     unsigned long long* h_acct = nullptr;    // pinned, ancuts::SG_ACCT
     double sparse_entry_steps = 0, sparse_nnz = 0;   // shared-memory sparse matvec: sum of k * entries, entries (last call)
     double cl_steps = 0, cl_full = 0;                // cluster kernel: Lanczos steps, steps with the full pass (last call)
@@ -35,15 +34,13 @@ struct ancuts_handle {
     std::vector<cudaEvent_t> pool;
     size_t pool_used = 0;
     bool attrs_set = false;
-    // Code paths with more than one implementation behind the same results (ancuts_set_option; every one is parity-tested):
+    // Code paths with more than one implementation behind the same results (ancuts_set_option; every one is parity-tested;
+    // option 0 is retired):
     int opt[ANCUTS_OPT_COUNT] = {0, 0, 0, 0, 0};
     int last_unconverged = 0;                // eigensolver nodes of the last segment call that stopped at lanczos_max_steps
-    cudaStream_t copy_stream = nullptr;      // host entry point: per-chunk H2D copies run ahead of the affinity kernels
-    std::vector<cudaEvent_t> copy_ev;        // one per chunk of the current host call
-    const cudaEvent_t* wait_ev = nullptr;    // set by the host entry point for segment_common (chunk c waits for wait_ev[c])
-    cudaEvent_t ev_host[2] = {nullptr, nullptr};     // batched pair stage: all coordinates have arrived ([1] unused)
-    cudaEvent_t ev_points = nullptr;                 // = ev_host[0] for the call in flight, else NULL
-    const cudaEvent_t* feat_ev = nullptr;            // per-chunk "features have arrived" events of the call in flight, else NULL
+    cudaStream_t copy_stream = nullptr;      // host entry point: H2D copies run ahead of the affinity kernels
+    cudaEvent_t points_ev = nullptr;         // host entry point: the coordinates of every chunk have arrived
+    std::vector<cudaEvent_t> copy_ev;        // host entry point: [c] chunk c's features have arrived, [num_chunks] copy fence
     unsigned long long* dbg = nullptr;       // device, 32 entries: phase cycles of the cluster kernel (ANCUTS_PHASES=1)
     char* post_ws = nullptr;                 // map_post.cu (merge / metrics): growable device workspace
     size_t post_ws_bytes = 0;

@@ -250,10 +250,9 @@ int ancuts_instance_metrics(ancuts_handle* h, int64_t n, const int32_t* d_all_la
  * (the Python drop-in raises, the array-level API warns). */
 int ancuts_last_unconverged(ancuts_handle* h);
 
-/* Alternative implementations behind the same results (each one parity-tested; 0 = the default):
- *   ANCUTS_OPT_AFFINITY_FORM  0 deferred (pairs queued, W written block by block after the root split),
- *                             1 dense two-pass (pairs + feature pass on the full N x N matrix), 2 dense one-kernel
- *   ANCUTS_OPT_PAIR_SEARCH    0 cell-sorted tile sweep, all chunks of the call in one launch, tile pairs pruned by their boxes,
+/* Alternative implementations behind the same results (each one parity-tested; 0 = the default).  Option 0 is retired
+ * (it selected a dense affinity form of the segment path); setting it returns ANCUTS_EINVAL.
+ *   ANCUTS_OPT_PAIR_SEARCH   0 cell-sorted tile sweep, all chunks of the call in one launch, tile pairs pruned by their boxes,
  *                             1 shuffled 64 x 64 tile sweep over the whole upper triangle, one launch per chunk
  *   ANCUTS_OPT_MATVEC         0 the cluster's row slices compressed (CSR) into shared memory once per node; a node whose
  *                               slices do not fit falls back, inside the kernel, to the dense form,
@@ -264,7 +263,6 @@ int ancuts_last_unconverged(ancuts_handle* h);
  *   ANCUTS_OPT_FUSED_CUT      0 a cluster kernel that holds its node as CSR slices also takes the node's cut decision (sign,
  *                               thresholds, buckets, N-cut scan, decision, side flags, component unions) in its epilogue,
  *                             1 the cut always runs as its own kernels after the eigensolver */
-#define ANCUTS_OPT_AFFINITY_FORM 0
 #define ANCUTS_OPT_PAIR_SEARCH   1
 #define ANCUTS_OPT_MATVEC        2
 #define ANCUTS_OPT_CLUSTER_MAP   3

@@ -94,6 +94,12 @@ def test_tensor_core_affinity_gives_the_same_labels(cuda_device):
     b = api.segment_packed(pk, affinity_impl=1, **kw)
     for la, lb in zip(a.labels, b.labels):
         assert R.same_partition(la, lb)
+    # resident inputs give the labels of the host entry, whose features arrive chunk by chunk, bit for bit
+    dev = pk.to_device(cuda_device)
+    api.segment_packed(pk, affinity_impl=1, dev_chunks=dev, **{k: v for k, v in kw.items() if k != "device"})
+    dl = dev.labels.cpu().numpy()
+    for c, lb in enumerate(b.labels):
+        assert np.array_equal(lb, dl[pk.off[c]:pk.off[c + 1]])
 
 
 def test_batched_equals_single(cuda_device):

@@ -1,5 +1,5 @@
-"""GPU tests of the alternative implementations behind the same C ABI (ancuts_set_option): affinity forms and the
-pair-queue overflow fallback, pair search, matvec forms; non-convergence reporting; the per-level trace."""
+"""GPU tests of the alternative implementations behind the same C ABI (ancuts_set_option): pair search, matvec forms,
+the stage entry's two-pass affinity and the pair-queue overflow fallback; non-convergence reporting; the per-level trace."""
 import numpy as np
 import pytest
 import scipy.sparse as sp
@@ -35,15 +35,26 @@ def check_affinity(W, A):
     assert np.array_equal(W, W.T)
 
 
-# include/autoinst_ncuts.h: ANCUTS_OPT_AFFINITY_FORM 0 (0 deferred, 1 dense two-pass, 2 dense one-kernel),
-# ANCUTS_OPT_PAIR_SEARCH 1 (0 cell-sorted sweep, 1 shuffled sweep), ANCUTS_OPT_MATVEC 2 (0 shared-memory slices, 1 dense from
-# HBM), ANCUTS_OPT_CLUSTER_MAP 3 (CTAs per node and size bin), ANCUTS_OPT_FUSED_CUT 4 (0 cut decision inside the sparse-form
-# eigensolver kernel, 1 its own kernels)
-AFF, PAIRS, MATVEC, CMAP, FUSED = 0, 1, 2, 3, 4
-VARIANTS = {"default": {}, "shuffled_pairs": {PAIRS: 1}, "dense_two_pass_affinity": {AFF: 1}, "one_kernel_affinity": {AFF: 2},
-            "dense_matvec": {MATVEC: 1}, "dense_matvec_shuffled_pairs": {MATVEC: 1, PAIRS: 1},
+# include/autoinst_ncuts.h: ANCUTS_OPT_PAIR_SEARCH 1 (0 cell-sorted sweep, 1 shuffled sweep), ANCUTS_OPT_MATVEC 2 (0 shared-
+# memory slices, 1 dense from HBM), ANCUTS_OPT_CLUSTER_MAP 3 (CTAs per node and size bin), ANCUTS_OPT_FUSED_CUT 4 (0 cut
+# decision inside the sparse-form eigensolver kernel, 1 its own kernels); option 0 is retired
+PAIRS, MATVEC, CMAP, FUSED = 1, 2, 3, 4
+VARIANTS = {"default": {}, "shuffled_pairs": {PAIRS: 1}, "dense_matvec": {MATVEC: 1},
+            "dense_matvec_shuffled_pairs": {MATVEC: 1, PAIRS: 1},
             "sparse_matvec_few_ctas": {CMAP: 112248}, "dense_matvec_many_ctas": {MATVEC: 1, CMAP: 224888},
             "separate_cut_kernels": {FUSED: 1}, "separate_cut_few_ctas": {FUSED: 1, CMAP: 112248}}
+
+
+def host_and_device_labels(api, packed, **kw):
+    """segment_packed through host buffers (ancuts_segment_chunks_host, inputs arriving on its copy stream) and with the
+    inputs resident on the device (ancuts_segment_chunks); the labels must be bit-identical.  Returns the host call."""
+    res = api.segment_packed(packed, **kw)
+    dev = packed.to_device(kw["device"])
+    api.segment_packed(packed, dev_chunks=dev, **{k: v for k, v in kw.items() if k != "device"})
+    labels = dev.labels.cpu().numpy()
+    for c, lab in enumerate(res.labels):
+        assert np.array_equal(lab, labels[packed.off[c]:packed.off[c + 1]]), c
+    return res
 
 
 @pytest.mark.parametrize("variant", list(VARIANTS))
@@ -53,8 +64,8 @@ def test_variants_give_oracle_labels(cuda_device, variant):
     cfg = CONFIGS["tarl_spatial"]
     chunks = [make_chunk(300 + i, n_target=1500 + 700 * i, features="tarl") for i in range(3)]
     packed = api.PackedChunks([c.points for c in chunks], [c.tarl for c in chunks], None, theta=cfg["theta"])
-    res = api.segment_packed(packed, device=cuda_device, lane=lane, alpha=cfg["alpha"], theta=cfg["theta"], T=cfg["T"],
-                             want_stats=True)
+    res = host_and_device_labels(api, packed, device=cuda_device, lane=lane, alpha=cfg["alpha"], theta=cfg["theta"],
+                                 T=cfg["T"], want_stats=True)
     assert int((res.stats["converged"] == 0).sum()) == 0 and res.unconverged == 0
     for ch, lab in zip(chunks, res.labels):
         A = affinity_ref(ch.points, ch.tarl, None, alpha=cfg["alpha"], theta=cfg["theta"])
@@ -140,35 +151,44 @@ def test_cut_sums_do_not_overflow_on_heavy_weights(cuda_device):
 
 
 @pytest.mark.parametrize("name", ["tarl_spatial", "tarl_spatial_dino"])
-def test_two_pass_and_one_kernel_affinity_agree_with_the_oracle(cuda_device, name):
+def test_two_pass_affinity_agrees_with_the_oracle(cuda_device, name):
+    """The stage entry's two-pass form (pairs, then the feature pass on the dense matrix).  The dense forms of the segment
+    path are no longer options: option 0 is retired and raises."""
     api = _api()
     cfg = CONFIGS[name]
     ch = make_chunk(41, n_target=2500, features="tarl_dino" if cfg["gamma"] else "tarl")
     A = affinity_ref(ch.points, ch.tarl, ch.dino if cfg["gamma"] else None, alpha=cfg["alpha"], theta=cfg["theta"], gamma=cfg["gamma"])
-    lane1 = variant_lane(cuda_device, VARIANTS["one_kernel_affinity"], 10 + list(VARIANTS).index("one_kernel_affinity"))
-    for lane in (0, lane1):
-        W = api.affinity(ch.points, ch.tarl, ch.dino if cfg["gamma"] else None, alpha=cfg["alpha"], theta=cfg["theta"],
-                         gamma=cfg["gamma"], device=cuda_device, lane=lane)
-        check_affinity(W, A)
+    W = api.affinity(ch.points, ch.tarl, ch.dino if cfg["gamma"] else None, alpha=cfg["alpha"], theta=cfg["theta"],
+                     gamma=cfg["gamma"], device=cuda_device, lane=0)
+    check_affinity(W, A)
+    with pytest.raises(RuntimeError, match="option 0 is retired"):
+        api.Handle.get(cuda_device, 0).set_option(0, 0)
 
 
 def test_pair_queue_overflow_falls_back(cuda_device):
     """More than 96 in-mask pairs per point on average: the queue of the two-pass form overflows and the one-kernel
-    form takes over, in the stage entry point (conditional launch) and in the segment call (host read-back)."""
+    form takes over, in the stage entry point (conditional launch) and in the segment call (host read-back), through host
+    buffers and with resident inputs alike, with TARL terms and with TARL and DINO terms."""
     api = _api()
     rng = np.random.default_rng(5)
     n = 900
     pts = (rng.normal(size=(n, 3)) * 0.2).astype(np.float32).astype(np.float64)       # one 1 m blob: almost every pair inside
     pts[n // 2:] += 7.0                                                                  # ... and a second one far away
     tarl = rng.normal(size=(n, 96)).astype(np.float32)
-    A = affinity_ref(pts, tarl.astype(np.float64), None, alpha=1.0, theta=0.5)
-    assert (A != 0).sum() > 2 * 96 * n
-    W = api.affinity(pts, tarl, alpha=1.0, theta=0.5, device=cuda_device)
-    check_affinity(W, A)
-    lab = api.segment_chunk(pts, tarl, alpha=1.0, theta=0.5, T=0.03, device=cuda_device)
-    with R.pinned_eigsh():
-        g = R.normalized_cut_ref(sp.csr_matrix(A), n, np.arange(n), T=0.03)
-    assert R.same_partition(lab, R.labels_from_groups(g, n))
+    dino_rows = rng.normal(size=(n, 384)).astype(np.float32)
+    for name in ("tarl_spatial", "tarl_spatial_dino"):
+        cfg = CONFIGS[name]
+        dino = dino_rows if cfg["gamma"] else None
+        kw = dict(alpha=cfg["alpha"], theta=cfg["theta"], gamma=cfg["gamma"])
+        A = affinity_ref(pts, tarl.astype(np.float64), None if dino is None else dino.astype(np.float64), **kw)
+        assert (A != 0).sum() > 2 * 96 * n
+        W = api.affinity(pts, tarl, dino, device=cuda_device, **kw)
+        check_affinity(W, A)
+        packed = api.PackedChunks([pts], [tarl], None if dino is None else [dino], theta=cfg["theta"], gamma=cfg["gamma"])
+        lab = host_and_device_labels(api, packed, device=cuda_device, T=cfg["T"], **kw).labels[0]
+        with R.pinned_eigsh():
+            g = R.normalized_cut_ref(sp.csr_matrix(A), n, np.arange(n), T=cfg["T"])
+        assert R.same_partition(lab, R.labels_from_groups(g, n)), name
 
 
 def test_level_trace(cuda_device):
