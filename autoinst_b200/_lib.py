@@ -28,6 +28,7 @@ EXPORTS = [
     "ancuts_merge_chunks", "ancuts_remove_semantics", "ancuts_instance_metrics", "ancuts_map_labels",
     "ancuts_last_sparse_accounting", "ancuts_dino_view_pixels", "ancuts_dino_mean",
     "ancuts_last_reorth_accounting", "ancuts_segment_csr_f32",
+    "ancuts_affinity_cams_f32", "ancuts_segment_chunks_cams", "ancuts_segment_chunks_cams_host",
 ]
 
 # ancuts_set_option (include/autoinst_ncuts.h; option 0 is retired)
@@ -102,6 +103,7 @@ def load():
     lib.ancuts_segment_workspace_bytes.argtypes = [C.c_int, i32p, C.c_int]
     lib.ancuts_segment_workspace_bytes.restype = C.c_int64
     lib.ancuts_affinity_f32.argtypes = [vp, C.c_int, vp, vp, vp, pp, vp, C.c_int64, vp, vp]
+    lib.ancuts_affinity_cams_f32.argtypes = [vp, C.c_int, vp, vp, vp, C.c_int, pp, vp, C.c_int64, vp, vp]
     lib.ancuts_degree_normalize_f32.argtypes = [vp, C.c_int, vp, C.c_int64, vp, vp, C.c_int64, vp]
     lib.ancuts_lanczos_fiedler_batched.argtypes = [vp, C.c_int, vp, C.c_int64, C.c_int, i32p, i32p, pp,
                                                    vp, dp, i32p, i32p, vp]
@@ -113,6 +115,10 @@ def load():
                                           i32p, vp]
     lib.ancuts_segment_chunks_host.argtypes = [vp, C.c_int, i64p, vp, vp, vp, pp, vp, i32p, sp,
                                                C.c_int32, i32p, vp]
+    lib.ancuts_segment_chunks_cams.argtypes = [vp, C.c_int, i64p, vp, vp, vp, C.c_int, pp, vp, i32p, sp, C.c_int32,
+                                               i32p, vp]
+    lib.ancuts_segment_chunks_cams_host.argtypes = [vp, C.c_int, i64p, vp, vp, vp, C.c_int, pp, vp, i32p, sp,
+                                                    C.c_int32, i32p, vp]
     lib.ancuts_segment_dense_f32.argtypes = [vp, C.c_int, vp, C.c_int64, C.c_int, pp, vp, i32p, sp,
                                              C.c_int32, i32p, vp]
     lib.ancuts_segment_csr_f32.argtypes = [vp, C.c_int, i64p, vp, vp, vp, C.c_int64, i32p, pp, vp, i32p, sp,

@@ -135,6 +135,34 @@ def _as_dev(x, dtype, device):
     return torch.as_tensor(np.ascontiguousarray(x), dtype=dtype).to(device)
 
 
+def _dino_shape(x):
+    """(cameras, width) of one chunk's DINOv2 input: an (n, D) array (one camera), a list or tuple of per-camera (n, D)
+    arrays (the reference's per-CAM_IDS means, ncuts_utils.py:81-110), or an (n, cams, D) array or tensor."""
+    if isinstance(x, (list, tuple)):
+        if len(x) == 0:
+            raise ValueError("The length should be longer than 0!")       # ncuts_utils.py:126-127
+        shapes = {tuple(int(d) for d in np.shape(c)) for c in x}
+        if len(shapes) != 1 or len(next(iter(shapes))) != 2:
+            raise ValueError(f"the cameras of a chunk need one (n, D) shape each, got {sorted(shapes)}")
+        return len(x), next(iter(shapes))[1]
+    shape = tuple(int(d) for d in x.shape)
+    if len(shape) == 2:
+        return 1, shape[1]
+    if len(shape) == 3:
+        return shape[1], shape[2]
+    raise ValueError(f"DINOv2 input must be (n, D), a list of (n, D) or (n, cams, D), got shape {shape}")
+
+
+def _dino_rows(x, device):
+    """One chunk's DINOv2 input on the device as point-major (n, cams * D) float32 rows; returns (rows, cams, D)."""
+    cams, width = _dino_shape(x)
+    if isinstance(x, (list, tuple)):
+        g = torch.stack([_as_dev(c, torch.float32, device) for c in x], dim=1)
+    else:
+        g = _as_dev(x, torch.float32, device)
+    return g.reshape(g.shape[0], cams * width).contiguous(), cams, width
+
+
 def padded_ld(n: int) -> int:
     return (int(n) + 31) // 32 * 32
 
@@ -151,24 +179,25 @@ def alloc_matrix(n, device):
 # ------------------------------------------------------------------------------------------------
 def affinity(points, tarl=None, dino=None, *, alpha=1.0, theta=0.0, gamma=0.0, proximity=1.0, impl=0,
              device=None, return_rowsum=False, lane: int = 0):
-    """Stage 1: dense float32 affinity (ncuts_utils.py:60-156).  Returns the n x n view of an n x ld buffer."""
+    """Stage 1: dense float32 affinity (ncuts_utils.py:60-156).  Returns the n x n view of an n x ld buffer.
+    dino: (n, D), a list of per-camera (n, D) arrays or (n, cams, D); several cameras multiply their terms."""
     device = _dev(device)
     hd = Handle.get(device, lane)
     pts = _as_dev(points, torch.float64, device)
     n = pts.shape[0]
     t = _as_dev(tarl, torch.float32, device) if theta else None
-    g = _as_dev(dino, torch.float32, device) if gamma else None
     if theta and t is None:
         raise ValueError("theta != 0 needs TARL features")
-    if gamma and g is None:
+    if gamma and dino is None:
         raise ValueError("The length should be longer than 0!")       # ncuts_utils.py:126-127
+    g, cams, width = _dino_rows(dino, device) if gamma else (None, 1, 0)
     p = make_params(alpha, theta, gamma, 0.0, proximity, tarl_dim=t.shape[1] if t is not None else 0,
-                    dino_dim=g.shape[1] if g is not None else 0, affinity_impl=impl)
+                    dino_dim=width, affinity_impl=impl)
     buf, view = alloc_matrix(n, device)
     rs = torch.empty(n, dtype=torch.float64, device=device) if return_rowsum else None
     with torch.cuda.device(device):
-        check(hd.lib.ancuts_affinity_f32(hd.h, n, _ptr(pts), _ptr(t), _ptr(g), C.byref(p), _ptr(buf), buf.stride(0),
-                                         _ptr(rs), _stream(device)))
+        check(hd.lib.ancuts_affinity_cams_f32(hd.h, n, _ptr(pts), _ptr(t), _ptr(g), cams, C.byref(p), _ptr(buf),
+                                              buf.stride(0), _ptr(rs), _stream(device)))
     return (view, rs) if return_rowsum else view
 
 
@@ -560,11 +589,18 @@ class _PinnedPool:
 def _pack_host(points_list, tarl_list, dino_list, use_t, use_d, pin=True, reuse=False):
     """Concatenate the chunks into (pinned) host buffers: float64 coordinates, float32 features.  The float64 -> float32
     conversion of the features (the reference hands float64 means, chunk_generation.py:252) goes straight into the buffer,
-    chunks in parallel on a few threads (numpy releases the GIL)."""
+    chunks in parallel on a few threads (numpy releases the GIL).  The DINOv2 buffer is point-major (P, cams * D): a
+    point's row holds camera 0's D values, then camera 1's, ...  Returns (sizes, off, points, tarl, dino, cams)."""
     sizes = [int(np.asarray(p).shape[0]) for p in points_list]
     off = np.zeros(len(sizes) + 1, dtype=np.int64)
     off[1:] = np.cumsum(sizes)
     total = int(off[-1])
+    cams, width = 1, 0
+    if use_d:
+        shapes = [_dino_shape(g) for g in dino_list]
+        if len(set(shapes)) != 1:
+            raise ValueError(f"every chunk of a call needs the same DINOv2 cameras and width, got {sorted(set(shapes))}")
+        cams, width = shapes[0]
 
     def mk(name, shape, dtype):
         if reuse:
@@ -573,7 +609,7 @@ def _pack_host(points_list, tarl_list, dino_list, use_t, use_d, pin=True, reuse=
         return t.pin_memory() if pin else t
     hp = mk("points", (total, 3), torch.float64)
     ht = mk("tarl", (total, np.asarray(tarl_list[0]).shape[1]), torch.float32) if use_t else None
-    hd_ = mk("dino", (total, np.asarray(dino_list[0]).shape[1]), torch.float32) if use_d else None
+    hd_ = mk("dino", (total, cams * width), torch.float32) if use_d else None
     hp_n = hp.numpy()
     ht_n = ht.numpy() if use_t else None
     hd_n = hd_.numpy() if use_d else None
@@ -584,7 +620,13 @@ def _pack_host(points_list, tarl_list, dino_list, use_t, use_d, pin=True, reuse=
         if use_t:
             np.copyto(ht_n[a:b], np.asarray(tarl_list[c]), casting="same_kind")
         if use_d:
-            np.copyto(hd_n[a:b], np.asarray(dino_list[c]), casting="same_kind")
+            g = dino_list[c]
+            if isinstance(g, (list, tuple)):
+                rows = hd_n[a:b].reshape(b - a, cams, width)
+                for k, cam in enumerate(g):
+                    np.copyto(rows[:, k], np.asarray(cam), casting="same_kind")
+            else:
+                np.copyto(hd_n[a:b].reshape(np.shape(g)), np.asarray(g), casting="same_kind")
     if len(sizes) >= 4 and total * (3 + (ht_n.shape[1] if use_t else 0) + (hd_n.shape[1] if use_d else 0)) > (1 << 22):
         from concurrent.futures import ThreadPoolExecutor
         import os as _os
@@ -593,11 +635,14 @@ def _pack_host(points_list, tarl_list, dino_list, use_t, use_d, pin=True, reuse=
     else:
         for c in range(len(sizes)):
             put(c)
-    return sizes, off, hp, ht, hd_
+    return sizes, off, hp, ht, hd_, cams
 
 
 class PackedChunks:
-    """Inputs of a batch of chunks packed once into pinned host buffers (what a data loader hands over)."""
+    """Inputs of a batch of chunks packed once into pinned host buffers (what a data loader hands over).  A chunk's DINOv2
+    input is an (n, D) array (one camera), a list or tuple of per-camera (n, D) arrays, or an (n, cams, D) array; every
+    chunk of a batch has the same cameras and width.  `dino` is (P, dino_cams * dino_dim), dino_dim the width of one
+    camera."""
 
     def __init__(self, points_list, tarl_list=None, dino_list=None, *, theta=0.0, gamma=0.0, pin=True, reuse=False):
         self.use_t = bool(theta) and tarl_list is not None
@@ -606,7 +651,7 @@ class PackedChunks:
             raise ValueError("theta != 0 needs TARL features")
         if gamma and dino_list is None:
             raise ValueError("The length should be longer than 0!")
-        self.sizes, self.off, self.points, self.tarl, self.dino = _pack_host(
+        self.sizes, self.off, self.points, self.tarl, self.dino, self.dino_cams = _pack_host(
             points_list, tarl_list, dino_list, self.use_t, self.use_d, pin, reuse)
         if reuse:      # buffers of the module-level pool: valid until the next PackedChunks(reuse=True)
             self.labels = _PinnedPool.take("labels", (int(self.off[-1]),), torch.int32, pin)
@@ -615,7 +660,7 @@ class PackedChunks:
             if pin:
                 self.labels = self.labels.pin_memory()
         self.tarl_dim = self.tarl.shape[1] if self.use_t else 0
-        self.dino_dim = self.dino.shape[1] if self.use_d else 0
+        self.dino_dim = self.dino.shape[1] // self.dino_cams if self.use_d else 0
 
     def h2d_bytes(self):
         b = self.points.numel() * 8
@@ -660,14 +705,14 @@ def _run_segment(hd, fn_host, packed, dev_chunks, p, want_stats, device):
     sp = stats.ctypes.data_as(C.POINTER(NodeStat)) if want_stats else None
     with torch.cuda.device(device):
         if fn_host:
-            check(hd.lib.ancuts_segment_chunks_host(
+            check(hd.lib.ancuts_segment_chunks_cams_host(
                 hd.h, B, off.ctypes.data_as(C.POINTER(C.c_int64)), _ptr(packed.points), _ptr(packed.tarl),
-                _ptr(packed.dino), C.byref(p), _ptr(packed.labels), nseg.ctypes.data_as(C.POINTER(C.c_int32)),
+                _ptr(packed.dino), packed.dino_cams, C.byref(p), _ptr(packed.labels), nseg.ctypes.data_as(C.POINTER(C.c_int32)),
                 sp, cap, C.byref(nstats), _stream(device)))
         else:
-            check(hd.lib.ancuts_segment_chunks(
+            check(hd.lib.ancuts_segment_chunks_cams(
                 hd.h, B, off.ctypes.data_as(C.POINTER(C.c_int64)), _ptr(dev_chunks.points), _ptr(dev_chunks.tarl),
-                _ptr(dev_chunks.dino), C.byref(p), _ptr(dev_chunks.labels), nseg.ctypes.data_as(C.POINTER(C.c_int32)),
+                _ptr(dev_chunks.dino), packed.dino_cams, C.byref(p), _ptr(dev_chunks.labels), nseg.ctypes.data_as(C.POINTER(C.c_int32)),
                 sp, cap, C.byref(nstats), _stream(device)))
     return nseg, (stats[:nstats.value].copy() if want_stats else None)
 
@@ -822,7 +867,8 @@ def segment_packed_lanes(packed_lanes, dev_lanes=None, **kw):
 def segment_chunks(points_list, tarl_list=None, dino_list=None, *, alpha=1.0, theta=0.0, gamma=0.0, T=0.01,
                    proximity=1.0, split_lim=0.01, device=None, want_stats=False, memory_budget=None,
                    **kw) -> SegmentResult:
-    """Segment a list of chunks (host arrays in, host labels out), batched to fit device memory."""
+    """Segment a list of chunks (host arrays in, host labels out), batched to fit device memory.  A chunk's DINOv2 input
+    takes any form PackedChunks takes (several cameras: a list of per-camera arrays or an (n, cams, D) array)."""
     device = _dev(device)
     sizes = [int(np.asarray(p).shape[0]) for p in points_list]
     if memory_budget is None:

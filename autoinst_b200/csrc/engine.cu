@@ -370,9 +370,10 @@ static int resolve_kmax(const ancuts_params* p) {
 }
 
 // feature inputs of an affinity call (stage entry, points input of the segment path)
-static int check_features(const ancuts_params* p, const float* tarl, const float* dino) {
+static int check_features(const ancuts_params* p, const float* tarl, const float* dino, int dcams) {
     const bool use_tarl = p->theta != 0.0 && tarl != nullptr;
     const bool use_dino = p->gamma != 0.0 && dino != nullptr;
+    if (dcams < 1) { set_error("dino_cams must be at least 1 (got %d)", dcams); return ANCUTS_EINVAL; }
     if (p->theta != 0.0 && tarl == nullptr) { set_error("theta != 0 but no TARL features"); return ANCUTS_EINVAL; }
     if (p->gamma != 0.0 && dino == nullptr) {
         set_error("The length should be longer than 0!");      // ncuts_utils.py:126-127
@@ -382,13 +383,17 @@ static int check_features(const ancuts_params* p, const float* tarl, const float
         set_error("feature dimensions must be positive multiples of 4 (got %d, %d)", p->tarl_dim, p->dino_dim);
         return ANCUTS_EUNSUPPORTED;
     }
+    if (use_dino && dcams > 1 && p->affinity_impl == 1) {
+        set_error("the tensor-core affinity form (affinity_impl = 1) takes one DINOv2 camera (got %d)", dcams);
+        return ANCUTS_EUNSUPPORTED;
+    }
     return ANCUTS_OK;
 }
 
 // W of one chunk written whole (inputs checked by check_features).  qctr != NULL selects the two-pass form of the stage
 // entry (feature terms only): pairs into the single queue pl.pairq, then the feature pass.
 static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, const float* tarl, const float* dino,
-                        const ancuts_params* p, float* W, long long ld, uint8_t* tarl_zero, cudaStream_t st,
+                        int dcams, const ancuts_params* p, float* W, long long ld, uint8_t* tarl_zero, cudaStream_t st,
                         int* qctr = nullptr) {
     const bool use_tarl = p->theta != 0.0 && tarl != nullptr;
     const bool use_dino = p->gamma != 0.0 && dino != nullptr;
@@ -406,12 +411,12 @@ static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, co
         LAUNCH(SG_AFFINITY, k_affinity_pairs<<<grid, 256, 0, st>>>(n, pts, p->alpha, p->proximity, W, ld, pl.pairq, pl.qcap, qctr,
                                                                    nullptr, 0));
         LAUNCH(SG_AFFINITY, k_affinity_feats<<<148 * 4, 256, 0, st>>>(pl.pairq, qctr, pl.qcap, use_tarl ? tarl : nullptr, p->tarl_dim,
-                                                                        use_dino ? dino : nullptr, p->dino_dim, tarl_zero, p->theta,
+                                                                        use_dino ? dino : nullptr, p->dino_dim, dcams, tarl_zero, p->theta,
                                                                         p->gamma, W, ld));
     } else {
         dim3 grid((unsigned)((ld + AT - 1) / AT), (n + AT - 1) / AT);
         LAUNCH(SG_AFFINITY, k_affinity_exact<<<grid, 256, 0, st>>>(n, pts, use_tarl ? tarl : nullptr, p->tarl_dim,
-                                                                   use_dino ? dino : nullptr, p->dino_dim, tarl_zero,
+                                                                   use_dino ? dino : nullptr, p->dino_dim, dcams, tarl_zero,
                                                                    p->alpha, p->theta, p->gamma, p->proximity, W, ld));
     }
     ANCUTS_CUDA(cudaGetLastError());
@@ -646,7 +651,8 @@ k_ev_stats(Eng e) {
 struct DeferredAffinity {
     const ancuts_params* p;
     const float* tarl;      // all chunks, input order
-    const float* dino;
+    const float* dino;      // point-major, dcams * dino_dim values per point
+    int dcams;
     const int64_t* chunk_off;
     const cudaEvent_t* feats;      // host entry: chunk c's features have arrived at feats[c], else NULL
     const int* order;              // batched pair stage: the queue holds cell-sorted ranks, order[base + rank] = input index
@@ -730,7 +736,7 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
             }
             LAUNCH(SG_AFFINITY, k_affinity_feats<<<148 * 4, 256, 0, st>>>(
                 pl.pairq + pl.qoff[c], pl.qctr + 2 * c, pl.qcap_c[c], use_tarl ? df->tarl + o * p->tarl_dim : nullptr, p->tarl_dim,
-                use_dino ? df->dino + o * p->dino_dim : nullptr, p->dino_dim, pl.tarl_zero + (o - (size_t)df->chunk_off[0]),
+                use_dino ? df->dino + o * df->dcams * p->dino_dim : nullptr, p->dino_dim, df->dcams, pl.tarl_zero + (o - (size_t)df->chunk_off[0]),
                 p->theta, p->gamma, dst, pl.ld[c], e.val, pl.base[c], e.rid, e.r_status,
                 df->order ? df->order + pl.base[c] : nullptr));
         }
@@ -981,9 +987,14 @@ int ancuts_last_accounting(ancuts_handle* h, double* bytes6, double* ms6, int64_
 
 int ancuts_affinity_f32(ancuts_handle* h, int n, const double* d_points, const float* d_tarl, const float* d_dino,
                         const ancuts_params* p, float* d_W, int64_t ld, double* d_rowsum, void* stream) {
+    return ancuts_affinity_cams_f32(h, n, d_points, d_tarl, d_dino, 1, p, d_W, ld, d_rowsum, stream);
+}
+
+int ancuts_affinity_cams_f32(ancuts_handle* h, int n, const double* d_points, const float* d_tarl, const float* d_dino,
+                             int dino_cams, const ancuts_params* p, float* d_W, int64_t ld, double* d_rowsum, void* stream) {
     if (!h || n <= 0 || !d_points || !d_W || ld < n || (ld % 4)) { set_error("bad argument to ancuts_affinity_f32"); return ANCUTS_EINVAL; }
     int rc = check_params(p);
-    if (!rc) rc = check_features(p, d_tarl, d_dino);
+    if (!rc) rc = check_features(p, d_tarl, d_dino, dino_cams);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     ANCUTS_CUDA(cudaSetDevice(h->device));
@@ -1006,14 +1017,14 @@ int ancuts_affinity_f32(ancuts_handle* h, int n, const double* d_points, const f
     int* qctr = two_pass ? (int*)(h->ws + o_ctr) : nullptr;
     begin_accounting(h);
     if (qctr) ANCUTS_CUDA(cudaMemsetAsync(qctr, 0, 2 * sizeof(int), st));
-    rc = run_affinity(h, pl, n, d_points, d_tarl, d_dino, p, d_W, ld, tz, st, qctr);
+    rc = run_affinity(h, pl, n, d_points, d_tarl, d_dino, dino_cams, p, d_W, ld, tz, st, qctr);
     if (rc) return rc;
     if (qctr) {
         // queue overflow (flag set by pass 1): the one-kernel form runs, otherwise its CTAs exit at once; no host sync
         const bool use_tarl = p->theta != 0.0 && d_tarl != nullptr, use_dino = p->gamma != 0.0 && d_dino != nullptr;
         dim3 grid((unsigned)((ld + AT - 1) / AT), (n + AT - 1) / AT);
         LAUNCH(SG_AFFINITY, k_affinity_exact<<<grid, 256, 0, st>>>(n, d_points, use_tarl ? d_tarl : nullptr, p->tarl_dim,
-                                                                   use_dino ? d_dino : nullptr, p->dino_dim, tz, p->alpha,
+                                                                   use_dino ? d_dino : nullptr, p->dino_dim, dino_cams, tz, p->alpha,
                                                                    p->theta, p->gamma, p->proximity, d_W, ld, qctr + 1));
     }
     if (d_rowsum) {
@@ -1025,7 +1036,8 @@ int ancuts_affinity_f32(ancuts_handle* h, int n, const double* d_points, const f
         ANCUTS_CUDA(cudaStreamSynchronize(st));
         for (auto& t : h->timed) { float ms = 0.f; if (cudaEventElapsedTime(&ms, t.a, t.b) == cudaSuccess) h->stage_ms[t.stage] += ms; }
         h->timed.clear();
-        h->stage_bytes[SG_AFFINITY] = 4.0 * n * (double)n + 4.0 * n * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? p->dino_dim : 0));
+        h->stage_bytes[SG_AFFINITY] = 4.0 * n * (double)n +
+                                      4.0 * n * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? dino_cams * p->dino_dim : 0));
     }
     return ANCUTS_OK;
 }
@@ -1525,12 +1537,12 @@ struct Arrival {
 };
 
 static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off, const double* d_points,
-                          const float* d_tarl, const float* d_dino, const float* d_W_dense, int64_t ld_dense,
+                          const float* d_tarl, const float* d_dino, int dcams, const float* d_W_dense, int64_t ld_dense,
                           int num_points_orig, const ancuts_params* p, int32_t* d_labels, int32_t* h_num_segments,
                           ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats, cudaStream_t st,
                           const CsrInput* csr = nullptr, const Arrival* arrival = nullptr) {
     int rc = check_params(p);
-    if (!rc && !d_W_dense && !csr) rc = check_features(p, d_tarl, d_dino);
+    if (!rc && !d_W_dense && !csr) rc = check_features(p, d_tarl, d_dino, dcams);
     if (rc) return rc;
     if (!h || num_chunks <= 0 || !h_chunk_off || !d_labels) { set_error("bad argument to segment"); return ANCUTS_EINVAL; }
     ANCUTS_CUDA(cudaSetDevice(h->device));
@@ -1562,7 +1574,7 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     layout(pl, h->ws, stats_cap, p->tarl_dim, p->dino_dim, need_tc);
     // deferred != NULL: the input stage builds the root-level forest and W is written after the root split (CSR: from the
     // stored entries); otherwise W is whole before the level loop
-    DeferredAffinity df{p, d_tarl, d_dino, h_chunk_off, arrival ? arrival->feats : nullptr, pl.grid_pairs ? pl.pg_sorted : nullptr};
+    DeferredAffinity df{p, d_tarl, d_dino, dcams, h_chunk_off, arrival ? arrival->feats : nullptr, pl.grid_pairs ? pl.pg_sorted : nullptr};
     if (csr) { df.row_ptr = csr->row_ptr; df.col = csr->col; df.val = csr->val; }
     const DeferredAffinity* deferred = (pl.deferred || pl.csr) ? &df : nullptr;
     rc = upload_tables(pl, st);
@@ -1617,8 +1629,8 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
                 int64_t o = h_chunk_off[c] - off0;
                 if (arrival) ANCUTS_CUDA(cudaStreamWaitEvent(st, arrival->feats[c], 0));
                 const float* tz = d_tarl ? d_tarl + (size_t)(h_chunk_off[c]) * p->tarl_dim : nullptr;
-                const float* dz = d_dino ? d_dino + (size_t)(h_chunk_off[c]) * p->dino_dim : nullptr;
-                rc = run_affinity(h, pl, n[c], d_points + (size_t)h_chunk_off[c] * 3, tz, dz, p, pl.hW0[c], pl.ld[c],
+                const float* dz = d_dino ? d_dino + (size_t)(h_chunk_off[c]) * dcams * p->dino_dim : nullptr;
+                rc = run_affinity(h, pl, n[c], d_points + (size_t)h_chunk_off[c] * 3, tz, dz, dcams, p, pl.hW0[c], pl.ld[c],
                                   pl.tarl_zero + o, st);
                 if (rc) return rc;
             }
@@ -1626,7 +1638,7 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
         double aff_bytes = 0.0;
         for (int c = 0; c < num_chunks; ++c)
             aff_bytes += 4.0 * n[c] * (double)n[c] +
-                         4.0 * n[c] * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? p->dino_dim : 0));
+                         4.0 * n[c] * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? dcams * p->dino_dim : 0));
         h->stage_bytes[SG_AFFINITY] = aff_bytes;
     }
     rc = run_levels(h, pl, p, 0, d_labels, h_num_segments, st, deferred);
@@ -1641,9 +1653,17 @@ int ancuts_segment_chunks(ancuts_handle* h, int num_chunks, const int64_t* h_chu
                           const float* d_tarl, const float* d_dino, const ancuts_params* p, int32_t* d_labels,
                           int32_t* h_num_segments, ancuts_node_stat* h_stats, int32_t stats_cap,
                           int32_t* h_num_stats, void* stream) {
+    return ancuts_segment_chunks_cams(h, num_chunks, h_chunk_off, d_points, d_tarl, d_dino, 1, p, d_labels, h_num_segments,
+                                      h_stats, stats_cap, h_num_stats, stream);
+}
+
+int ancuts_segment_chunks_cams(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off, const double* d_points,
+                               const float* d_tarl, const float* d_dino, int dino_cams, const ancuts_params* p,
+                               int32_t* d_labels, int32_t* h_num_segments, ancuts_node_stat* h_stats, int32_t stats_cap,
+                               int32_t* h_num_stats, void* stream) {
     if (!d_points) { set_error("d_points is NULL"); return ANCUTS_EINVAL; }
     if (h_chunk_off && h_chunk_off[0] != 0) { set_error("h_chunk_off[0] must be 0"); return ANCUTS_EINVAL; }
-    return segment_common(h, num_chunks, h_chunk_off, d_points, d_tarl, d_dino, nullptr, 0, 0, p, d_labels,
+    return segment_common(h, num_chunks, h_chunk_off, d_points, d_tarl, d_dino, dino_cams, nullptr, 0, 0, p, d_labels,
                           h_num_segments, h_stats, stats_cap, h_num_stats, (cudaStream_t)stream);
 }
 
@@ -1652,7 +1672,7 @@ int ancuts_segment_dense_f32(ancuts_handle* h, int n, const float* d_W, int64_t 
                              ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats, void* stream) {
     if (!d_W || n <= 0 || ld < n) { set_error("bad argument to ancuts_segment_dense_f32"); return ANCUTS_EINVAL; }
     int64_t off[2] = {0, n};
-    return segment_common(h, 1, off, nullptr, nullptr, nullptr, d_W, ld, num_points_orig, p, d_labels,
+    return segment_common(h, 1, off, nullptr, nullptr, nullptr, 1, d_W, ld, num_points_orig, p, d_labels,
                           h_num_segments, h_stats, stats_cap, h_num_stats, (cudaStream_t)stream);
 }
 
@@ -1663,7 +1683,7 @@ int ancuts_segment_csr_f32(ancuts_handle* h, int num_graphs, const int64_t* h_gr
     if (!d_row_ptr || nnz < 0 || (nnz > 0 && (!d_col || !d_val))) { set_error("bad argument to ancuts_segment_csr_f32"); return ANCUTS_EINVAL; }
     if (h_graph_off && h_graph_off[0] != 0) { set_error("h_graph_off[0] must be 0"); return ANCUTS_EINVAL; }
     CsrInput csr{d_row_ptr, d_col, d_val, nnz, h_num_points_orig};
-    return segment_common(h, num_graphs, h_graph_off, nullptr, nullptr, nullptr, nullptr, 0, 0, p, d_labels, h_num_segments,
+    return segment_common(h, num_graphs, h_graph_off, nullptr, nullptr, nullptr, 1, nullptr, 0, 0, p, d_labels, h_num_segments,
                           h_stats, stats_cap, h_num_stats, (cudaStream_t)stream, &csr);
 }
 
@@ -1671,14 +1691,24 @@ int ancuts_segment_chunks_host(ancuts_handle* h, int num_chunks, const int64_t* 
                                const float* h_tarl, const float* h_dino, const ancuts_params* p, int32_t* h_labels,
                                int32_t* h_num_segments, ancuts_node_stat* h_stats, int32_t stats_cap,
                                int32_t* h_num_stats, void* stream) {
+    return ancuts_segment_chunks_cams_host(h, num_chunks, h_chunk_off, h_points, h_tarl, h_dino, 1, p, h_labels,
+                                           h_num_segments, h_stats, stats_cap, h_num_stats, stream);
+}
+
+int ancuts_segment_chunks_cams_host(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off, const double* h_points,
+                                    const float* h_tarl, const float* h_dino, int dino_cams, const ancuts_params* p,
+                                    int32_t* h_labels, int32_t* h_num_segments, ancuts_node_stat* h_stats,
+                                    int32_t stats_cap, int32_t* h_num_stats, void* stream) {
     if (!h || !h_points || !h_labels || !h_chunk_off || num_chunks <= 0 || !p) { set_error("bad argument to ancuts_segment_chunks_host"); return ANCUTS_EINVAL; }
     if (h_chunk_off[0] != 0) { set_error("h_chunk_off[0] must be 0"); return ANCUTS_EINVAL; }
     cudaStream_t st = (cudaStream_t)stream;
     ANCUTS_CUDA(cudaSetDevice(h->device));
     const size_t P = (size_t)h_chunk_off[num_chunks];
     const bool use_t = h_tarl && p->theta != 0.0, use_d = h_dino && p->gamma != 0.0;
+    if (use_d && dino_cams < 1) { set_error("dino_cams must be at least 1 (got %d)", dino_cams); return ANCUTS_EINVAL; }
+    const size_t drow = use_d ? (size_t)dino_cams * p->dino_dim : 0;        // floats per point, every camera
     size_t bp = P * 3 * sizeof(double), bt = use_t ? P * p->tarl_dim * sizeof(float) : 0,
-           bd = use_d ? P * p->dino_dim * sizeof(float) : 0, bl = P * sizeof(int32_t);
+           bd = P * drow * sizeof(float), bl = P * sizeof(int32_t);
     size_t total = align_up(bp, 256) + align_up(bt, 256) + align_up(bd, 256) + align_up(bl, 256);
     if (total > h->stage_cap) {
         if (h->stage) cudaFree(h->stage);
@@ -1709,13 +1739,13 @@ int ancuts_segment_chunks_host(ancuts_handle* h, int num_chunks, const int64_t* 
         const size_t o = (size_t)h_chunk_off[c], m = (size_t)(h_chunk_off[c + 1] - h_chunk_off[c]);
         if (use_t) ce = cudaMemcpyAsync(d_tarl + o * p->tarl_dim, h_tarl + o * p->tarl_dim, m * p->tarl_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
         if (ce == cudaSuccess && use_d)
-            ce = cudaMemcpyAsync(d_dino + o * p->dino_dim, h_dino + o * p->dino_dim, m * p->dino_dim * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
+            ce = cudaMemcpyAsync(d_dino + o * drow, h_dino + o * drow, m * drow * sizeof(float), cudaMemcpyHostToDevice, h->copy_stream);
         if (ce == cudaSuccess) ce = cudaEventRecord(h->copy_ev[c], h->copy_stream);
     }
     if (ce != cudaSuccess) { set_error("H2D copy failed: %s", cudaGetErrorString(ce)); rc = ANCUTS_ECUDA; cudaStreamSynchronize(h->copy_stream); }
     const Arrival arrival{h->points_ev, h->copy_ev.data()};
     if (rc == ANCUTS_OK)
-        rc = segment_common(h, num_chunks, h_chunk_off, d_points, d_tarl, d_dino, nullptr, 0, 0, p, d_labels,
+        rc = segment_common(h, num_chunks, h_chunk_off, d_points, d_tarl, d_dino, dino_cams, nullptr, 0, 0, p, d_labels,
                             h_num_segments, h_stats, stats_cap, h_num_stats, st, nullptr, &arrival);
     if (rc != ANCUTS_OK) cudaStreamSynchronize(h->copy_stream);        // the caller may release its buffers after an error
     if (rc == ANCUTS_OK) {

@@ -75,9 +75,50 @@ __device__ __forceinline__ double feat_dist8(const float* __restrict__ a, const 
     return sqrt(s);
 }
 
+// DINOv2 term over several cameras: S = dd_0 + dd_1 + ... with dd_c = ||a_c - b_c||, a_c = a + c * dim (rows are point-major,
+// camera c's dim values at c * dim).  The reference multiplies exp(-gamma dd_c) over the cameras (ncuts_utils.py:129-133); the
+// kernels evaluate the single exponential exp(-gamma S).  One float64 sum of squares and one sqrt per camera, the distances added
+// in camera order.  The loads of up to CAM_BATCH cameras are issued before their shuffle reductions, so a second camera adds
+// bandwidth rather than another dependent round trip.  One camera takes feat_dist8 itself (S = dd_0, bit for bit).
+constexpr int CAM_BATCH = 4;
+
+__device__ __forceinline__ double feat_dist8_cams(const float* __restrict__ a, const float* __restrict__ b,
+                                                  int dim, int cams, int lane8) {
+    if (cams == 1) return feat_dist8(a, b, dim, lane8);
+    double S = 0.0;
+    for (int c0 = 0; c0 < cams; c0 += CAM_BATCH) {
+        double s[CAM_BATCH];
+#pragma unroll
+        for (int c = 0; c < CAM_BATCH; ++c) s[c] = 0.0;
+        for (int k = lane8 * 4; k < dim; k += 32) {
+#pragma unroll
+            for (int c = 0; c < CAM_BATCH; ++c) {
+                if (c0 + c < cams) {
+                    const size_t o = (size_t)(c0 + c) * dim + k;
+                    float4 x = *reinterpret_cast<const float4*>(a + o);
+                    float4 y = *reinterpret_cast<const float4*>(b + o);
+                    double d0 = (double)x.x - (double)y.x, d1 = (double)x.y - (double)y.y;
+                    double d2 = (double)x.z - (double)y.z, d3 = (double)x.w - (double)y.w;
+                    s[c] += d0 * d0 + d1 * d1 + d2 * d2 + d3 * d3;
+                }
+            }
+        }
+#pragma unroll
+        for (int c = 0; c < CAM_BATCH; ++c) {
+            if (c0 + c < cams) {                       // uniform over the warp: cams is a kernel argument
+                s[c] += __shfl_xor_sync(0xffffffffu, s[c], 4);
+                s[c] += __shfl_xor_sync(0xffffffffu, s[c], 2);
+                s[c] += __shfl_xor_sync(0xffffffffu, s[c], 1);
+                S += sqrt(s[c]);
+            }
+        }
+    }
+    return S;
+}
+
 __global__ void __launch_bounds__(256)
 k_affinity_exact(int n, const double* __restrict__ pts, const float* __restrict__ tarl, int tdim,
-                 const float* __restrict__ dino, int ddim, const uint8_t* __restrict__ tarl_zero,
+                 const float* __restrict__ dino, int ddim, int dcams, const uint8_t* __restrict__ tarl_zero,
                  double alpha, double theta, double gamma, double prox,
                  float* __restrict__ W, long long ld, const int* __restrict__ only_if = nullptr) {
     if (only_if && !*only_if) return;       // conditional fallback after the two-pass form (pair queue overflow)
@@ -158,7 +199,8 @@ k_affinity_exact(int n, const double* __restrict__ pts, const float* __restrict_
                 arg += theta * td;
             }
             if (gamma != 0.0 && dino != nullptr) {
-                double dd = feat_dist8(dino + (size_t)gi * ddim, dino + (size_t)gj * ddim, ddim, lane8);
+                const size_t ds = (size_t)dcams * ddim;
+                double dd = feat_dist8_cams(dino + gi * ds, dino + gj * ds, ddim, dcams, lane8);
                 arg += gamma * dd;                                    // :129-133
             }
             if (live && lane8 == 0) tile[r][c] = (float)exp(-((double)tile[r][c] + arg));
@@ -610,7 +652,7 @@ k_pair_unions(const PairQ* __restrict__ q_all, const long long* __restrict__ q_o
 // pass 2: grid-stride over the queue, one 8-lane group per pair.
 __global__ void __launch_bounds__(256)
 k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int qcap,
-                 const float* __restrict__ tarl, int tdim, const float* __restrict__ dino, int ddim,
+                 const float* __restrict__ tarl, int tdim, const float* __restrict__ dino, int ddim, int dcams,
                  const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
                  float* __restrict__ W, long long ld,
                  const int* __restrict__ inv = nullptr, int base = 0, const int* __restrict__ rid = nullptr,
@@ -654,8 +696,9 @@ k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int 
         }
         if (gamma != 0.0 && dino != nullptr) {
             double dd[2];
+            const size_t ds = (size_t)dcams * ddim;          // row stride: every camera's ddim values
 #pragma unroll
-            for (int s = 0; s < 2; ++s) dd[s] = feat_dist8(dino + (size_t)fi[s] * ddim, dino + (size_t)fj[s] * ddim, ddim, lane8);
+            for (int s = 0; s < 2; ++s) dd[s] = feat_dist8_cams(dino + fi[s] * ds, dino + fj[s] * ds, ddim, dcams, lane8);
 #pragma unroll
             for (int s = 0; s < 2; ++s) arg[s] += gamma * dd[s];         // :129-133
         }

@@ -35,7 +35,7 @@ class Chunk:
     points: np.ndarray                  # (N,3) float64, float32-representable
     instance: np.ndarray                # (N,) int32 ground-truth instance id (>=1)
     tarl: np.ndarray | None = None      # (N,96) float64 from float32, 5 % zero rows
-    dino: np.ndarray | None = None      # (N,384) float64 from float32, 30 % zero rows
+    dino: np.ndarray | list | None = None   # (N,384) float64 from float32, 30 % zero rows ("dino2": one per camera)
     center: np.ndarray = field(default_factory=lambda: np.zeros(3))
 
     @property
@@ -208,6 +208,12 @@ def make_chunk(chunk_id: int = 0, n_target: int = 8192, features: str = "tarl_di
         g = (proto[im] + 0.3 * rng.normal(0, 1, size=(n, 384))).astype(np.float32)
         g[rng.random(n) < 0.30] = 0.0                          # never visible in camera 0
         ch.dino = g.astype(np.float64)
+        if "dino2" in features:
+            # a second camera (CAM_IDS = [0, 1]): same prototypes, its own noise and unseen rows; drawn after every other
+            # draw, so that the other feature strings keep their chunks byte for byte.  ch.dino = [camera 0, camera 1]
+            g2 = (proto[im] + 0.3 * rng.normal(0, 1, size=(n, 384))).astype(np.float32)
+            g2[rng.random(n) < 0.30] = 0.0
+            ch.dino = [ch.dino, g2.astype(np.float64)]
     return ch
 
 

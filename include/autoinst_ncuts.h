@@ -85,6 +85,17 @@ int ancuts_affinity_f32(ancuts_handle* h, int n, const double* d_points, const f
                         const float* d_dino, const ancuts_params* p, float* d_W, int64_t ld,
                         double* d_rowsum, void* stream);
 
+/* DINOv2 term over several cameras (the reference's CAM_IDS, ncuts_utils.py:125-133: exp(-gamma cdist(g_c, g_c)) multiplied
+ * over the cameras c).  The ancuts_*_cams* entry points take d_dino / h_dino point-major: n x dino_cams x p->dino_dim float32,
+ * row i = camera 0's dino_dim values, then camera 1's, ...; p->dino_dim is the width of ONE camera (a multiple of 4).  The term
+ * is evaluated as exp(-gamma * S) with S = dd_0 + dd_1 + ... (float64, camera order), dd_c the Euclidean distance of the two
+ * rows' camera-c slices; zero rows are not neutralised in any camera.  dino_cams >= 1; dino_cams = 1 gives exactly what the
+ * entry point without _cams gives (which forwards here with dino_cams = 1).  dino_cams > 1 with affinity_impl = 1 (tensor-core
+ * form) returns ANCUTS_EUNSUPPORTED. */
+int ancuts_affinity_cams_f32(ancuts_handle* h, int n, const double* d_points, const float* d_tarl,
+                             const float* d_dino, int dino_cams, const ancuts_params* p, float* d_W, int64_t ld,
+                             double* d_rowsum, void* stream);
+
 /* Stage 2 — replaces normalized_cut.py:38,42-47 (W = w + I, d = W.sum(0), D^-1/2 W D^-1/2).
  * d_deg[i] = 1 + sum_j w_ij (float64).  If d_M != NULL also writes M = D^-1/2 (w+I) D^-1/2 in
  * float32 (the pipeline itself applies the scaling inside the matvec and never materialises M). */
@@ -137,6 +148,19 @@ int ancuts_segment_chunks_host(ancuts_handle* h, int num_chunks, const int64_t* 
                                const ancuts_params* p, int32_t* h_labels, int32_t* h_num_segments,
                                ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats,
                                void* stream);
+
+/* The two above with the DINOv2 input of several cameras (layout and term: ancuts_affinity_cams_f32).  The host form copies
+ * each chunk's n_c x dino_cams x dino_dim floats as one piece. */
+int ancuts_segment_chunks_cams(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off,
+                               const double* d_points, const float* d_tarl, const float* d_dino, int dino_cams,
+                               const ancuts_params* p, int32_t* d_labels, int32_t* h_num_segments,
+                               ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats,
+                               void* stream);
+int ancuts_segment_chunks_cams_host(ancuts_handle* h, int num_chunks, const int64_t* h_chunk_off,
+                                    const double* h_points, const float* h_tarl, const float* h_dino, int dino_cams,
+                                    const ancuts_params* p, int32_t* h_labels, int32_t* h_num_segments,
+                                    ancuts_node_stat* h_stats, int32_t stats_cap, int32_t* h_num_stats,
+                                    void* stream);
 
 /* normalized_cut(w, num_points_orig, labels, T, split_lim) (normalized_cut.py:37) on a dense
  * float32 copy of w already on the device (n x n, unit diagonal, symmetric). Blocks. */

@@ -45,10 +45,7 @@ def segment_major_points(points_major, tarl_features=None, dino_features=None, c
         cams = dino_features if isinstance(dino_features, (list, tuple)) else ([dino_features] if dino_features is not None else [])
         if len(cams) == 0:
             raise ValueError("The length should be longer than 0!")          # ncuts_utils.py:126-127
-        if len(cams) > 1:
-            # exp(-g d1) * exp(-g d2) is not a single Euclidean distance; CAM_IDS = [0] in the reference (config.py:72)
-            raise NotImplementedError("more than one camera for the DINOv2 term")
-        dino = cams[0]
+        dino = list(cams)                    # one term per camera (CAM_IDS), multiplied as at ncuts_utils.py:129-133
     if cfg["theta"] and tarl_features is None:
         raise ValueError("theta != 0 needs TARL features")
     seg = api.segment_chunk(points_major, tarl_features if cfg["theta"] else None, dino,

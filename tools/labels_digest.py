@@ -1,6 +1,6 @@
 """Digest of what one segment call returns for the bench batch (labels, node records): to compare two builds of the
 library (ANCUTS_LIB_PATH) that are meant to give bit-identical results.
-    python tools/labels_digest.py [--batch 32] [--matvec 1]"""
+    python tools/labels_digest.py [--batch 32] [--matvec 1] [--config tarl_spatial_dino]"""
 import argparse
 import hashlib
 import os
@@ -16,18 +16,21 @@ def main():
     ap.add_argument("--batch", type=int, default=32)
     ap.add_argument("--n-target", dest="n_target", type=int, default=8192)
     ap.add_argument("--matvec", type=int, default=0, help="ANCUTS_OPT_MATVEC: 0 shared-memory sparse (default), 1 dense")
+    ap.add_argument("--config", default="tarl_spatial", choices=["spatial", "tarl_spatial", "tarl_spatial_dino"])
     args = ap.parse_args()
     import torch
     from autoinst_b200 import api
     from autoinst_b200.synthetic import CONFIGS, make_chunk
-    cfg = CONFIGS["tarl_spatial"]
-    chunks = [make_chunk(1000 + i, n_target=args.n_target, features="tarl") for i in range(args.batch)]
-    packed = api.PackedChunks([c.points for c in chunks], [c.tarl for c in chunks], None, theta=cfg["theta"])
+    cfg = CONFIGS[args.config]
+    chunks = [make_chunk(1000 + i, n_target=args.n_target, features="tarl_dino" if cfg["gamma"] else "tarl")
+              for i in range(args.batch)]
+    packed = api.PackedChunks([c.points for c in chunks], [c.tarl for c in chunks], [c.dino for c in chunks],
+                              theta=cfg["theta"], gamma=cfg["gamma"])
     from autoinst_b200._lib import OPT_MATVEC
     hd = api.Handle.get(torch.device("cuda:0"))
     hd.set_option(OPT_MATVEC, args.matvec)
-    res = api.segment_packed(packed, device=torch.device("cuda:0"), alpha=cfg["alpha"], theta=cfg["theta"], T=cfg["T"],
-                             want_stats=True)
+    res = api.segment_packed(packed, device=torch.device("cuda:0"), alpha=cfg["alpha"], theta=cfg["theta"],
+                             gamma=cfg["gamma"], T=cfg["T"], want_stats=True)
     h = hashlib.sha1()
     for lab in res.labels:
         h.update(np.ascontiguousarray(lab).tobytes())
