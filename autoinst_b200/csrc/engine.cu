@@ -75,7 +75,7 @@ struct Plan {
     PairQ* pairq = nullptr; int* qctr = nullptr;     // pair queue, [2c]=count [2c+1]=overflow
     int qcap = 0;                          // stage entry (ancuts_affinity_f32): capacity of its single queue
     bool deferred = false;                 // points input: per-chunk pair queues kept until the root split (deferred affinity)
-    std::vector<size_t> qoff;              // deferred: first queue entry of chunk c
+    std::vector<long long> qoff;           // deferred: first queue entry of chunk c
     std::vector<int> qcap_c;               // deferred: queue capacity of chunk c
     int* pg_cells = nullptr; int* pg_sorted = nullptr; int* pg_tmp = nullptr; double* pg_spts = nullptr; PairGrid* pg_grid = nullptr;   // deferred: cell grids of the pair search
     int* c_tile0 = nullptr; double* tbox = nullptr; long long* d_qoff = nullptr; int* d_qcap = nullptr;          // cell-sorted sweep
@@ -653,7 +653,6 @@ struct DeferredAffinity {
     const float* tarl;      // all chunks, input order
     const float* dino;      // point-major, dcams * dino_dim values per point
     int dcams;
-    const int64_t* chunk_off;
     const cudaEvent_t* feats;      // host entry: chunk c's features have arrived at feats[c], else NULL
     const int* order;              // batched pair stage: the queue holds cell-sorted ranks, order[base + rank] = input index
     // caller graphs (ancuts_segment_csr_f32): the stored entries take the place of the queued pairs
@@ -725,20 +724,26 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
         }
         const ancuts_params* p = df->p;
         const bool use_tarl = p->theta != 0.0 && df->tarl, use_dino = p->gamma != 0.0 && df->dino;
-        for (int c = 0; c < e.B; ++c) {
-            const size_t o = (size_t)df->chunk_off[c];
-            float* dst = cur ? pl.hW0[c] : pl.hW1[c];
-            if (df->feats) {
+        // the feature arrays hold every chunk from its first point on (chunk offsets start at 0): chunk c at row base[c]
+        if (!df->feats) {
+            // resident inputs: every chunk's pass in one launch
+            LAUNCH(SG_AFFINITY, k_affinity_feats_b<<<dim3(148 * 4, e.B), 256, 0, st>>>(
+                pl.pairq, pl.d_qoff, pl.d_qcap, pl.qctr, pl.c_base, use_tarl ? df->tarl : nullptr, p->tarl_dim,
+                use_dino ? df->dino : nullptr, p->dino_dim, df->dcams, pl.tarl_zero, p->theta, p->gamma, cur ? pl.c_W0 : pl.c_W1,
+                pl.c_ld, e.val, e.rid, e.r_status, df->order));
+        } else {
+            // host entry: each chunk's pass waits for its features
+            for (int c = 0; c < e.B; ++c) {
+                const size_t o = (size_t)pl.base[c];
                 ANCUTS_CUDA(cudaStreamWaitEvent(st, df->feats[c], 0));
                 if (use_tarl)
                     LAUNCH(SG_AFFINITY, k_zero_rows<<<(pl.n[c] + 7) / 8, 256, 0, st>>>(pl.n[c], df->tarl + o * p->tarl_dim, p->tarl_dim,
-                                                                                      pl.tarl_zero + (o - (size_t)df->chunk_off[0])));
+                                                                                      pl.tarl_zero + o));
+                LAUNCH(SG_AFFINITY, k_affinity_feats<<<148 * 4, 256, 0, st>>>(
+                    pl.pairq + pl.qoff[c], pl.qctr + 2 * c, pl.qcap_c[c], use_tarl ? df->tarl : nullptr, p->tarl_dim,
+                    use_dino ? df->dino : nullptr, p->dino_dim, df->dcams, pl.tarl_zero, p->theta, p->gamma,
+                    cur ? pl.hW0[c] : pl.hW1[c], pl.ld[c], e.val, pl.base[c], e.rid, e.r_status, df->order));
             }
-            LAUNCH(SG_AFFINITY, k_affinity_feats<<<148 * 4, 256, 0, st>>>(
-                pl.pairq + pl.qoff[c], pl.qctr + 2 * c, pl.qcap_c[c], use_tarl ? df->tarl + o * p->tarl_dim : nullptr, p->tarl_dim,
-                use_dino ? df->dino + o * df->dcams * p->dino_dim : nullptr, p->dino_dim, df->dcams, pl.tarl_zero + (o - (size_t)df->chunk_off[0]),
-                p->theta, p->gamma, dst, pl.ld[c], e.val, pl.base[c], e.rid, e.r_status,
-                df->order ? df->order + pl.base[c] : nullptr));
         }
         ANCUTS_CUDA(cudaGetLastError());
         cur ^= 1;
@@ -1390,13 +1395,8 @@ int ancuts_feature_pool(ancuts_handle* h, int num_major, const double* d_major, 
 static int run_pairs_batched(ancuts_handle* h, Plan& pl, const double* d_points, const ancuts_params* p, cudaEvent_t points_ev,
                              cudaStream_t st) {
     const int B = pl.B;
-    std::vector<long long> qo(B);
-    for (int c = 0; c < B; ++c) qo[c] = (long long)pl.qoff[c];
     ANCUTS_CUDA(cudaMemcpyAsync(pl.c_tile0, pl.tile0.data(), (B + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
-    ANCUTS_CUDA(cudaMemcpyAsync(pl.d_qoff, qo.data(), B * sizeof(long long), cudaMemcpyHostToDevice, st));
-    ANCUTS_CUDA(cudaMemcpyAsync(pl.d_qcap, pl.qcap_c.data(), B * sizeof(int), cudaMemcpyHostToDevice, st));
-    ANCUTS_CUDA(cudaStreamSynchronize(st));              // qo is a local
-    if (points_ev) ANCUTS_CUDA(cudaStreamWaitEvent(st, points_ev, 0));      // after the synchronise, which so does not wait for the copy
+    if (points_ev) ANCUTS_CUDA(cudaStreamWaitEvent(st, points_ev, 0));
     LAUNCH(SG_AFFINITY, k_pair_grid_b<<<B, 1024, PG_CELLS * sizeof(int), st>>>(pl.c_n, pl.c_base, d_points, p->proximity,
                                                                               pl.pg_cells, pl.pg_sorted, pl.pg_tmp, pl.pg_spts, pl.pg_grid));
     LAUNCH(SG_AFFINITY, k_tile_boxes<<<dim3(pl.max_tiles, B), PS_T, 0, st>>>(pl.c_n, pl.c_base, pl.c_tile0, pl.pg_spts, pl.tbox));
@@ -1574,7 +1574,7 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     layout(pl, h->ws, stats_cap, p->tarl_dim, p->dino_dim, need_tc);
     // deferred != NULL: the input stage builds the root-level forest and W is written after the root split (CSR: from the
     // stored entries); otherwise W is whole before the level loop
-    DeferredAffinity df{p, d_tarl, d_dino, dcams, h_chunk_off, arrival ? arrival->feats : nullptr, pl.grid_pairs ? pl.pg_sorted : nullptr};
+    DeferredAffinity df{p, d_tarl, d_dino, dcams, arrival ? arrival->feats : nullptr, pl.grid_pairs ? pl.pg_sorted : nullptr};
     if (csr) { df.row_ptr = csr->row_ptr; df.col = csr->col; df.val = csr->val; }
     const DeferredAffinity* deferred = (pl.deferred || pl.csr) ? &df : nullptr;
     rc = upload_tables(pl, st);
@@ -1600,6 +1600,9 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     } else {
         if (pl.deferred) {
             ANCUTS_CUDA(cudaMemsetAsync(pl.qctr, 0, 2 * (size_t)num_chunks * sizeof(int), st));
+            // queue offsets and capacities for the kernels that take every chunk in one launch
+            ANCUTS_CUDA(cudaMemcpyAsync(pl.d_qoff, pl.qoff.data(), num_chunks * sizeof(long long), cudaMemcpyHostToDevice, st));
+            ANCUTS_CUDA(cudaMemcpyAsync(pl.d_qcap, pl.qcap_c.data(), num_chunks * sizeof(int), cudaMemcpyHostToDevice, st));
             const int gP = (pl.P + 255) / 256;
             LAUNCH(SG_PARTITION, k_cc_init<<<gP, 256, 0, st>>>(pl.e));          // forest of the root-level components
             if (pl.grid_pairs) {

@@ -649,25 +649,24 @@ k_pair_unions(const PairQ* __restrict__ q_all, const long long* __restrict__ q_o
     }
 }
 
-// pass 2: grid-stride over the queue, one 8-lane group per pair.
-__global__ void __launch_bounds__(256)
-k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int qcap,
-                 const float* __restrict__ tarl, int tdim, const float* __restrict__ dino, int ddim, int dcams,
-                 const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
-                 float* __restrict__ W, long long ld,
-                 const int* __restrict__ inv = nullptr, int base = 0, const int* __restrict__ rid = nullptr,
-                 const int* __restrict__ r_status = nullptr, const int* __restrict__ order = nullptr) {
-    // order != NULL: the queue holds cell-sorted ranks (= root positions); order[rank] = input index, where the features are
-    // inv != NULL (deferred mode): the pair is written at the positions its points have AFTER the root split
-    // (inv[old global position] = new global position), and only if their range goes on to the eigensolver.
-    const int total = min(qctr[0], qcap);
-    if (qctr[1]) return;                             // overflow: everything is redone by the one-kernel form
+// pass 2: one 8-lane group per pair.  Block blk of nblk takes its piece of the `total` queued pairs.
+// The queue holds chunk-local indices; the chunk's rows of tarl, dino, tarl_zero, order and inv start at row `base`.
+// order != NULL: the queue holds cell-sorted ranks (= root positions); order[rank] = input index, where the features are
+// inv != NULL (deferred mode): the pair is written at the positions its points have AFTER the root split
+// (inv[old global position] = new global position), and only if their range goes on to the eigensolver.
+__device__ __forceinline__ void
+affinity_feats_piece(const PairQ* __restrict__ q, int total, int blk, int nblk,
+                     const float* __restrict__ tarl, int tdim, const float* __restrict__ dino, int ddim, int dcams,
+                     const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
+                     float* __restrict__ W, long long ld,
+                     const int* __restrict__ inv, int base, const int* __restrict__ rid,
+                     const int* __restrict__ r_status, const int* __restrict__ order) {
     const int lane8 = threadIdx.x & 7;
     // a block takes a CONTIGUOUS piece of the queue: the sweep appends the hits of one tile pair (128 x 128 points) together,
     // so the piece touches a few hundred feature rows, each about twenty times -- they stay in L1 (a grid-stride walk sent
     // every row read to L2: 147 MB per 8.4 k-point chunk)
-    const int per_block = (((total + (int)gridDim.x - 1) / (int)gridDim.x) + 31) & ~31;
-    const int b0 = blockIdx.x * per_block, b1 = min(total, b0 + per_block);
+    const int per_block = (((total + nblk - 1) / nblk) + 31) & ~31;
+    const int b0 = blk * per_block, b1 = min(total, b0 + per_block);
     // two pairs per 8-lane group and trip, written as two independent instruction streams: a pair is a chain of six
     // dependent global-memory round trips (queue entry, order table, feature rows, position table, range id, range state),
     // and a thread only makes about ten trips -- with one pair at a time the kernel ran at the latency of that chain
@@ -683,7 +682,11 @@ k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int 
             if (live[s]) { PairQ e = q[idx]; gi[s] = e.i; gj[s] = e.j; a[s] = e.a; }
         }
 #pragma unroll
-        for (int s = 0; s < 2; ++s) { fi[s] = order ? order[gi[s]] : gi[s]; fj[s] = order ? order[gj[s]] : gj[s]; arg[s] = 0.0; }
+        for (int s = 0; s < 2; ++s) {
+            fi[s] = base + (order ? order[base + gi[s]] : gi[s]);
+            fj[s] = base + (order ? order[base + gj[s]] : gj[s]);
+            arg[s] = 0.0;
+        }
         if (theta != 0.0 && tarl != nullptr) {
             double td[2];
 #pragma unroll
@@ -724,6 +727,38 @@ k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int 
             }
         }
     }
+}
+
+// one queue (the stage entry, and the host entry's per-chunk passes, which wait for each chunk's features)
+__global__ void __launch_bounds__(256)
+k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int qcap,
+                 const float* __restrict__ tarl, int tdim, const float* __restrict__ dino, int ddim, int dcams,
+                 const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
+                 float* __restrict__ W, long long ld,
+                 const int* __restrict__ inv = nullptr, int base = 0, const int* __restrict__ rid = nullptr,
+                 const int* __restrict__ r_status = nullptr, const int* __restrict__ order = nullptr) {
+    if (qctr[1]) return;                             // overflow: everything is redone by the one-kernel form
+    affinity_feats_piece(q, min(qctr[0], qcap), blockIdx.x, gridDim.x, tarl, tdim, dino, ddim, dcams, tarl_zero, theta, gamma,
+                         W, ld, inv, base, rid, r_status, order);
+}
+
+// deferred pass of a resident batch in one launch, grid (blocks per chunk, chunks): block (x, c) takes the piece of chunk c's
+// queue that block x of a k_affinity_feats launch over that queue alone would take, so every W entry gets the same value.
+// With one launch per chunk a 128-chunk step ran 128 launches of one wave each (592 blocks of 64 registers fill the 148 SMs
+// once) on one stream.  Chunk c's rows start at c_base[c]; its blocks go to Wc[c] with leading dimension c_ld[c].
+__global__ void __launch_bounds__(256)
+k_affinity_feats_b(const PairQ* __restrict__ q_all, const long long* __restrict__ q_off, const int* __restrict__ q_cap,
+                   const int* __restrict__ qctr_all, const int* __restrict__ c_base,
+                   const float* __restrict__ tarl, int tdim, const float* __restrict__ dino, int ddim, int dcams,
+                   const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
+                   float* const* __restrict__ Wc, const int* __restrict__ c_ld,
+                   const int* __restrict__ inv, const int* __restrict__ rid, const int* __restrict__ r_status,
+                   const int* __restrict__ order) {
+    const int c = blockIdx.y;
+    const int* qctr = qctr_all + 2 * c;
+    if (qctr[1]) return;                             // overflow: everything is redone by the one-kernel form
+    affinity_feats_piece(q_all + q_off[c], min(qctr[0], q_cap[c]), blockIdx.x, gridDim.x, tarl, tdim, dino, ddim, dcams,
+                         tarl_zero, theta, gamma, Wc[c], c_ld[c], inv, c_base[c], rid, r_status, order);
 }
 
 // ---------------------------------------------------------------------------------------------
