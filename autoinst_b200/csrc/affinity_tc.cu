@@ -9,7 +9,10 @@
 //   B200: accumulating all 36 MMAs into one TMEM accumulator loses ~0.5 ulp(|acc|) per MMA (1.7e-5 relative
 //   error of W).  So every K = 8 slice of hi.hi gets its OWN accumulator (one MMA, no accumulation, 12 x 32
 //   TMEM columns) and the small cross terms share a 13th; the epilogue adds the 13 partials in float64.
-//   Pairs whose squared distance cancels below 1 % of |f_i|^2 + |f_j|^2 are re-evaluated by direct differences.
+//   Pairs whose squared distance cancels below 1 % of |f_i|^2 + |f_j|^2 are re-evaluated by direct differences, and so
+//   are pairs whose distance is small against theta (|f_i|^2 + |f_j|^2): the error of d^2 is relative to the norms
+//   (measured on B200: up to ~8e-8 (|f_i|^2 + |f_j|^2)), W's relative error is theta err(d^2) / (2 td), and at TARL rows
+//   ten times the synthetic norm it reached 3e-5 with the 1 % rule alone (tests/test_gpu_affinity_edges.py).
 // One CTA (128 threads) per 128 x 32 output tile:
 //   thread 0: mbarrier init, TMA loads of the four operand tiles, 36 MMAs (K = 96 = 3 swizzle atoms x 4),
 //             tcgen05.commit;   warp 0: TMEM alloc/dealloc (512 columns);
@@ -247,6 +250,9 @@ k_affinity_tc(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
     const bool zi = (gi < n && P.tarl_zero) ? (P.tarl_zero[gi] != 0) : false;
     const float ox = (float)(px - prow[0]), oy = (float)(py - prow[1]), oz = (float)(pz - prow[2]);
     const float lim32 = (float)((P.prox + 1e-2) * (P.prox + 1e-2) * 1.001);
+    // direct differences below td = 2e-2 theta (|f_i|^2 + |f_j|^2): W's relative error stays below 25 x the relative
+    // error of d^2 (~2e-6) at any feature scale
+    const double near_rel = 2e-2 * P.theta;
 #pragma unroll 2
     for (int c = 0; c < TC_N; ++c) {
         float out = 0.0f;
@@ -266,7 +272,7 @@ k_affinity_tc(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
                         double d2 = nsum - 2.0 * grow[c];
                         if (gi == gj) {
                             d2 = 0.0;
-                        } else if (d2 < 1e-2 * nsum) {                    // cancellation: direct differences
+                        } else if (d2 < 1e-2 * nsum || d2 < (near_rel * nsum) * (near_rel * nsum)) {   // direct differences
                             const float* fa = P.tarl + (size_t)gi * P.tdim;
                             const float* fb = P.tarl + (size_t)gj * P.tdim;
                             double acc2 = 0.0;

@@ -192,7 +192,11 @@ k_affinity_exact(int n, const double* __restrict__ pts, const float* __restrict_
             int r = idx / AT, c = idx % AT;
             int gi = row0 + r, gj = col0 + c;
             if (!live) { gi = 0; gj = 0; }                            // keep the 8-lane shuffles uniform
-            double arg = 0.0;
+            // alpha * spatial distance again in float64 (the tile holds it rounded to float32, one ulp of W off the
+            // rounded reference)
+            const double dx = pr[r][0] - pc[c][0], dy = pr[r][1] - pc[c][1], dz = pr[r][2] - pc[c][2];
+            const double sd = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
+            double arg = alpha != 0.0 ? alpha * sd : 0.0;
             if (theta != 0.0 && tarl != nullptr) {
                 double td = feat_dist8(tarl + (size_t)gi * tdim, tarl + (size_t)gj * tdim, tdim, lane8);
                 if (tarl_zero[gi] | tarl_zero[gj]) td = 0.0;          // ncuts_utils.py:145-146
@@ -203,7 +207,7 @@ k_affinity_exact(int n, const double* __restrict__ pts, const float* __restrict_
                 double dd = feat_dist8_cams(dino + gi * ds, dino + gj * ds, ddim, dcams, lane8);
                 arg += gamma * dd;                                    // :129-133
             }
-            if (live && lane8 == 0) tile[r][c] = (float)exp(-((double)tile[r][c] + arg));
+            if (live && lane8 == 0) tile[r][c] = (float)exp(-arg);
         }
         __syncthreads();
     }
