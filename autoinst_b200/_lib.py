@@ -32,7 +32,7 @@ EXPORTS = [
 ]
 
 # ancuts_set_option (include/autoinst_ncuts.h; option 0 is retired)
-OPT_PAIR_SEARCH, OPT_MATVEC, OPT_CLUSTER_MAP, OPT_FUSED_CUT = 1, 2, 3, 4
+OPT_PAIR_SEARCH, OPT_MATVEC, OPT_CLUSTER_MAP, OPT_FUSED_CUT, OPT_NODE_FORM = 1, 2, 3, 4, 5
 PAIRS_SORTED, PAIRS_SHUFFLED = 0, 1
 MATVEC_SPARSE, MATVEC_DENSE = 0, 1
 

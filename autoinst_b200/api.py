@@ -58,7 +58,8 @@ class Handle:
         """Alternative implementations behind the same results (`ancuts_set_option`): _lib.OPT_PAIR_SEARCH
         (0 cell-sorted sweep, 1 shuffled sweep), OPT_MATVEC (0 slices compressed into shared memory, 1 dense blocks
         from HBM), OPT_CLUSTER_MAP (tuning), OPT_FUSED_CUT (0 the cut decision inside the sparse-form eigensolver kernel,
-        1 as its own kernels).  Option 0 is retired and raises."""
+        1 as its own kernels), OPT_NODE_FORM (0 recursion nodes as CSR, dense blocks only where a kernel reads them,
+        1 every node as a dense block).  Option 0 is retired and raises."""
         check(self.lib.ancuts_set_option(self.h, int(option), int(value)))
 
     def sparse_accounting(self) -> dict:

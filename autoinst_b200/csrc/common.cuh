@@ -162,7 +162,7 @@ struct Eng {
     double* deg; double* sinv; double* wbuf; double* ybuf; double* ev;
     double* zbuf;           // S wbuf (input of the matvec), P + 4 entries
     uint8_t* bucket; uint8_t* side;
-    int* rownnz;            // stored (non-zero) entries of every row inside its node's block, written by k_degree
+    int* rownnz;            // stored (non-zero) entries of every row inside its node's block, written by k_degree (or with the CSR rows)
     int* parent; int* croot;
     unsigned long long* key; unsigned long long* key2; int* val; int* val2; int* flag; int* incl;
     double* V;              // (kmax+2) rows of P
@@ -204,6 +204,12 @@ struct Eng {
     unsigned long long* dbg;   // optional [4 cluster sizes][8] phase cycle sums of the cluster kernel (thread 0 of rank 0), or NULL
     int w_guard;          // 1 = entries next to a block may be non-finite (caller-provided W without a gather)
     const double* pts;    // [P][3] input coordinates (chunk c at c_base[c], input order) for the Lanczos start vector, or NULL
+    // node form (ANCUTS_OPT_NODE_FORM): node_csr = 1 keeps every active node as CSR rows over global positions (columns local
+    // to the node, ascending; the unit diagonal and the non-zero float32 affinities only): rows of position g at
+    // [csr_ptr[g], csr_ptr[g + 1]).  The dense blocks then hold only the nodes k_ncsr_densify wrote this level.
+    int node_csr;
+    const int* csr_ptr; const int* csr_col; const float* csr_val;
+    int* dn_list; int* dn_count;          // slots k_ncsr_need lists for k_ncsr_densify
 };
 
 }  // namespace ancuts

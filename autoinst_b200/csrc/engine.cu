@@ -14,6 +14,7 @@
 #include "kernels_pool.cuh"
 #include "kernels_dino.cuh"
 #include "kernels_csr.cuh"
+#include "kernels_nodecsr.cuh"
 
 namespace ancuts {
 
@@ -83,6 +84,12 @@ struct Plan {
     bool grid_pairs = false;
     bool csr = false;                      // caller graphs in CSR form (ancuts_segment_csr_f32)
     unsigned long long* csr_err = nullptr; int* csr_out = nullptr;      // k_csr_validate: first violation per graph, range flag
+    // CSR node form (deferred points input, ANCUTS_OPT_NODE_FORM = 0): two row sets (the level's and its children's), the
+    // per-pair values of the feature pass, per-row counts / cursors, the list of slots k_ncsr_densify writes
+    bool node_csr = false;
+    int* ncsr_ptr[2] = {nullptr, nullptr}; int* ncsr_col[2] = {nullptr, nullptr}; float* ncsr_val[2] = {nullptr, nullptr};
+    int ncsr_cur = 0;
+    int* ncsr_cnt = nullptr; float* pslot = nullptr; int* ncsr_list = nullptr; int* ncsr_count = nullptr;
     ancuts_node_stat* stats;
     Eng e{};            // zero: optional pointers (sel, unfused, dbg, stats) are NULL unless a call sets them
 };
@@ -92,7 +99,9 @@ static size_t cub_temp_bytes(int P) {
     cub::DeviceRadixSort::SortPairs(nullptr, a, (unsigned long long*)nullptr, (unsigned long long*)nullptr,
                                     (int*)nullptr, (int*)nullptr, P, 0, 64);
     cub::DeviceScan::InclusiveSum(nullptr, b, (int*)nullptr, (int*)nullptr, P);
-    return std::max(a, b) + 256;
+    size_t c = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, c, (int*)nullptr, (int*)nullptr, P + 1);     // row pointers of the CSR node form
+    return std::max(std::max(a, b), c) + 256;
 }
 
 // lay out every buffer; with base == nullptr only the size is computed
@@ -177,6 +186,22 @@ static size_t layout(Plan& pl, char* base, int stats_cap, int tdim, int ddim, bo
         pl.tbox = ar.take<double>((size_t)pl.tile0[B] * 6);
         pl.d_qoff = ar.take<long long>((size_t)B);
         pl.d_qcap = ar.take<int>((size_t)B);
+        // CSR node form: at most both directions of every queued pair plus the diagonal (int row pointers)
+        const size_t ecap = 2 * total + (size_t)P;
+        if (ecap > 0x7fffffffULL) pl.node_csr = false;
+        if (pl.node_csr) {
+            for (int k = 0; k < 2; ++k) {
+                pl.ncsr_ptr[k] = ar.take<int>((size_t)P + 1);
+                pl.ncsr_col[k] = ar.take<int>(ecap);
+                pl.ncsr_val[k] = ar.take<float>(ecap);
+            }
+            pl.ncsr_cnt = ar.take<int>((size_t)P + 1);
+            pl.pslot = ar.take<float>(total);
+            pl.ncsr_list = ar.take<int>((size_t)pl.active_cap);
+            pl.ncsr_count = ar.take<int>(1);
+        }
+    } else {
+        pl.node_csr = false;
     }
     pl.csr_err = nullptr; pl.csr_out = nullptr;
     if (pl.csr) { pl.csr_err = ar.take<unsigned long long>(B); pl.csr_out = ar.take<int>(1); }
@@ -423,9 +448,23 @@ static int run_affinity(ancuts_handle* h, Plan& pl, int n, const double* pts, co
     return ANCUTS_OK;
 }
 
+// CSR node form: dense blocks of the level's nodes that read dense W (all != 0: every node, for the grid-wide Lanczos
+// path and the cut kernels after it; otherwise nodes above CL_NMAX points and slices that would not fit the cluster kernel)
+static int densify_nodes(ancuts_handle* h, Eng& e, int cur, int num_active, bool all, unsigned cmap, cudaStream_t st) {
+    ANCUTS_CUDA(cudaMemsetAsync(e.dn_count, 0, sizeof(int), st));
+    LAUNCH(SG_PARTITION, k_ncsr_need<<<num_active, 256, 0, st>>>(e, all ? 1 : 0, cmap, e.dn_list, e.dn_count));
+    LAUNCH(SG_PARTITION, k_ncsr_densify<<<dim3(ZB_BLOCKS, num_active), 256, 0, st>>>(e, cur, e.dn_list, e.dn_count));
+    ANCUTS_CUDA(cudaGetLastError());
+    return ANCUTS_OK;
+}
+
 // Lanczos for all active nodes of the current table (degrees must be set)
 static int run_lanczos(ancuts_handle* h, Eng& e, int cur, int num_active, int max_n, cudaStream_t st) {
     const int KS = e.KS;
+    if (e.node_csr) {                 // k_matvec, and after it the cut kernels, read every node's dense block
+        int rc = densify_nodes(h, e, cur, num_active, true, 0u, st);
+        if (rc) return rc;
+    }
     LAUNCH(SG_REORTH, k_lanczos_init<<<num_active, 256, 0, st>>>(e));
     const int nch_max = (max_n + CH - 1) / CH;
     const size_t up_smem = (size_t)(KS + CH + 8) * 8;
@@ -505,10 +544,6 @@ static cudaError_t launch_cluster(const Eng& e, int cur, const int* ids, int cou
 static int run_lanczos_all(ancuts_handle* h, Eng& e, int cur, int num_active, int max_n, const int* class_cnt,
                            int big_cnt, cudaStream_t st) {
     ANCUTS_CUDA(cudaMemsetAsync(e.ctr + 4, 0, sizeof(int), st));
-    // one timed "launch" per level: the concurrent cluster kernels from fork to join on the launching stream
-    cudaEvent_t t_a = nullptr, t_b = nullptr;
-    if (h->stage_timing) { t_a = take_event(h); t_b = take_event(h); cudaEventRecord(t_a, st); }
-    ANCUTS_CUDA(cudaEventRecord(h->ev_fork, st));
     bool any = false, launch_failed = false;
     // bins <=320, <=512, <=640, <=1024, <=2048, <=4096 points.  Latency mapping (short critical path) when all
     // clusters of the level are resident at once; otherwise the level is bound by SM time and fewer CTAs per
@@ -533,6 +568,17 @@ static int run_lanczos_all(ancuts_handle* h, Eng& e, int cur, int num_active, in
         for (int b = 0; b < CL_CLASSES; ++b) ok &= ((nmax[b] + c_user[b] - 1) / c_user[b] <= CL_RPMAX);
         if (ok && d == 0) cmap = c_user;
     }
+    if (e.node_csr && sparse_on) {    // nodes whose slices would not fit read their dense block inside the cluster kernel
+        unsigned packed = 0;
+        for (int b = 0; b < CL_CLASSES; ++b) packed |= (unsigned)cmap[b] << (4 * b);
+        int rc = densify_nodes(h, e, cur, num_active, false, packed, st);
+        if (rc) return rc;
+    }
+    // one timed "launch" per level: the concurrent cluster kernels from fork to join on the launching stream (the fork
+    // follows the dense blocks the cluster kernels read)
+    cudaEvent_t t_a = nullptr, t_b = nullptr;
+    if (h->stage_timing) { t_a = take_event(h); t_b = take_event(h); cudaEventRecord(t_a, st); }
+    ANCUTS_CUDA(cudaEventRecord(h->ev_fork, st));
     for (int cls = CL_CLASSES - 1; cls >= 0; --cls) {          // largest nodes first
         int cnt = class_cnt[cls];
         if (cnt <= 0) continue;
@@ -661,6 +707,32 @@ struct DeferredAffinity {
     const float* val = nullptr;
 };
 
+static void set_node_csr(Plan& pl, int s) {
+    pl.ncsr_cur = s;
+    pl.e.csr_ptr = pl.ncsr_ptr[s]; pl.e.csr_col = pl.ncsr_col[s]; pl.e.csr_val = pl.ncsr_val[s];
+}
+
+// CSR node form, root level (after the root split and the feature pass, which counted the entries per row on top of the
+// diagonal k_ncsr_diag set; inv = e.val): scan, fill (diagonal first, then the pairs through atomic cursors), sort each
+// row by column into the other row set and take its degree.
+static int build_root_csr(ancuts_handle* h, Plan& pl, cudaStream_t st) {
+    Eng& e = pl.e;
+    const int P = e.P, g1 = (P + 1 + 255) / 256;
+    const dim3 gq(148 * 4, e.B);
+    size_t tmp = pl.cub_bytes;
+    h->launches_total++; h->stage_launches[SG_AFFINITY]++;
+    ANCUTS_CUDA(cub::DeviceScan::ExclusiveSum(pl.cub_tmp, tmp, pl.ncsr_cnt, pl.ncsr_ptr[0], P + 1, st));
+    LAUNCH(SG_AFFINITY, k_ncsr_fill_diag<<<g1, 256, 0, st>>>(e, pl.ncsr_ptr[0], pl.ncsr_cnt, pl.ncsr_col[0], pl.ncsr_val[0]));
+    LAUNCH(SG_AFFINITY, k_ncsr_pairs<<<gq, 256, 0, st>>>(pl.pairq, pl.d_qoff, pl.d_qcap, pl.qctr, pl.c_base, pl.pslot,
+                                                                 e, e.val, pl.ncsr_cnt, pl.ncsr_col[0], pl.ncsr_val[0]));
+    ANCUTS_CUDA(cudaMemcpyAsync(pl.ncsr_ptr[1], pl.ncsr_ptr[0], (size_t)(P + 1) * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    LAUNCH(SG_DEGREE, k_ncsr_sort_rows<<<(P + 7) / 8, 256, 0, st>>>(e, pl.ncsr_ptr[0], pl.ncsr_col[0], pl.ncsr_val[0],
+                                                                       pl.ncsr_col[1], pl.ncsr_val[1]));
+    ANCUTS_CUDA(cudaGetLastError());
+    set_node_csr(pl, 1);
+    return ANCUTS_OK;
+}
+
 static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int max_split_n, bool components,
                        cudaStream_t st, int* class_cnt = nullptr, int* big_cnt = nullptr,
                        const DeferredAffinity* df = nullptr, bool forest_inited = false) {
@@ -708,10 +780,12 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
     std::swap(e.r_status, e.q_status); std::swap(e.r_level, e.q_level);
     std::swap(e.rid, e.rid2); std::swap(e.perm, e.perm2);
     if (num_active > 0 && df) {
-        // deferred affinity: there is no matrix to gather from.  Zero the blocks of the active ranges (unit diagonal)
-        // and scatter the queued pairs of every chunk to the positions their points have now.
-        LAUNCH(SG_AFFINITY, k_zero_blocks<<<dim3(ZB_BLOCKS, num_active), 256, 0, st>>>(e, cur));
+        // deferred affinity: there is no matrix to gather from.  Dense node form: zero the blocks of the active ranges (unit
+        // diagonal) and scatter the queued pairs of every chunk to the positions their points have now.  CSR node form: the
+        // feature pass writes one value per queued pair and build_root_csr places them.
+        if (!pl.node_csr) LAUNCH(SG_AFFINITY, k_zero_blocks<<<dim3(ZB_BLOCKS, num_active), 256, 0, st>>>(e, cur));
         LAUNCH(SG_PARTITION, k_inverse_positions<<<gP, tb, 0, st>>>(e, e.val));
+        if (pl.node_csr) LAUNCH(SG_AFFINITY, k_ncsr_diag<<<(P + 1 + 255) / 256, 256, 0, st>>>(e, pl.ncsr_cnt));
         if (df->row_ptr) {
             // caller graphs: one pass over every graph's rows in input order
             int nmax = 0;
@@ -730,7 +804,7 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
             LAUNCH(SG_AFFINITY, k_affinity_feats_b<<<dim3(148 * 4, e.B), 256, 0, st>>>(
                 pl.pairq, pl.d_qoff, pl.d_qcap, pl.qctr, pl.c_base, use_tarl ? df->tarl : nullptr, p->tarl_dim,
                 use_dino ? df->dino : nullptr, p->dino_dim, df->dcams, pl.tarl_zero, p->theta, p->gamma, cur ? pl.c_W0 : pl.c_W1,
-                pl.c_ld, e.val, e.rid, e.r_status, df->order));
+                pl.c_ld, e.val, e.rid, e.r_status, df->order, pl.node_csr ? pl.pslot : nullptr, pl.ncsr_cnt));
         } else {
             // host entry: each chunk's pass waits for its features
             for (int c = 0; c < e.B; ++c) {
@@ -742,11 +816,31 @@ static int run_rebuild(ancuts_handle* h, Plan& pl, int& cur, int num_split, int 
                 LAUNCH(SG_AFFINITY, k_affinity_feats<<<148 * 4, 256, 0, st>>>(
                     pl.pairq + pl.qoff[c], pl.qctr + 2 * c, pl.qcap_c[c], use_tarl ? df->tarl : nullptr, p->tarl_dim,
                     use_dino ? df->dino : nullptr, p->dino_dim, df->dcams, pl.tarl_zero, p->theta, p->gamma,
-                    cur ? pl.hW0[c] : pl.hW1[c], pl.ld[c], e.val, pl.base[c], e.rid, e.r_status, df->order));
+                    pl.node_csr ? nullptr : (cur ? pl.hW0[c] : pl.hW1[c]), pl.ld[c], e.val, pl.base[c], e.rid, e.r_status,
+                    df->order, pl.node_csr ? pl.pslot + pl.qoff[c] : nullptr, pl.ncsr_cnt));
             }
         }
         ANCUTS_CUDA(cudaGetLastError());
+        if (pl.node_csr) {
+            int rc2 = build_root_csr(h, pl, st);
+            if (rc2) return rc2;
+        }
         cur ^= 1;
+    } else if (num_active > 0 && pl.node_csr) {
+        // children's rows from their parents' rows (no dense block is gathered)
+        LAUNCH(SG_PARTITION, k_inverse_positions<<<gP, tb, 0, st>>>(e, e.val));
+        const int s = pl.ncsr_cur, gr = (P + 1 + 7) / 8;
+        LAUNCH(SG_PARTITION, k_ncsr_children<false><<<gr, 256, 0, st>>>(e, e.val, pl.ncsr_ptr[s], pl.ncsr_col[s],
+                                                                          pl.ncsr_val[s], pl.ncsr_cnt, nullptr, nullptr));
+        tmp = pl.cub_bytes;
+        h->launches_total++; h->stage_launches[SG_PARTITION]++;
+        ANCUTS_CUDA(cub::DeviceScan::ExclusiveSum(pl.cub_tmp, tmp, pl.ncsr_cnt, pl.ncsr_ptr[s ^ 1], P + 1, st));
+        LAUNCH(SG_DEGREE, k_ncsr_children<true><<<gr, 256, 0, st>>>(e, e.val, pl.ncsr_ptr[s], pl.ncsr_col[s],
+                                                                         pl.ncsr_val[s], pl.ncsr_ptr[s ^ 1], pl.ncsr_col[s ^ 1],
+                                                                         pl.ncsr_val[s ^ 1]));
+        ANCUTS_CUDA(cudaGetLastError());
+        set_node_csr(pl, s ^ 1);
+        cur ^= 1;          // the level's on-demand dense blocks go to the other buffer (k_cc_union reads the previous one)
     } else if (num_active > 0) {
         dim3 g((max_n + 255) / 256, (max_n + 15) / 16, num_active);
         LAUNCH(SG_PARTITION, k_gather_blocks_cur<<<g, 256, 0, st>>>(e, cur));
@@ -784,7 +878,7 @@ static int run_levels(ancuts_handle* h, Plan& pl, const ancuts_params* p, int cu
         int num_active = h->h_ctr[1], max_n = h->h_ctr[2];
         if (num_active == 0) break;
         dim3 gdeg((max_n + 7) / 8, num_active);
-        LAUNCH(SG_DEGREE, k_degree<<<gdeg, 256, 0, st>>>(e, cur));
+        if (!e.node_csr) LAUNCH(SG_DEGREE, k_degree<<<gdeg, 256, 0, st>>>(e, cur));   // CSR rows: taken as they were written
         // the split list and the component forest of this level start empty BEFORE the Lanczos launch: cluster kernels that
         // hold their node as CSR slices decide the cut and join the components themselves (cl_fused_cut)
         ANCUTS_CUDA(cudaMemsetAsync(e.ctr + 5, 0, sizeof(int), st));
@@ -916,6 +1010,7 @@ int64_t ancuts_segment_workspace_bytes(int num_chunks, const int32_t* h_chunk_n,
     int kmax = lanczos_max_steps > 0 ? lanczos_max_steps : KMAX_DEFAULT;
     make_plan(pl, num_chunks, h_chunk_n, nullptr, nullptr, kmax, 0);
     pl.deferred = true;                                // upper bound: tensor-core scratch and pair queues both counted
+    pl.node_csr = true;                                // and the CSR node form's rows
     return (int64_t)layout(pl, nullptr, 1 << 16, 96, 384, true);
 }
 
@@ -1568,6 +1663,11 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
     pl.deferred = !d_W_dense && !csr && p->affinity_impl == 0;
     pl.grid_pairs = pl.deferred && h->opt[ANCUTS_OPT_PAIR_SEARCH] == 0;     // cell-sorted, batched sweep (default) or the shuffled one
     if (pl.grid_pairs) ANCUTS_CUDA(cudaFuncSetAttribute(k_pair_grid_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(PG_CELLS * sizeof(int))));
+    // CSR node form: the cell-sorted pair queue with the default eigensolver forms (shared-memory slices, fused cut, cluster
+    // kernels).  A dense matvec, the separate cut kernels, the grid-wide Lanczos path and the shuffled pair search (its
+    // queue holds input indices) read or build every node's dense block anyway: those calls keep the dense node form.
+    pl.node_csr = pl.grid_pairs && h->opt[ANCUTS_OPT_NODE_FORM] == 0 && h->opt[ANCUTS_OPT_MATVEC] == 0 &&
+                  h->opt[ANCUTS_OPT_FUSED_CUT] == 0 && p->lanczos_impl != 1;
     size_t bytes = layout(pl, nullptr, stats_cap, p->tarl_dim, p->dino_dim, need_tc);
     rc = ensure_ws(h, bytes);
     if (rc) return rc;
@@ -1623,6 +1723,7 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
             ANCUTS_CUDA(cudaStreamSynchronize(st));
             for (int c = 0; c < num_chunks; ++c)
                 if (hq[2 * c + 1] != 0) deferred = nullptr;
+            if (!deferred) pl.node_csr = false;             // the one-kernel form writes dense W: dense node form
         } else if (arrival) {
             ANCUTS_CUDA(cudaStreamWaitEvent(st, arrival->points, 0));
         }
@@ -1644,6 +1745,8 @@ static int segment_common(ancuts_handle* h, int num_chunks, const int64_t* h_chu
                          4.0 * n[c] * (3 + (p->theta != 0 ? p->tarl_dim : 0) + (p->gamma != 0 ? dcams * p->dino_dim : 0));
         h->stage_bytes[SG_AFFINITY] = aff_bytes;
     }
+    pl.e.node_csr = pl.node_csr ? 1 : 0;
+    pl.e.dn_list = pl.ncsr_list; pl.e.dn_count = pl.ncsr_count;
     rc = run_levels(h, pl, p, 0, d_labels, h_num_segments, st, deferred);
     if (rc) return rc;
     rc = copy_stats(h, pl, h_stats, stats_cap, h_num_stats, st);

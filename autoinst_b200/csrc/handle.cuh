@@ -36,7 +36,7 @@ struct ancuts_handle {
     bool attrs_set = false;
     // Code paths with more than one implementation behind the same results (ancuts_set_option; every one is parity-tested;
     // option 0 is retired):
-    int opt[ANCUTS_OPT_COUNT] = {0, 0, 0, 0, 0};
+    int opt[ANCUTS_OPT_COUNT] = {0, 0, 0, 0, 0, 0};
     int last_unconverged = 0;                // eigensolver nodes of the last segment call that stopped at lanczos_max_steps
     cudaStream_t copy_stream = nullptr;      // host entry point: H2D copies run ahead of the affinity kernels
     cudaEvent_t points_ev = nullptr;         // host entry point: the coordinates of every chunk have arrived

@@ -1050,10 +1050,22 @@ k_lanczos_cluster(Eng e, int cur, const int* __restrict__ ids, int dyn_doubles) 
             if (tid < nr) ptr[tid] = sp_wtot[warp] + incl - mine;
             if (tid == 0) ptr[nr] = total;
             __syncthreads();
-            for (int i = warp; i < nr; i += 2 * CL_WARPS) {
-                const int i2 = i + CL_WARPS;
-                sp_fill_rows(v.W + (size_t)(v.ro + r0 + i) * v.ld, i2 < nr ? v.W + (size_t)(v.ro + r0 + i2) * v.ld : nullptr, a0,
-                             c_lo, c_hi, lane, val, col, ptr[i], i2 < nr ? ptr[i2] : 0, pad);
+            if (e.node_csr) {
+                // the node's CSR rows hold exactly the entries sp_fill_rows keeps, in the same order: copy them
+                for (int i = warp; i < nr; i += CL_WARPS) {
+                    const int b = e.csr_ptr[g0 + i], cnt = e.csr_ptr[g0 + i + 1] - b, o = ptr[i];
+                    for (int k = lane; k < cnt; k += 32) {
+                        val[o + k] = e.csr_val[b + k];
+                        col[o + k] = (unsigned short)((e.csr_col[b + k] + pad) << 3);
+                    }
+                    if (lane < ((4 - (cnt & 3)) & 3)) { val[o + cnt + lane] = 0.0f; col[o + cnt + lane] = 0; }
+                }
+            } else {
+                for (int i = warp; i < nr; i += 2 * CL_WARPS) {
+                    const int i2 = i + CL_WARPS;
+                    sp_fill_rows(v.W + (size_t)(v.ro + r0 + i) * v.ld, i2 < nr ? v.W + (size_t)(v.ro + r0 + i2) * v.ld : nullptr,
+                                 a0, c_lo, c_hi, lane, val, col, ptr[i], i2 < nr ? ptr[i2] : 0, pad);
+                }
             }
             sp.val = val; sp.col = col; sp.ptr = ptr;
             if (tid == 0) S.sp_nnz = total - fill;       // accounting only: shared memory, not a register across the steps

@@ -664,7 +664,8 @@ affinity_feats_piece(const PairQ* __restrict__ q, int total, int blk, int nblk,
                      const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
                      float* __restrict__ W, long long ld,
                      const int* __restrict__ inv, int base, const int* __restrict__ rid,
-                     const int* __restrict__ r_status, const int* __restrict__ order) {
+                     const int* __restrict__ r_status, const int* __restrict__ order, float* __restrict__ slot,
+                     int* __restrict__ cnt) {
     const int lane8 = threadIdx.x & 7;
     // a block takes a CONTIGUOUS piece of the queue: the sweep appends the hits of one tile pair (128 x 128 points) together,
     // so the piece touches a few hundred feature rows, each about twenty times -- they stay in L1 (a grid-stride walk sent
@@ -723,7 +724,18 @@ affinity_feats_piece(const PairQ* __restrict__ q, int total, int blk, int nblk,
             }
 #pragma unroll
             for (int s = 0; s < 2; ++s) {
-                if (keep[s]) {
+                if (slot) {
+                    // CSR node form: the value in queue order (0 = not stored), coalesced, and one more entry in the two
+                    // rows (k_ncsr_pairs places it with the same test)
+                    if (live[s]) {
+                        const float w = keep[s] ? (float)exp(-(a[s] + arg[s])) : 0.0f;
+                        slot[i0 + 32 * s + (threadIdx.x >> 3)] = w;
+                        if (w != 0.0f && rid[base + wi[s]] == rid[base + wj[s]]) {
+                            atomicAdd(cnt + base + wi[s], 1);
+                            atomicAdd(cnt + base + wj[s], 1);
+                        }
+                    }
+                } else if (keep[s]) {
                     const float w = (float)exp(-(a[s] + arg[s]));
                     W[(size_t)wi[s] * ld + wj[s]] = w;
                     W[(size_t)wj[s] * ld + wi[s]] = w;
@@ -740,16 +752,18 @@ k_affinity_feats(const PairQ* __restrict__ q, const int* __restrict__ qctr, int 
                  const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
                  float* __restrict__ W, long long ld,
                  const int* __restrict__ inv = nullptr, int base = 0, const int* __restrict__ rid = nullptr,
-                 const int* __restrict__ r_status = nullptr, const int* __restrict__ order = nullptr) {
+                 const int* __restrict__ r_status = nullptr, const int* __restrict__ order = nullptr,
+                 float* __restrict__ slot = nullptr, int* __restrict__ cnt = nullptr) {
     if (qctr[1]) return;                             // overflow: everything is redone by the one-kernel form
     affinity_feats_piece(q, min(qctr[0], qcap), blockIdx.x, gridDim.x, tarl, tdim, dino, ddim, dcams, tarl_zero, theta, gamma,
-                         W, ld, inv, base, rid, r_status, order);
+                         W, ld, inv, base, rid, r_status, order, slot, cnt);
 }
 
 // deferred pass of a resident batch in one launch, grid (blocks per chunk, chunks): block (x, c) takes the piece of chunk c's
 // queue that block x of a k_affinity_feats launch over that queue alone would take, so every W entry gets the same value.
 // With one launch per chunk a 128-chunk step ran 128 launches of one wave each (592 blocks of 64 registers fill the 148 SMs
-// once) on one stream.  Chunk c's rows start at c_base[c]; its blocks go to Wc[c] with leading dimension c_ld[c].
+// once) on one stream.  Chunk c's rows start at c_base[c]; its blocks go to Wc[c] with leading dimension c_ld[c], or, with
+// slot != NULL (CSR node form), the values to slot[q_off[c] + queue index] and the rows' entry counts to cnt.
 __global__ void __launch_bounds__(256)
 k_affinity_feats_b(const PairQ* __restrict__ q_all, const long long* __restrict__ q_off, const int* __restrict__ q_cap,
                    const int* __restrict__ qctr_all, const int* __restrict__ c_base,
@@ -757,12 +771,13 @@ k_affinity_feats_b(const PairQ* __restrict__ q_all, const long long* __restrict_
                    const uint8_t* __restrict__ tarl_zero, double theta, double gamma,
                    float* const* __restrict__ Wc, const int* __restrict__ c_ld,
                    const int* __restrict__ inv, const int* __restrict__ rid, const int* __restrict__ r_status,
-                   const int* __restrict__ order) {
+                   const int* __restrict__ order, float* __restrict__ slot, int* __restrict__ cnt) {
     const int c = blockIdx.y;
     const int* qctr = qctr_all + 2 * c;
     if (qctr[1]) return;                             // overflow: everything is redone by the one-kernel form
     affinity_feats_piece(q_all + q_off[c], min(qctr[0], q_cap[c]), blockIdx.x, gridDim.x, tarl, tdim, dino, ddim, dcams,
-                         tarl_zero, theta, gamma, Wc[c], c_ld[c], inv, c_base[c], rid, r_status, order);
+                         tarl_zero, theta, gamma, slot ? nullptr : Wc[c], c_ld[c], inv, c_base[c], rid, r_status, order,
+                         slot ? slot + q_off[c] : nullptr, cnt);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -286,12 +286,20 @@ int ancuts_last_unconverged(ancuts_handle* h);
  *                             <= 320, 512, 640, 1024, 2048, 4096 points (tuning)
  *   ANCUTS_OPT_FUSED_CUT      0 a cluster kernel that holds its node as CSR slices also takes the node's cut decision (sign,
  *                               thresholds, buckets, N-cut scan, decision, side flags, component unions) in its epilogue,
- *                             1 the cut always runs as its own kernels after the eigensolver */
+ *                             1 the cut always runs as its own kernels after the eigensolver
+ *   ANCUTS_OPT_NODE_FORM      0 recursion nodes of the segment path kept as CSR (built from the pair queue, children
+ *                               compacted from the parent's rows); a node's dense block is written only for the nodes that
+ *                               read dense W (slices that do not fit, nodes above 4096 points or past the cluster kernel's
+ *                               step limit),
+ *                             1 every node as a dense block in HBM (zeroed, scattered and gathered on every level).
+ *                             Calls with a dense matvec, separate cut kernels, the grid-wide Lanczos path, the shuffled
+ *                             pair search, caller-supplied graphs or an overflowed pair queue take form 1 */
 #define ANCUTS_OPT_PAIR_SEARCH   1
 #define ANCUTS_OPT_MATVEC        2
 #define ANCUTS_OPT_CLUSTER_MAP   3
 #define ANCUTS_OPT_FUSED_CUT     4
-#define ANCUTS_OPT_COUNT         5
+#define ANCUTS_OPT_NODE_FORM     5
+#define ANCUTS_OPT_COUNT         6
 int ancuts_set_option(ancuts_handle* h, int option, int value);
 
 /* Shared-memory sparse matvec form (ANCUTS_OPT_MATVEC = 0), last segment call: out2[0] = sum over the nodes it ran of
